@@ -6,6 +6,7 @@
          --master-port P bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...      # CPU arm: the C port of gnark's MultiExp on host cores, SAME size
   python bench.py --workload prove ...      # second metric: synthetic WHIR-verifier-shaped Groth16 prove
+  python bench.py --dump-outputs DIR ...    # also writes the last timed step's result as DIR/<name>.npy
 
 A "step" is one multi-scalar multiplication of 2^logn points (default 2^24, uniform scalars), bases resident in
 HBM.  With N ranks the point range is sharded N ways (strong scaling), each rank runs a local Pippenger, and one
@@ -44,6 +45,16 @@ def rand_fr(rs, n):
     a = rs.integers(0, 1 << 62, size=(n, 4), dtype=np.uint64)
     a[:, 3] &= np.uint64((1 << 60) - 1)        # < 2^252 < r: every row is a valid Montgomery residue
     return a
+
+
+def dump_outputs(dirname, points):
+    """--dump-outputs: each group element (uint64 limbs as the C-ABI returns them: affine x then y, Montgomery form)
+    as DIR/<name>.npy, float64 rows of eight little-endian 32-bit words (exact in float64), one row per base-field
+    coordinate, so that two builds can be compared bit for bit."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, p in points.items():
+        words = np.ascontiguousarray(p, dtype="<u8").view("<u4").reshape(-1, 8)
+        np.save(os.path.join(dirname, f"{name}.npy"), words.astype(np.float64))
 
 
 def load_peaks():
@@ -259,12 +270,13 @@ def to_dev(torch, dev, a, pin=False):
 
 
 # --------------------------------------------------------------------------------------------- prove benchmark
-def prove_bench(ctx, D, rank, L, args, steps, warmup, want_e2e, want_cpu):
+def prove_bench(ctx, D, rank, L, args, steps, warmup, want_e2e, want_cpu, dump_dir=None):
     """Synthetic WHIR-verifier-shaped Groth16 prove of 2^L constraints and as many wires on a known-discrete-log key
     (oracle/synth.py) sharded by point range over the ranks.  Inside the timed region, per step: the BSB22
     Pedersen commitment MSM (gnark runs it inside Solve), the prove (5 MSMs + computeH), the Pedersen
     proof-of-knowledge MSM.  Gate: every MSM output, h, Ar / Bs / Krs, commitment and PoK equal the
-    closed forms computed by the C restatement on rank 0."""
+    closed forms computed by the C restatement on rank 0.  With dump_dir, rank 0 writes the proof, commitment
+    and PoK of the last timed step there."""
     import torch
 
     from gnark_whir_b200 import lib, sharded
@@ -351,11 +363,14 @@ def prove_bench(ctx, D, rank, L, args, steps, warmup, want_e2e, want_cpu):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        step()
+        last = step()[:3]          # not h: the next step's clone must be able to reuse its buffer
     e1.record()
     D.sync_all()
     ms = D.reduce(e0.elapsed_time(e1) / steps, "max")
     launches = ctx.launch_count() - l0
+    if dump_dir and rank == 0:
+        proof, com, pok = last
+        dump_outputs(dump_dir, dict(proof, commitment=com, pok=pok))
     out = {"log2_constraints": L, "wires": N, "committed_wires": nc, "ms": round(ms, 3), "n_gpus": world,
            "window_tables": bool(args.table), "witness_mix": "40% 0/1, 30% bytes, 30% uniform (SURVEY §8d config 1)",
            "timed_region": "Pedersen Commit MSM + Pedersen PoK MSM (b200g16_msm_g1_begin_dev, collected after the prove) + b200g16_prove_dev (5 MSMs, computeH, host assembly); "
@@ -558,7 +573,7 @@ def run_b200(args, rank, local_rank, world):
         "roofline": roofline,
         "roofline_hbm": roofline_hbm,
     }
-    return ctx, D, out, dict(dev=dev, bases=bases, tmad_peak=tmad_peak, acc_ms=acc_ms, m=m, peaks=peaks)
+    return ctx, D, out, dict(dev=dev, bases=bases, tmad_peak=tmad_peak, acc_ms=acc_ms, m=m, peaks=peaks, result=res_a)
 
 
 def extras_single_gpu(ctx, D, st, args):
@@ -670,7 +685,8 @@ def run_prove_workload(args, rank, local_rank, world):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    res = prove_bench(ctx, D, rank, L, args, args.steps, args.warmup, want_e2e=True, want_cpu=not args.no_cpu_baseline)
+    res = prove_bench(ctx, D, rank, L, args, args.steps, args.warmup, want_e2e=True, want_cpu=not args.no_cpu_baseline,
+                      dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
     if rank == 0:
         line = {"metric": "WHIR-verifier-shaped Groth16 prove latency", "value": res["ms"], "unit": "ms",
@@ -712,7 +728,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ncu-traffic", type=float, default=None,
                     help="override: dram bytes per k_accumulate launch (default: newest profiles/*ncu_traffic*.json)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (the MSM "
+                         "point, or the proof, commitment and PoK of --workload prove; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU arm's results (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -729,6 +752,8 @@ def main():
         run_prove_workload(args, rank, local_rank, world)
         return
     ctx, D, out, st = run_b200(args, rank, local_rank, world)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"msm_g1": st["result"]})
     st["bases"].free()
     import torch
     torch.cuda.empty_cache()

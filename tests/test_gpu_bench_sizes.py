@@ -8,15 +8,22 @@
   G2 MSM 2^20         closed form
   NTT 2^22 / 2^24     every output element vs the C port for DIF/DIT x coset x inverse (the 4-column-tile passes of
                       large transforms are only taken at these sizes); computeH 2^22 full output vs the C port
+  bench.py --dump-outputs   (small sizes) the written MSM point, commitment and PoK equal their closed forms
 """
+import os
+import subprocess
+import sys
+
 import numpy as np
 import pytest
 import torch
 
+import bench
 from gnark_whir_b200 import lib
 from oracle import cport, synth
 
 pytestmark = pytest.mark.gpu
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _dev(a):
@@ -92,3 +99,47 @@ def test_compute_h_2p22_full_output_vs_c_port(ctx):
     n = 1 << 22
     a, b, c = synth.rand_fr(rs, n - 3), synth.rand_fr(rs, n - 3), synth.rand_fr(rs, n - 3)      # zero padded to 2^22
     assert np.array_equal(ctx.compute_h(a, b, c, 22), cport.compute_h(a, b, c, 22))
+
+
+def _run_bench(out_dir, *args):
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--no-extras",
+           "--no-cpu-baseline", "--dump-outputs", str(out_dir), *args]
+    out = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-2000:]
+
+
+def _load_point(path, rows):
+    w = np.load(path)
+    assert w.dtype == np.float64 and w.shape == (rows, 8)
+    return w.astype("<u4").view("<u8").reshape(-1).astype(np.uint64)
+
+
+def test_bench_dump_outputs_msm(tmp_path):
+    log2n = 14
+    _run_bench(tmp_path, "--logn", str(log2n))
+    assert sorted(os.listdir(tmp_path)) == ["msm_g1.npy"]
+    rs = np.random.Generator(np.random.PCG64(bench.SEED))       # bench.run_b200's inputs on rank 0
+    ks = bench.rand_fr(rs, 1 << log2n)
+    sc = bench.rand_fr(rs, 1 << log2n)
+    assert np.array_equal(_load_point(tmp_path / "msm_g1.npy", 2), cport.g1_gen_mul(cport.fr_dot(ks, sc)))
+
+
+def test_bench_dump_outputs_prove(tmp_path):
+    L = 10
+    _run_bench(tmp_path, "--workload", "prove", "--prove-logn", str(L))
+    g1 = ["ar", "bs1", "commitment", "krs", "msm_a", "msm_b1", "msm_k", "msm_z", "pok"]
+    assert sorted(os.listdir(tmp_path)) == sorted(f"{n}.npy" for n in g1 + ["bs", "msm_b2"])
+    for n in g1:
+        _load_point(tmp_path / f"{n}.npy", 2)
+    for n in ("bs", "msm_b2"):
+        _load_point(tmp_path / f"{n}.npy", 4)
+    N = 1 << L                                                   # bench.prove_bench's inputs
+    rs = np.random.Generator(np.random.PCG64(bench.SEED + 17 * L))
+    wires = synth.whir_mix(rs, N)
+    for n in (N, N, N, 1, 1):                                    # a, b, c, r, s
+        bench.rand_fr(rs, n)
+    nc = N // 8
+    kc = bench.rand_fr(rs, 2 * nc).reshape(2, nc, 4)
+    committed = wires[1:1 + nc]
+    assert np.array_equal(_load_point(tmp_path / "commitment.npy", 2), cport.g1_gen_mul(cport.fr_dot(kc[0], committed)))
+    assert np.array_equal(_load_point(tmp_path / "pok.npy", 2), cport.g1_gen_mul(cport.fr_dot(kc[1], committed)))
