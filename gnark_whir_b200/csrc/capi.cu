@@ -253,7 +253,7 @@ void b200g16_destroy(b200g16_ctx* ctx) {
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
   cudaStreamSynchronize(ctx->tail_stream);
-  std::vector<DevBuf*> bufs = {&ctx->msm.scalars, &ctx->msm.digits, &ctx->msm.entries, &ctx->ntt.a, &ctx->ntt.b,
+  std::vector<DevBuf*> bufs = {&ctx->msm.scalars, &ctx->msm.part, &ctx->msm.bins, &ctx->msm.entries, &ctx->ntt.a, &ctx->ntt.b,
                                &ctx->ntt.c,       &ctx->ntt.tw,     &ctx->ntt.coset,   &ctx->ntt.fused, &ctx->ntt.dist, &ctx->io_a,  &ctx->io_b,
                                &ctx->io_c};
   for (int i = 0; i < MSM_SETS; i++)

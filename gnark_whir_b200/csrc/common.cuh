@@ -71,7 +71,8 @@ constexpr int AFF_WS_LEVELS = 4;  // = AFF_LEVELS_MAX of msm_affine.cuh (checked
 struct MsmWorkspace {
   // everything the "tail" of an MSM reads (merge of split buckets + bucket reduction) exists MSM_SETS times: the
   // tail runs on a second stream while the next MSMs' sort + accumulate ("front") fill the other sets
-  DevBuf scalars, digits, entries, counts[MSM_SETS], partials[MSM_SETS], chunks[MSM_SETS], misc[MSM_SETS], tasks[MSM_SETS];
+  // part: the (bucket, entry) pairs in coarse-bin order, bins: bin counters and tiles (msm_sort.cuh)
+  DevBuf scalars, part, bins, entries, counts[MSM_SETS], partials[MSM_SETS], chunks[MSM_SETS], misc[MSM_SETS], tasks[MSM_SETS];
   // batched-affine accumulation: level buffers of the pair tree (aff_lvl[l - 1] = inputs of level l), one spill slot per
   // thread.  One set: accumulate kernels of consecutive MSMs are serialised on the main stream.
   DevBuf aff_lvl[AFF_WS_LEVELS], aff_desc, aff_spill, aff_spill_task;
@@ -108,7 +109,7 @@ struct MsmCfg {
   uint32_t nch;   // chunks per window
 };
 
-// The sorted state (digits, entries, counts, offsets, tasks) the last MSM left behind.  A following MSM over
+// The sorted state (entries, counts, offsets, tasks) the last MSM left behind.  A following MSM over
 // the SAME scalar vector and the same decomposition — groth16's Bs1 (G1) right after Bs2 (G2), both over
 // wireValuesB — skips its sort phase and accumulates over these lists with its own bases.
 struct MsmSorted {
@@ -181,6 +182,7 @@ struct b200g16_ctx {
   int msm_affine_levels = 3;    // pair-tree levels at most (1 .. 4)
   uint32_t msm_affine_min_pairs = 192;  // additions per inversion below which a level is not worth running
   uint64_t launches = 0;        // kernels launched by this ctx (bench's gpu_launches)
+  bool sort_smem_set = false;   // k_sort_coarse_part's dynamic shared-memory limit raised on this device
 };
 
 struct b200g16_bases {

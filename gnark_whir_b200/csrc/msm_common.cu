@@ -1,4 +1,4 @@
-// Group-independent front half of the MSM: scalar recoding, histogram, scan, scatter.
+// Group-independent front half of the MSM: scalar recoding and the two-level counting sort (msm_sort.cuh), task table.
 // See msm_impl.cuh for the pipeline overview.
 #include <cstdlib>
 #include "msm_impl.cuh"
@@ -41,13 +41,16 @@ int msm_pick_window(size_t n) {
 }
 
 int msm_pick_table_window(size_t n) {
-  // Measured on B200 with the tree reduction (profiles/r02f_window_sweep.jsonl: whole-MSM device time, uniform
-  // scalars, c = 15..22): 2^18: c = 17 (1.35 ms);  2^19: c = 19 / 20 tie (2.14);  2^20: c = 20 (3.24 against 3.46 at
-  // 19);  2^21: 20 (5.41 / 6.17);  2^22: 20 (9.96 / 11.6);  2^24: 20 (37.7; c = 22 saves 3 ms of additions and loses 4
-  // in the sort and the reduction).  Widths whose TOP window holds only a few scalar bits (c = 18, 19, 21: 2 / 7 / 2
-  // bits) pile every point's top digit into a handful of low buckets of the shared bucket set and pay for it in the
-  // histogram, the scatter and the merge — c = 20 (14 top bits) and c = 17 (16) do not.
+  // Measured on B200 (1000 W, 1965 MHz) with the tree reduction and the two-level sort
+  // (profiles/r03a_window_sweep.jsonl: whole-MSM device time, uniform scalars): 2^20: c = 20 (2.81 ms against 2.95 at 19
+  // and 3.15 at 21);  2^22: 20 (9.36 / 9.60 at 21);  2^24: 22 (33.17 against 35.68 at 20 and 35.35 at 21: 2.4 ms fewer
+  // additions, 0.7 ms more reduction; the sort costs the same at both widths).  Older figures with the one-atomic-per-entry
+  // scatter (profiles/r02f_window_sweep.jsonl): 2^18: c = 17 (1.35 ms);  2^19: c = 19 / 20 tie (2.14);  2^21: 20 (5.41 /
+  // 6.17).  Widths whose TOP window holds only a few scalar bits (c = 18, 19, 21: 2 / 7 / 2 bits) pile every point's top
+  // digit into a handful of low buckets of the shared bucket set and pay for it in the merge of their split buckets
+  // (0.2 - 0.4 ms against 0.05) — c = 22 (12 top bits), 20 (14) and 17 (16) do not.
   auto fits = [&](int c) { return (double)n * msm_num_windows(c) < 2.0e9; };
+  if (n >= ((size_t)1 << 24) && fits(22)) return 22;
   if (n >= ((size_t)3 << 17) && fits(20)) return 20;
   int best = 8;
   double best_cost = 1e300;
@@ -61,66 +64,100 @@ int msm_pick_table_window(size_t n) {
 }
 
 // ------------------------------------------------------------------------------ kernels
-// Window 0 is where small witness values (bits, bytes) pile up — 20% of a WHIR-verifier witness is
-// the scalar 1, i.e. one bucket — and the top window may hold only a few scalar bits (2 bits at
-// c = 18), i.e. a handful of buckets; the histogram / scatter atomics of those two windows are
-// warp-aggregated (match.any: one atomic per distinct bucket per warp).  The windows in between
-// see near-uniform digits and use plain atomics.
-__global__ void __launch_bounds__(256) k_digits(const Fr* __restrict__ scalars, uint32_t n, int c, int W,
-                                                 uint32_t bstride, int32_t* __restrict__ digits,
-                                                 uint32_t* __restrict__ counts, uint32_t* __restrict__ totals) {
-  __shared__ uint32_t s_nz[8];
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t lane = threadIdx.x & 31;
-  const bool valid = i < n;
-  uint32_t limbs[9];
-#pragma unroll
-  for (int k = 0; k < 9; k++) limbs[k] = 0;
-  if (valid) {
-    Fr s = Fr::from_mont(scalars[i]);
-#pragma unroll
-    for (int k = 0; k < 8; k++) limbs[k] = s.l[k];
-  }
-  const uint32_t mask = (c == 32) ? 0xffffffffu : ((1u << c) - 1u);
-  const uint32_t half = 1u << (c - 1);
-  uint32_t carry = 0, nz = 0;
-  for (int w = 0; w < W; w++) {
-    int bit = w * c;
-    int q = bit >> 5, r = bit & 31;
-    uint32_t raw = 0;
-    if (q < 8) {
-      uint64_t two = (uint64_t)limbs[q] | ((uint64_t)limbs[q + 1] << 32);
-      raw = (uint32_t)(two >> r) & mask;
-    }
-    raw += carry;
-    int32_t d;
-    if (raw >= half) { d = (int32_t)raw - (int32_t)(1u << c); carry = 1; }
-    else { d = (int32_t)raw; carry = 0; }
-    if (valid) digits[(size_t)w * n + i] = d;
-    const bool hit = d != 0;
-    const uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
-    if (w == 0 || w == W - 1) {
-      const unsigned active = __ballot_sync(0xffffffffu, hit);
-      if (hit) {
-        const uint32_t key = (uint32_t)w * bstride + mag - 1;
-        const unsigned peers = __match_any_sync(active, key);
-        if ((int)lane == __ffs(peers) - 1) atomicAdd(&counts[key], (uint32_t)__popc(peers));
-      }
-    } else if (hit) {
-      atomicAdd(&counts[(uint32_t)w * bstride + mag - 1], 1u);
-    }
-    nz += hit ? 1u : 0u;
-  }
-  // number of (window, point) entries this launch produces -> totals[3] (drives the task size)
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) nz += __shfl_down_sync(0xffffffffu, nz, off);
-  if (lane == 0) s_nz[threadIdx.x >> 5] = nz;
+// The two-level counting sort (msm_sort.cuh): each kernel runs the header's steps thread by thread between barriers.
+
+// pass 1: coarse count.  s[SORT_BINS] counts the CTA's entries (-> totals[3], which drives the task size)
+__global__ void __launch_bounds__(SORT_CTA) k_sort_coarse_count(const SortArgs A) {
+  __shared__ uint32_t s[SORT_BINS + 1];
+  sort_coarse_init(A, threadIdx.x, s);
   __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t t = 0;
-    for (int k = 0; k < 8; k++) t += s_nz[k];
-    if (t) atomicAdd(&totals[3], t);
+  sort_coarse_count(A, blockIdx.x, threadIdx.x, s);
+  __syncthreads();
+  sort_coarse_flush(A, threadIdx.x, s);
+}
+
+// in-place exclusive scan of s[0, N) by SORT_CTA threads (N / SORT_CTA words each); the total goes to s[N]
+template <uint32_t N>
+__device__ void sort_block_scan(uint32_t* s) {
+  constexpr uint32_t PER = N / SORT_CTA;
+  __shared__ uint32_t wsum[SORT_CTA / 32];
+  const uint32_t t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  uint32_t a = 0;
+#pragma unroll
+  for (uint32_t j = 0; j < PER; j++) a += s[t * PER + j];
+  uint32_t ia = a;
+#pragma unroll
+  for (int off = 1; off < 32; off <<= 1) {
+    const uint32_t x = __shfl_up_sync(0xffffffffu, ia, off);
+    if (lane >= (uint32_t)off) ia += x;
   }
+  if (lane == 31) wsum[warp] = ia;
+  __syncthreads();
+  uint32_t e = ia - a;
+  for (uint32_t w = 0; w < warp; w++) e += wsum[w];
+#pragma unroll
+  for (uint32_t j = 0; j < PER; j++) {
+    const uint32_t k = t * PER + j, v = s[k];
+    s[k] = e;
+    e += v;
+  }
+  if (t == SORT_CTA - 1) s[N] = e;
+  __syncthreads();
+}
+
+// pass 2, one CTA: exclusive scans of the bins' entries and tiles, then bin offsets and the tile list
+__global__ void __launch_bounds__(SORT_CTA) k_sort_bins(const SortArgs A) {
+  __shared__ uint32_t sa[SORT_BINS + 1], sb[SORT_BINS + 1];
+  sort_bins_load(A, threadIdx.x, sa, sb);
+  __syncthreads();
+  sort_block_scan<SORT_BINS>(sa);
+  sort_block_scan<SORT_BINS>(sb);
+  sort_bins_write(A, threadIdx.x, sa, sb);
+}
+
+// pass 3: coarse partition into part[] (bin order), staged in dynamic shared memory (sort_part_smem bytes)
+__global__ void __launch_bounds__(SORT_CTA) k_sort_coarse_part(const SortArgs A) {
+  extern __shared__ __align__(8) unsigned char sort_smem[];
+  SortItem* stage = reinterpret_cast<SortItem*>(sort_smem);
+  uint32_t* s = reinterpret_cast<uint32_t*>(stage + SORT_STAGE);
+  uint32_t* loc = s + SORT_BINS + 1;
+  uint32_t* glob = loc + SORT_BINS;
+  for (uint32_t b = threadIdx.x; b < SORT_BINS; b += SORT_CTA) s[b] = 0;
+  __syncthreads();
+  sort_part_count(A, blockIdx.x, threadIdx.x, s);
+  __syncthreads();
+  sort_block_scan<SORT_BINS>(s);
+  sort_part_reserve(A, threadIdx.x, s, loc, glob);
+  __syncthreads();
+  sort_part_stage(A, blockIdx.x, threadIdx.x, s, stage);
+  __syncthreads();
+  sort_part_write(A, threadIdx.x, s[SORT_BINS], loc, glob, stage);
+}
+
+// pass 4: fine count, one CTA per tile (the grid is an upper bound on the tiles)
+__global__ void __launch_bounds__(SORT_CTA) k_sort_fine_count(const SortArgs A) {
+  __shared__ uint32_t s[1u << SORT_FINE_MAX_BITS];
+  if (blockIdx.x >= *A.ntiles) return;   // whole CTA past the last tile
+  const SortSpan sp = sort_tile_span(A, blockIdx.x);
+  sort_fine_init(A, threadIdx.x, s);
+  __syncthreads();
+  sort_fine_count(A, sp, threadIdx.x, s, true);
+  __syncthreads();
+  sort_fine_flush(A, sp, threadIdx.x, s);
+}
+
+// pass 6: fine place into entries[] (bucket order)
+__global__ void __launch_bounds__(SORT_CTA) k_sort_fine_place(const SortArgs A) {
+  __shared__ uint32_t s[1u << SORT_FINE_MAX_BITS];
+  if (blockIdx.x >= *A.ntiles) return;
+  const SortSpan sp = sort_tile_span(A, blockIdx.x);
+  sort_fine_init(A, threadIdx.x, s);
+  __syncthreads();
+  sort_fine_count(A, sp, threadIdx.x, s, false);
+  __syncthreads();
+  sort_fine_reserve(A, sp, threadIdx.x, s);
+  __syncthreads();
+  sort_fine_place(A, sp, threadIdx.x, s);
 }
 
 // task size.  Many buckets (nb >= target / 2): evenly loaded buckets stay one task each (seg = 2 x mean),
@@ -239,38 +276,6 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_apply(const uint32_t* __r
   }
 }
 
-// grid: (ceil(n/256), W) — window-major so that one window's scatter targets (4n bytes) live in L2
-// bstride: bucket-index stride between windows (2^(c-1), or 0 when all windows share one bucket set
-// because the bases carry a window table); entry = index into the (table of) bases
-// = w * ent_stride + ent_off + i.
-__global__ void __launch_bounds__(256) k_scatter(const int32_t* __restrict__ digits, uint32_t n, uint32_t bstride,
-                                                  uint32_t ent_stride, uint32_t ent_off,
-                                                  uint32_t* __restrict__ cursor, uint32_t* __restrict__ entries) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t w = blockIdx.y;
-  const uint32_t lane = threadIdx.x & 31;
-  const int32_t d = i < n ? digits[(size_t)w * n + i] : 0;
-  const bool hit = d != 0;
-  const uint32_t neg = d < 0;
-  const uint32_t mag = neg ? (uint32_t)(-d) : (uint32_t)d;
-  if (w == 0 || w == gridDim.y - 1) {  // warp-aggregated: one atomic per distinct bucket per warp (see k_digits)
-    const unsigned active = __ballot_sync(0xffffffffu, hit);
-    if (hit) {
-      const uint32_t key = w * bstride + mag - 1;
-      const unsigned peers = __match_any_sync(active, key);
-      const int leader = __ffs(peers) - 1;
-      const uint32_t rank = __popc(peers & ((1u << lane) - 1u));
-      uint32_t base = 0;
-      if ((int)lane == leader) base = atomicAdd(&cursor[key], (uint32_t)__popc(peers));
-      base = __shfl_sync(peers, base, leader);
-      entries[base + rank] = ((w * ent_stride + ent_off + i) << 1) | neg;
-    }
-  } else if (hit) {
-    uint32_t pos = atomicAdd(&cursor[w * bstride + mag - 1], 1u);
-    entries[pos] = ((w * ent_stride + ent_off + i) << 1) | neg;
-  }
-}
-
 __global__ void __launch_bounds__(256) k_tasks(const uint32_t* __restrict__ counts, const uint32_t* __restrict__ task_off,
                                                 uint32_t nb, uint32_t* __restrict__ totals,
                                                 uint32_t* __restrict__ task_bucket) {
@@ -367,9 +372,9 @@ __global__ void __launch_bounds__(TASK_CTA) k_task_order(const uint32_t* __restr
   if (valid) task_order[h[bin] + rank] = t;
 }
 
-int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, int32_t* digits,
-                   uint32_t* counts, uint32_t* offsets, uint32_t* cursor, uint32_t* task_off, uint32_t* totals,
-                   uint32_t* entries, uint32_t* task_bucket, uint32_t* task_order, uint32_t max_tasks,
+int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, SortItem* part,
+                   uint32_t* bins, uint32_t* counts, uint32_t* offsets, uint32_t* cursor, uint32_t* task_off,
+                   uint32_t* totals, uint32_t* entries, uint32_t* task_bucket, uint32_t* task_order, uint32_t max_tasks,
                    uint32_t* scan_scratch, int* ev) {
   cudaStream_t st = ctx->stream;
   auto mark = [&]() { if (ev && *ev < 18) cudaEventRecord(ctx->ev[(*ev)++], st); };
@@ -382,15 +387,53 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
   int nt = 0;
   if (trace && !tev_made) { for (auto& e : tev) cudaEventCreate(&e); tev_made = true; }
   auto tr = [&]() { if (trace && nt < 16) cudaEventRecord(tev[nt++], st); };
+  SortArgs A;
+  A.scalars = d_scalars;
+  A.n = n;
+  A.c = cfg.c;
+  A.W = cfg.W;
+  A.bstride = cfg.bstride;
+  A.ent_stride = cfg.ent_stride;
+  A.ent_off = cfg.ent_off;
+  A.F = sort_fine_bits(cfg.nb);
+  A.nbins = sort_num_bins(cfg.nb, A.F);
+  A.part_points = sort_part_points(cfg.W);
+  A.bin_count = bins;
+  A.bin_cursor = bins + SORT_BINS;
+  A.bin_off = bins + 2 * SORT_BINS;
+  A.ntiles = bins + 3 * SORT_BINS + 1;
+  A.tiles = reinterpret_cast<SortTile*>(bins + SORT_BIN_WORDS);
+  A.part = part;
+  // canonical scalars between passes 1 and 3: entries (4 W bytes per point, W >= 11 at every width) is not written
+  // before pass 6
+  static_assert(sizeof(Fr) == 32, "canonical scalar scratch: 32 bytes per point");
+  if (cfg.W < 8) return fail(B200G16_ERR_ARG, "msm sort: W = %d leaves no room for the canonical scalars", cfg.W);
+  A.canon = reinterpret_cast<Fr*>(entries);
+  A.counts = counts;
+  A.cursor = cursor;
+  A.entries = entries;
+  A.totals = totals;
+  const unsigned max_tiles = (unsigned)sort_max_tiles(A.nbins, (size_t)n * cfg.W);
   mark();
   tr();
   B200_CUDA(cudaMemsetAsync(counts, 0, (size_t)cfg.nb * sizeof(uint32_t), st));
   B200_CUDA(cudaMemsetAsync(totals, 0, 16 * sizeof(uint32_t), st));
-  k_digits<<<cdiv(n, 256), 256, 0, st>>>(d_scalars, n, cfg.c, cfg.W, cfg.bstride, digits, counts, totals);
+  B200_CUDA(cudaMemsetAsync(A.bin_count, 0, SORT_BINS * sizeof(uint32_t), st));
+  k_sort_coarse_count<<<cdiv(n, SORT_POINTS), SORT_CTA, 0, st>>>(A);
   tr();
   k_pick_seg<<<1, 1, 0, st>>>(totals, cfg.nb, cfg.target_tasks);
   tr();
   mark();
+  k_sort_bins<<<1, SORT_CTA, 0, st>>>(A);
+  tr();
+  if (!ctx->sort_smem_set) {   // once per context (= device)
+    B200_CUDA(cudaFuncSetAttribute(k_sort_coarse_part, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_part_smem()));
+    ctx->sort_smem_set = true;
+  }
+  k_sort_coarse_part<<<cdiv(n, A.part_points), SORT_CTA, sort_part_smem(), st>>>(A);
+  tr();
+  k_sort_fine_count<<<max_tiles, SORT_CTA, 0, st>>>(A);
+  tr();
   const uint32_t ntiles = cdiv(cfg.nb, SCAN_TILE);
   uint2* tile_sums = reinterpret_cast<uint2*>(scan_scratch);
   uint32_t* hist = scan_scratch + 2 * (size_t)(ntiles + 1);   // 2 x TASK_BINS words after the tile sums
@@ -399,7 +442,7 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
   k_scan_top<<<1, 1024, 0, st>>>(tile_sums, ntiles, totals);
   k_scan_apply<<<ntiles, SCAN_THREADS, 0, st>>>(counts, cfg.nb, totals, tile_sums, offsets, cursor, task_off);
   tr();
-  k_scatter<<<dim3(cdiv(n, 256), cfg.W), 256, 0, st>>>(digits, n, cfg.bstride, cfg.ent_stride, cfg.ent_off, cursor, entries);
+  k_sort_fine_place<<<max_tiles, SORT_CTA, 0, st>>>(A);
   tr();
   k_tasks<<<cdiv(cfg.nb, 256), 256, 0, st>>>(counts, task_off, cfg.nb, totals, task_bucket);
   tr();
@@ -412,9 +455,9 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
   mark();
   if (trace) {
     cudaStreamSynchronize(st);
-    static const char* what[] = {"memsets + k_digits", "k_pick_seg", "scan x3", "k_scatter", "k_tasks", "memset + k_task_hist",
-                                 "k_task_scan + k_task_order"};
-    fprintf(stderr, "[sort trace n=%u c=%d]", n, cfg.c);
+    static const char* what[] = {"memsets + coarse count", "k_pick_seg", "bin scan", "coarse partition", "fine count",
+                                 "scan x3", "fine place", "k_tasks", "memset + k_task_hist", "k_task_scan + k_task_order"};
+    fprintf(stderr, "[sort trace n=%u c=%d F=%d]", n, cfg.c, A.F);
     for (int i = 0; i + 1 < nt; i++) {
       float ms = 0;
       cudaEventElapsedTime(&ms, tev[i], tev[i + 1]);
@@ -422,7 +465,7 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
     }
     fprintf(stderr, "\n");
   }
-  ctx->launches += 10;
+  ctx->launches += 13;
   B200_CUDA(cudaGetLastError());
   return 0;
 }

@@ -6,13 +6,12 @@
 // /root/reference/mt.go:496.  Only the result (the group element, in affine normal form) is
 // observable at that boundary, so the decomposition below is B200-first, not gnark's:
 //
-//   k_digits      scalar Montgomery->canonical, signed c-bit digits (partitionScalars' job),
-//                 per-(window,bucket) histogram
+//   k_sort_*      scalar Montgomery->canonical, signed c-bit digits (partitionScalars' job), and a two-level
+//                 counting sort of the (window, point) entries into bucket order: coarse bins (bucket >> F), then
+//                 the buckets inside each bin, one atomic per CTA and bin or bucket (msm_sort.cuh)
 //   k_scan_*      exclusive scan of the histogram -> entry offsets; buckets larger than `seg`
 //                 are split into several tasks (0/1-heavy witnesses put millions of points in
 //                 bucket "1" of window 0) -> task offsets
-//   k_scatter     window-major counting-sort scatter of (entry index, sign) into bucket order;
-//                 one window's 4n bytes of targets stay resident in the 126 MB L2
 //   k_tasks, k_task_*  task -> bucket table; tasks ordered by length so a warp's lanes finish together
 //   k_accumulate  one thread per task: gathers its affine points with 128-bit loads, mixed
 //                 XYZZ adds (10 modmul) on the integer pipe; next point prefetched during the add
@@ -30,6 +29,7 @@
 
 #include "common.cuh"
 #include "ec.cuh"
+#include "msm_sort.cuh"
 
 namespace b200 {
 
@@ -38,10 +38,11 @@ namespace b200 {
 // msm_common.cu
 int msm_num_windows(int c);
 int msm_pick_window(size_t n);
-// digits + histogram + scan + scatter + task table on ctx->stream (4 kernels + 1 memset)
-int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, int32_t* digits,
-                   uint32_t* counts, uint32_t* offsets, uint32_t* cursor, uint32_t* task_off, uint32_t* totals,
-                   uint32_t* entries, uint32_t* task_bucket, uint32_t* task_order, uint32_t max_tasks,
+// two-level counting sort into bucket order + task table on ctx->stream (13 kernels + 4 memsets).
+// part: n * W items; bins: sort_bin_bytes(bins, n * W) bytes
+int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, SortItem* part,
+                   uint32_t* bins, uint32_t* counts, uint32_t* offsets, uint32_t* cursor, uint32_t* task_off,
+                   uint32_t* totals, uint32_t* entries, uint32_t* task_bucket, uint32_t* task_order, uint32_t max_tasks,
                    uint32_t* scan_scratch, int* ev);
 
 static inline unsigned cdiv(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
@@ -342,7 +343,9 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
                      ls.c == cfg.c && ls.bstride == cfg.bstride && ls.ent_stride == cfg.ent_stride &&
                      ls.ent_off == cfg.ent_off;
   const int spar = reuse ? ls.par : par;  // set holding the sorted state: counts, offsets, tasks, totals
-  B200_TRY(ws.digits.ensure(m_max * sizeof(int32_t)));
+  const int sort_F = sort_fine_bits(cfg.nb);
+  B200_TRY(ws.part.ensure(m_max * sizeof(SortItem)));
+  B200_TRY(ws.bins.ensure(sort_bin_bytes(sort_num_bins(cfg.nb, sort_F), m_max)));
   B200_TRY(ws.entries.ensure(m_max * sizeof(uint32_t)));
   // totals[16] + two lists of split buckets [nb each] + scan tile sums (uint2 per 2048 buckets, 8-byte aligned)
   const size_t scan_off = (64 + 2 * (size_t)cfg.nb * sizeof(uint32_t) + 7) & ~(size_t)7;
@@ -369,7 +372,7 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
   uint32_t* cursor = offsets + cfg.nb;
   uint32_t* task_off = cursor + cfg.nb;
   uint32_t* totals = ws.misc[spar].as<uint32_t>();
-  int32_t* digits = ws.digits.as<int32_t>();
+  SortItem* part = ws.part.as<SortItem>();
   uint32_t* entries = ws.entries.as<uint32_t>();
   uint32_t* task_bucket = ws.tasks[spar].as<uint32_t>();
   uint32_t* task_order = task_bucket + max_tasks;
@@ -390,7 +393,7 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
     if (rd >= 0 && ctx->tail_pending[rd]) B200_CUDA(cudaStreamWaitEvent(st, ctx->ev_tail[rd], 0));
     ctx->sort_reader[par] = -1;
     ctx->last_sort.valid = false;
-    B200_TRY(msm_sort_phase(ctx, cfg, d_scalars, n32, digits, counts, offsets, cursor, task_off, totals, entries,
+    B200_TRY(msm_sort_phase(ctx, cfg, d_scalars, n32, part, ws.bins.as<uint32_t>(), counts, offsets, cursor, task_off, totals, entries,
                             task_bucket, task_order, (uint32_t)max_tasks,
                             reinterpret_cast<uint32_t*>(ws.misc[par].as<char>() + scan_off),
                             record_events ? &ev : nullptr));

@@ -48,7 +48,8 @@ def window_sweep(ctx):
     """Table-mode window width per (shard) size: whole-MSM device time for c = 15..21 at 2^18..2^22 (the per-GPU shard
     sizes of an 8-way sharded 2^21..2^24 job), uniform scalars.  Feeds msm_pick_table_window."""
     gen = g16.g1_point(g16.G1_GEN)
-    for logn in (18, 19, 20, 21, 22, 24):
+    arg = [a for a in sys.argv if a.startswith("--logs=")]
+    for logn in ([int(x) for x in arg[0][7:].split(",")] if arg else (18, 19, 20, 21, 22, 24)):
         n = 1 << logn
         ks = rand_fr(n)
         sc = torch.from_numpy(rand_fr(n).view(np.int64)).cuda()
@@ -299,6 +300,9 @@ def main():
                      Mpts_s=round(n / ms / 1e3, 2), phases_ms=[round(x, 3) for x in best], bit_exact_vs_oracle=ok)
             bases.free()
             del d_uni, d_mix
+    if "--msm" in sys.argv:     # the MSM section alone
+        ctx.close()
+        return
 
     # ---- NTT / computeH sweeps
     for logn in ([18, 20, 22, 24, 26] if big else [18, 20, 22, 24]):
