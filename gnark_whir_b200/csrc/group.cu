@@ -329,6 +329,16 @@ static int group_prove_dist(b200g16_group* g, const b200g16_group_pk* gpk, const
     // ---- allocate / publish slices
     int st = [&]() -> int {
       B200_CUDA(cudaSetDevice(ctx->device));
+      DistH& D = ctx->dist_h;
+      bool mapped = false;
+      for (int v = 0; v < 3; v++)
+        for (int d = 0; d < 8; d++) mapped = mapped || D.ipc_opened[v][d];
+      if (D.g && !mapped && (D.L != L || D.g != gl || D.me != i)) {
+        // a key of another size: the previous prove ended with a stream sync and a barrier, and the peer pointers
+        // are taken again after the next barrier, so nobody reads these slices any more
+        for (int v = 0; v < 3; v++) D.slice[v].release();
+        D = DistH();
+      }
       return dist_h_alloc(ctx, (unsigned)L, n, i);
     }();
     st = bar.arrive(st);

@@ -431,7 +431,9 @@ void b200g16_group_pk_free(b200g16_group_pk* pk);
  * a, b, c are uploaded to up to three devices (one vector each: iNTT + coset NTT there), the root device
  * receives the other two by peer copies, finishes h and every device fetches its slice of h by one peer copy
  * (cudaMemcpyPeerAsync over NVLink); the five MSMs run on every device's shard and the n x 5 partial points
- * are added on the host. */
+ * are added on the host.  With 2, 4 or 8 devices and log2 N >= 2 log2(n) + 1, computeH is split over all the
+ * devices instead (as b200g16_dist_h_* below, over peer pointers).  A group may prove keys of different sizes one
+ * after another: the split computeH's slices are set up again when the domain size changes. */
 int b200g16_group_prove(b200g16_group* g, const b200g16_group_pk* pk, const uint64_t* wires, size_t n_wires,
                         const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints,
                         const uint64_t r[4], const uint64_t s[4], b200g16_proof* proof_out, uint64_t* h_out);
@@ -441,7 +443,9 @@ int b200g16_group_prove(b200g16_group* g, const b200g16_group_pk* pk, const uint
  * [me M, (me + 1) M), M = 2^log2n / n_peers, of a, b, c (zero padded) in three slice buffers owned by the library.
  * The levels of every transform whose partner lies on another GPU run as kernels over CUDA-IPC mapped peer
  * memory (NVLink loads / stores, no collective library); all other levels are ordinary size-M passes.
- *   init   allocates the slices, returns their 3 x 64-byte IPC handles (exchange them: e.g. all_gather)
+ *   init   allocates the slices, returns their 3 x 64-byte IPC handles (exchange them: e.g. all_gather); on a
+ *          context already set up for another shape it fails with B200G16_ERR_STATE (peers may hold mapped
+ *          handles of the old slices): close first
  *   open   maps every peer's slices (all_handles = n_peers x 3 x 64 bytes, rank-major)
  *   load   copies this rank's slices of a, b, c (device pointers, M elements each) into the slice buffers
  *   slice  device pointer of the local slice of a (0), b (1), c (2) (to write the inputs in place instead)

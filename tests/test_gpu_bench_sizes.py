@@ -6,8 +6,8 @@
                       (rotating MSM buffer sets, Bs1 reusing Bs2's sorted lists while its tail still runs,
                       a / b / c arriving on the copy stream), WHIR-shaped witness          /root/reference/mt.go:496
   G2 MSM 2^20         closed form
-  NTT 2^22 / 2^24     every output element vs the C port for DIF/DIT x coset x inverse (the 4-column-tile passes of
-                      large transforms are only taken at these sizes); computeH 2^22 full output vs the C port
+  NTT 2^22 / 2^24     every output element vs the C port for DIF/DIT x coset x inverse (3 passes of 2-column tiles,
+                      8+7+7 and 8+8+8 levels); computeH 2^22 full output vs the C port
   bench.py --dump-outputs   (small sizes) the written MSM point, commitment and PoK equal their closed forms
 """
 import os
