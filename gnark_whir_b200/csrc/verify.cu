@@ -55,8 +55,9 @@ __global__ void __launch_bounds__(PAIR_THREADS) k_pairing_products(const G1Affin
 }
 
 // n_prod products over pairs laid out back to back; host arrays, device scratch in ctx->io_c
-static int pairing_products(b200g16_ctx* ctx, const G1Affine* P, const G2Affine* Q, const uint32_t* flags,
-                            const uint32_t* first, int n_prod, bool with_cofactor, Fp12* gt, int* is_one, int* valid) {
+// (also the per-proof fallback of b200g16_verify_batch, verify_batch.cu)
+int pairing_products(b200g16_ctx* ctx, const G1Affine* P, const G2Affine* Q, const uint32_t* flags,
+                     const uint32_t* first, int n_prod, bool with_cofactor, Fp12* gt, int* is_one, int* valid) {
   const size_t n = first[n_prod];
   auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
   const size_t o_q = up(n * sizeof(G1Affine)), o_fl = o_q + up(n * sizeof(G2Affine)), o_first = o_fl + up(n * 4),

@@ -12,6 +12,7 @@ restated.  What runs where:
           GPU : Pedersen commit + PoK (b200g16_msm_g1), computeH, the five MSMs, via b200g16_prove
   Verify  host: the BSB22 challenge hash
           GPU : public-input MSM, Pedersen PoK check and the pairing product, via b200g16_verify
+  BatchVerify  k proofs of one circuit in one b200g16_verify_batch call (small-exponent batch test)
   wire formats (gnark / gnark-crypto marshal.go): Proof, VerifyingKey, ProvingKey, fft.Domain; the point encodings run
           batched on the GPU (b200g16_g1/g2_encode / _decode)
 
@@ -539,11 +540,9 @@ def Prove(ctx, r1cs, pk, witness, r=None, s=None, resolve=None, want_h=False):
     return Proof(out["ar"], out["krs"], out["bs"], proof_commitments, pok, dbg)
 
 
-def Verify(ctx, proof, vk, public_witness):
-    """groth16.Verify(proof, vk, publicWitness) -> None, raises on an invalid proof (gnark returns
-    an error).  public_witness: values of the public wires WITHOUT the constant-one wire, as in
-    gnark's witness.Public().  Runs b200g16_verify: the public-input MSM and the pairing product
-    on the GPU; only the BSB22 challenge hash (SHA-256 over ~100 bytes) is computed here."""
+def _verify_inputs(proof, vk, public_witness):
+    """The public inputs b200g16_verify takes for one proof (the public witness, then the BSB22 challenge when the
+    circuit has a commitment) and the proof's commitment and proof of knowledge (None without one)."""
     pub = [int(v) % R_MOD for v in public_witness]
     com = pok = None
     if vk.has_commitment:
@@ -553,9 +552,64 @@ def Verify(ctx, proof, vk, public_witness):
         # PublicAndCommitmentCommitted holds wire indexes (wire 0 = the constant one)
         committed = [1 if i == 0 else pub[i - 1] for i in vk.PublicAndCommitmentCommitted]
         pub.append(commitment_challenge(com, committed))
+    return pub, com, pok
+
+
+def Verify(ctx, proof, vk, public_witness):
+    """groth16.Verify(proof, vk, publicWitness) -> None, raises on an invalid proof (gnark returns
+    an error).  public_witness: values of the public wires WITHOUT the constant-one wire, as in
+    gnark's witness.Public().  Runs b200g16_verify: the public-input MSM and the pairing product
+    on the GPU; only the BSB22 challenge hash (SHA-256 over ~100 bytes) is computed here."""
+    pub, com, pok = _verify_inputs(proof, vk, public_witness)
     ok = ctx.verify(vk.G1_Alpha, vk.G2_Beta, vk.G2_Gamma, vk.G2_Delta, vk.G1_K, proof.Ar, proof.Bs, proof.Krs,
                     fr_array(pub) if pub else np.zeros((0, 4), dtype=np.uint64), commitment=com, pok=pok,
                     ped_g=vk.PedersenG if vk.has_commitment else None,
                     ped_g_sigma_neg=vk.PedersenGSigmaNeg if vk.has_commitment else None)
     if not ok:
         raise ValueError("groth16.Verify: pairing check failed")
+
+
+def BatchVerify(ctx, proofs, vk, public_witnesses, coeffs=None):
+    """Verify k proofs of one circuit in one call (b200g16_verify_batch) -> list of k bools, each equal to what
+    Verify decides for that proof alone.  public_witnesses[i] is proof i's public witness, as Verify takes it.
+
+    coeffs: k nonzero integers < 2^128 (then k more with a commitment) for the small-exponent batch test.  They must be
+    unpredictable to whoever made the proofs; by default they are drawn with secrets.randbits(128).  Passing them
+    makes a run reproducible, like r and s in Prove.  Malformed input raises as in Verify."""
+    k = len(proofs)
+    if len(public_witnesses) != k:
+        raise ValueError("groth16.BatchVerify: %d proofs but %d public witnesses" % (k, len(public_witnesses)))
+    n_coef = 2 * k if vk.has_commitment else k
+    if coeffs is None:
+        coeffs = []
+        while len(coeffs) < n_coef:
+            c = secrets.randbits(128)
+            if c:
+                coeffs.append(c)
+    if len(coeffs) != n_coef:
+        raise ValueError("groth16.BatchVerify: %d coefficients, expected %d" % (len(coeffs), n_coef))
+    if any(not 0 < int(c) < 1 << 128 for c in coeffs):
+        raise ValueError("groth16.BatchVerify: coefficients must be nonzero and below 2^128")
+    co = np.array([(int(c) & _M64, int(c) >> 64) for c in coeffs], dtype=np.uint64).reshape(-1, 2)
+    n_pub = len(vk.G1_K) - 1
+    pubs = np.zeros((k, n_pub, 4), dtype=np.uint64)
+    coms, poks = [], []
+    for i, (proof, pw) in enumerate(zip(proofs, public_witnesses)):
+        pub, com, pok = _verify_inputs(proof, vk, pw)
+        if len(pub) != n_pub:
+            raise lib.B200Error("groth16.BatchVerify: proof %d has %d public inputs, vk.G1.K expects %d"
+                                % (i, len(pub), n_pub))
+        if pub:
+            pubs[i] = fr_array(pub)
+        coms.append(com)
+        poks.append(pok)
+    stack = lambda pts, w: np.array([np.asarray(p, dtype=np.uint64).reshape(w) for p in pts],
+                                    dtype=np.uint64).reshape(k, w)
+    _, each = ctx.verify_batch(vk.G1_Alpha, vk.G2_Beta, vk.G2_Gamma, vk.G2_Delta, vk.G1_K,
+                               stack([p.Ar for p in proofs], 8), stack([p.Bs for p in proofs], 16),
+                               stack([p.Krs for p in proofs], 8), pubs, co,
+                               commitments=stack(coms, 8) if vk.has_commitment else None,
+                               poks=stack(poks, 8) if vk.has_commitment else None,
+                               ped_g=vk.PedersenG if vk.has_commitment else None,
+                               ped_g_sigma_neg=vk.PedersenGSigmaNeg if vk.has_commitment else None)
+    return [bool(x) for x in each]

@@ -80,6 +80,7 @@ SIGNATURES = {
     "b200g16_pairing_check": (C.c_int, [_vp, _vp, _vp, _sz, C.POINTER(C.c_int)]),
     "b200g16_pair": (C.c_int, [_vp, _vp, _vp, _sz, _vp]),
     "b200g16_verify": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(C.c_int)]),
+    "b200g16_verify_batch": (C.c_int, [_vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, C.POINTER(C.c_int), _vp]),
     "b200g16_g1_decode": (C.c_int, [_vp, _vp, _sz, C.c_int, _vp, _vp]),
     "b200g16_g2_decode": (C.c_int, [_vp, _vp, _sz, C.c_int, C.c_int, _vp, _vp]),
     "b200g16_g1_encode": (C.c_int, [_vp, _vp, _sz, C.c_int, _vp]),
@@ -202,6 +203,18 @@ class VkDesc(C.Structure):
     """struct b200g16_vk_desc (include/b200g16.h)"""
     _fields_ = [("g1_alpha", _vp), ("g2_beta", _vp), ("g2_gamma", _vp), ("g2_delta", _vp), ("g1_k", _vp), ("n_k", _sz),
                 ("ped_g", _vp), ("ped_g_sigma_neg", _vp)]
+
+
+def _vk_desc(alpha, beta2, gamma2, delta2, K, ped_g, ped_g_sigma_neg):
+    """struct b200g16_vk_desc from numpy points -> (desc, arrays to keep alive during the call)"""
+    keep = [_u64(alpha).reshape(8), _u64(beta2).reshape(16), _u64(gamma2).reshape(16), _u64(delta2).reshape(16),
+            _u64(K, 8)] + [None if v is None else _u64(v).reshape(16) for v in (ped_g, ped_g_sigma_neg)]
+    d = VkDesc()
+    d.g1_alpha, d.g2_beta, d.g2_gamma, d.g2_delta, d.g1_k = [_ptr(a) for a in keep[:5]]
+    d.n_k = keep[4].shape[0]
+    d.ped_g = _ptr(keep[5]) if keep[5] is not None else None
+    d.ped_g_sigma_neg = _ptr(keep[6]) if keep[6] is not None else None
+    return d, keep
 
 
 class ProofOut(C.Structure):
@@ -567,23 +580,44 @@ class Context:
 
     def verify(self, alpha, beta2, gamma2, delta2, K, ar, bs, krs, public_inputs, commitment=None, pok=None,
                ped_g=None, ped_g_sigma_neg=None):
-        keep = [_u64(alpha).reshape(8), _u64(beta2).reshape(16), _u64(gamma2).reshape(16), _u64(delta2).reshape(16),
-                _u64(K, 8)]
-        d = VkDesc()
-        d.g1_alpha, d.g2_beta, d.g2_gamma, d.g2_delta, d.g1_k = [_ptr(a) for a in keep]
-        d.n_k = keep[4].shape[0]
-        opt = [None if v is None else _u64(v).reshape(w) for v, w in ((ped_g, 16), (ped_g_sigma_neg, 16),
-                                                                        (commitment, 8), (pok, 8))]
-        d.ped_g = _ptr(opt[0]) if opt[0] is not None else None
-        d.ped_g_sigma_neg = _ptr(opt[1]) if opt[1] is not None else None
+        d, keep = _vk_desc(alpha, beta2, gamma2, delta2, K, ped_g, ped_g_sigma_neg)
+        opt = [None if v is None else _u64(v).reshape(w) for v, w in ((commitment, 8), (pok, 8))]
         pts = [_u64(ar).reshape(8), _u64(bs).reshape(16), _u64(krs).reshape(8)]
         pub = _u64(public_inputs, 4)
         ok = C.c_int()
         _check(load().b200g16_verify(self.h, C.byref(d), _ptr(pts[0]), _ptr(pts[1]), _ptr(pts[2]),
-                                     _ptr(opt[2]) if opt[2] is not None else None,
-                                     _ptr(opt[3]) if opt[3] is not None else None,
+                                     _ptr(opt[0]) if opt[0] is not None else None,
+                                     _ptr(opt[1]) if opt[1] is not None else None,
                                      _ptr(pub) if pub.shape[0] else None, pub.shape[0], C.byref(ok)))
         return bool(ok.value)
+
+    def verify_batch(self, alpha, beta2, gamma2, delta2, K, ar, bs, krs, public_inputs, coeffs, commitments=None,
+                     poks=None, ped_g=None, ped_g_sigma_neg=None, want_each=True):
+        """b200g16_verify_batch: k proofs against one vk.  ar (k,8), bs (k,16), krs (k,8), public_inputs (k, n_public, 4)
+        Montgomery, coeffs (k or 2k, 2) 128-bit little-endian (rho, then tau with commitments), commitments / poks
+        (k,8) or None.  -> (ok_all, ok_each (k,) bool or None)"""
+        d, keep = _vk_desc(alpha, beta2, gamma2, delta2, K, ped_g, ped_g_sigma_neg)
+        ar, bs, krs = _u64(ar, 8), _u64(bs, 16), _u64(krs, 8)
+        k = ar.shape[0]
+        if bs.shape[0] != k or krs.shape[0] != k:
+            raise B200Error("verify_batch: Ar, Bs, Krs differ in length")
+        pub = np.ascontiguousarray(public_inputs, dtype=np.uint64)
+        if pub.ndim != 3:
+            pub = pub.reshape(k, -1, 4) if pub.size else np.zeros((k, 0, 4), dtype=np.uint64)
+        if pub.shape[0] != k:
+            raise B200Error("verify_batch: public inputs for %d proofs, %d proofs given" % (pub.shape[0], k))
+        co = _u64(coeffs, 2)
+        com = None if commitments is None else _u64(commitments, 8)
+        pk_ = None if poks is None else _u64(poks, 8)
+        if co.shape[0] != (2 * k if com is not None else k) or any(a is not None and a.shape[0] != k for a in (com, pk_)):
+            raise B200Error("verify_batch: coefficient / commitment / pok count does not match the proofs")
+        ok = C.c_int()
+        each = np.zeros(k, dtype=np.uint8) if want_each else None
+        _check(load().b200g16_verify_batch(
+            self.h, C.byref(d), k, _ptr(ar), _ptr(bs), _ptr(krs), _ptr(com) if com is not None else None,
+            _ptr(pk_) if pk_ is not None else None, _ptr(pub) if pub.size else None, pub.shape[1],
+            _ptr(co), C.byref(ok), _ptr(each) if want_each and k else None))
+        return bool(ok.value), (each.astype(bool) if want_each else None)
 
     # -- gnark-crypto point encodings (G1Affine.Bytes / RawBytes / SetBytes and the G2 counterparts)
     def encode_points(self, points, group=1, raw=False):

@@ -353,6 +353,32 @@ int b200g16_pair(b200g16_ctx* ctx, const uint64_t* g1_points, const uint64_t* g2
 int b200g16_verify(b200g16_ctx* ctx, const b200g16_vk_desc* vk, const uint64_t ar[8], const uint64_t bs[16],
                    const uint64_t krs[8], const uint64_t* commitment, const uint64_t* commitment_pok,
                    const uint64_t* public_inputs, size_t n_public, int* ok_out);
+/* k proofs against one verifying key in one call: the small-exponent batch test (Bellare-Garay-Rabin).  With
+ * coefficients rho_i (and, with commitments, independent tau_i for the proofs of knowledge) the batch is accepted iff
+ * every proof point is valid (as b200g16_verify checks them) and
+ *   prod_i e(rho_i Ar_i, Bs_i) e(-S alpha, beta) e(-(S K_0 + sum_j y_j K_j + sum_i rho_i D_i), gamma)
+ *     e(-sum_i rho_i Krs_i, delta) e(sum_i tau_i D_i, GSigmaNeg) e(sum_i tau_i P_i, G) == 1,
+ *   S = sum_i rho_i, y_j = sum_i rho_i x_ij (mod r):
+ * k + 3 (k + 5) Miller loops, one per proof on its own GPU thread, and one final exponentiation.
+ *   ar, bs, krs   : k x 8 / 16 / 8 words (Proof.Ar, Bs, Krs), back to back
+ *   commitments, poks : k x 8 words each (Proof.Commitments[0], CommitmentPok), or both NULL; given exactly when
+ *                   the vk carries the Pedersen keys
+ *   public_inputs : k x n_public fr.Elements, proof i's laid out as b200g16_verify takes them (n_public + 1 == n_k)
+ *   coeffs        : 128-bit little-endian integers, 2 words each: k rho_i, then (with commitments) k tau_i; nonzero
+ *   ok_each       : k bytes or NULL.  All 1 when the batch passes; otherwise ok_each[i] is exactly b200g16_verify's
+ *                   answer for proof i, from a per-proof pass on the GPU (costs about one b200g16_verify call, more
+ *                   for large k: DESIGN.md section 6)
+ * SOUNDNESS: the coefficients must be unpredictable to whoever produced the proofs (draw them from a CSPRNG after
+ * the proofs are fixed).  Then a batch holding an invalid proof passes with probability about 2^-128; with
+ * predictable coefficients a forger can make invalid proofs cancel each other.
+ * Errors (B200G16_ERR_ARG) as b200g16_verify, plus: a zero coefficient, k > 2^20, commitments without poks or
+ * Pedersen keys or the reverse.  k = 0 accepts.  B200G16_ERR_STATE while a split prove is open.  Uses the ctx's MSM
+ * scratch; the ctx stays fully usable.  b200g16_last_timings: upload, per-proof kernel, fold + MSMs, fixed pairs +
+ * product tree, final exponentiation[, per-proof pass]. */
+int b200g16_verify_batch(b200g16_ctx* ctx, const b200g16_vk_desc* vk, size_t k, const uint64_t* ar,
+                         const uint64_t* bs, const uint64_t* krs, const uint64_t* commitments, const uint64_t* poks,
+                         const uint64_t* public_inputs, size_t n_public, const uint64_t* coeffs, int* ok_out,
+                         uint8_t* ok_each);
 
 /* b200g16_prove_dev with computeH already done: d_h holds h (N elements, bit-reversed order, as
  * b200g16_compute_h_dev leaves it in d_a). */
