@@ -27,6 +27,10 @@ int sponge_batch_device(b200g16_ctx* ctx, const uint8_t* d_in, size_t in_len, si
 int merkle_paths_device(b200g16_ctx* ctx, const uint8_t* d_leaves, size_t leaf_len, const uint64_t* d_sib,
                         const uint64_t* d_auth, const uint64_t* d_idx, unsigned height, size_t n,
                         const uint64_t* d_expected_root, uint64_t* d_roots, uint8_t* d_ok);
+int keccak_duplex_device(b200g16_ctx* ctx, uint64_t* d_digests, size_t n, const uint8_t* tag, size_t tag_len,
+                         const b200g16_duplex_op* d_ops, size_t n_ops, const uint8_t* d_in, size_t in_stride,
+                         uint8_t* d_out, size_t out_stride);
+int keccak_duplex_check_device(b200g16_ctx* ctx, const uint64_t* d_digests, size_t n, uint32_t* d_flag, bool* bad);
 
 // out[i] = k_i * base; result either copied to the host (out_host) or kept as a new bases handle
 template <class F>
@@ -554,6 +558,79 @@ int b200g16_keccak_sponge_batch(b200g16_ctx* ctx, const uint8_t* inputs, size_t 
   if (in_len) B200_TRY(h2d_copy(ctx, ctx->io_a.p, inputs, n * in_len, ctx->stream));
   B200_TRY(sponge_batch_device(ctx, ctx->io_a.as<uint8_t>(), in_len, n, ctx->io_b.as<uint8_t>(), out_len));
   B200_TRY(d2h_copy(ctx, outputs, ctx->io_b.p, n * out_len, ctx->stream));
+  return 0;
+}
+
+// Argument checks shared by both duplex entry points: fills the script's absorbed (*in_len) and squeezed (*out_len)
+// bytes per sponge.  Returns 0 or B200G16_ERR_ARG (with the message set).
+static int duplex_args(b200g16_ctx* ctx, const void* digests, size_t n, const uint8_t* tag, size_t tag_len,
+                       const b200g16_duplex_op* ops, size_t n_ops, const void* inputs, const void* outputs,
+                       size_t* in_len, size_t* out_len) {
+  if (!ctx || (n && !digests) || (n_ops && !ops)) return fail(B200G16_ERR_ARG, "keccak_duplex: null");
+  if (tag_len > 64) return fail(B200G16_ERR_ARG, "keccak_duplex: tag_len %zu > 64", tag_len);
+  size_t a = 0, s = 0;
+  for (size_t k = 0; k < n_ops; k++) {
+    if (ops[k].squeeze > 1) return fail(B200G16_ERR_ARG, "keccak_duplex: op %zu has kind %u", k, ops[k].squeeze);
+    size_t& acc = ops[k].squeeze ? s : a;
+    if (acc > SIZE_MAX - ops[k].len) return fail(B200G16_ERR_ARG, "keccak_duplex: script length overflows");
+    acc += ops[k].len;
+  }
+  if (n && (a > SIZE_MAX / n || s > SIZE_MAX / n)) return fail(B200G16_ERR_ARG, "keccak_duplex: n x row overflows");
+  if (n && a && !inputs) return fail(B200G16_ERR_ARG, "keccak_duplex: null inputs");
+  if (n && s && !outputs) return fail(B200G16_ERR_ARG, "keccak_duplex: null outputs");
+  *in_len = a;
+  *out_len = s;
+  return 0;
+}
+
+int b200g16_keccak_duplex_batch(b200g16_ctx* ctx, b200g16_keccak_digest* digests, size_t n, const uint8_t* tag,
+                                size_t tag_len, const b200g16_duplex_op* ops, size_t n_ops, const uint8_t* inputs,
+                                uint8_t* outputs) {
+  size_t A, S;
+  B200_TRY(duplex_args(ctx, digests, n, tag, tag_len, ops, n_ops, inputs, outputs, &A, &S));
+  if (!tag)
+    for (size_t i = 0; i < n; i++)
+      if (digests[i].absorb_pos > 136 || digests[i].squeeze_pos > 136)
+        return fail(B200G16_ERR_ARG, "keccak_duplex: digest %zu has a position above 136", i);
+  if (n == 0 || (n_ops == 0 && !tag)) return 0;
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  B200_CUDA(cudaSetDevice(ctx->device));
+  auto up16 = [](size_t v) { return (v + 15) & ~(size_t)15; };
+  const size_t sz_dg = n * sizeof(b200g16_keccak_digest), sz_ops = n_ops * sizeof(b200g16_duplex_op);
+  const size_t o_ops = up16(sz_dg), o_in = o_ops + up16(sz_ops);
+  B200_TRY(ctx->io_a.ensure(o_in + n * A));
+  B200_TRY(ctx->io_b.ensure(n * S ? n * S : 1));
+  char* d = ctx->io_a.as<char>();
+  cudaStream_t st = ctx->stream;
+  if (!tag) B200_TRY(h2d_copy(ctx, d, digests, sz_dg, st));
+  if (sz_ops) B200_CUDA(cudaMemcpyAsync(d + o_ops, ops, sz_ops, cudaMemcpyHostToDevice, st));
+  if (A) B200_TRY(h2d_copy(ctx, d + o_in, inputs, n * A, st));
+  B200_TRY(keccak_duplex_device(ctx, (uint64_t*)d, n, tag, tag_len, (const b200g16_duplex_op*)(d + o_ops), n_ops,
+                                (const uint8_t*)(d + o_in), A, ctx->io_b.as<uint8_t>(), S));
+  if (S) B200_TRY(d2h_copy(ctx, outputs, ctx->io_b.p, n * S, st));
+  B200_TRY(d2h_copy(ctx, digests, d, sz_dg, st));
+  return 0;
+}
+
+int b200g16_keccak_duplex_batch_dev(b200g16_ctx* ctx, void* d_digests, size_t n, const uint8_t* tag, size_t tag_len,
+                                    const b200g16_duplex_op* ops, size_t n_ops, const void* d_inputs, void* d_outputs) {
+  size_t A, S;
+  B200_TRY(duplex_args(ctx, d_digests, n, tag, tag_len, ops, n_ops, d_inputs, d_outputs, &A, &S));
+  if (n == 0 || (n_ops == 0 && !tag)) return 0;
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  B200_CUDA(cudaSetDevice(ctx->device));
+  const size_t sz_ops = n_ops * sizeof(b200g16_duplex_op), o_flag = (sz_ops + 15) & ~(size_t)15;
+  B200_TRY(ctx->io_a.ensure(o_flag + 16));
+  char* d = ctx->io_a.as<char>();
+  if (!tag) {   // every position is checked before any digest changes
+    bool bad = false;
+    B200_TRY(keccak_duplex_check_device(ctx, (const uint64_t*)d_digests, n, (uint32_t*)(d + o_flag), &bad));
+    if (bad) return fail(B200G16_ERR_ARG, "keccak_duplex: a digest has a position above 136");
+  }
+  if (sz_ops) B200_CUDA(cudaMemcpyAsync(d, ops, sz_ops, cudaMemcpyHostToDevice, ctx->stream));
+  B200_TRY(keccak_duplex_device(ctx, (uint64_t*)d_digests, n, tag, tag_len, (const b200g16_duplex_op*)d, n_ops,
+                                (const uint8_t*)d_inputs, A, (uint8_t*)d_outputs, S));
+  B200_CUDA(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
 

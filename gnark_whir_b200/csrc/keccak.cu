@@ -7,6 +7,8 @@
 //   k_sponge_batch    <- keccakSponge.Digest: NewKeccak / Absorb / Squeeze
 //                        (keccakSponge.go:17-30, 40-56, 64-75): rate 136 B, OVERWRITE absorb,
 //                        no padding, permute-on-full and permute-before-first-squeeze
+//   k_duplex_thread,  <- the whole keccakSponge.Digest (keccakSponge.go:17-75): NewKeccakWithTag, Absorb /
+//   k_duplex_warp        Squeeze in any order, the state carried across calls (byte rules: keccak_duplex.cuh)
 //   k_merkle_paths    <- VerifyMerkleTreeProofs (/root/reference/mtUtilities.go:109-141): leaf hash,
 //                        then per level pair with the sibling by the index bit (bit 0 uses
 //                        LeafSiblingHashes, bit k>=1 uses AuthPaths[k-1]; set bit => current node
@@ -19,6 +21,7 @@
 #include <cstdlib>
 
 #include "common.cuh"
+#include "keccak_duplex.cuh"
 
 namespace b200 {
 
@@ -400,6 +403,186 @@ __global__ void __launch_bounds__(32 * WARPS) k_merkle_paths_warp(const uint8_t*
   }
 }
 
+// ---- Keccak duplex (b200g16_keccak_duplex_batch): keccakSponge.Digest with Absorb / Squeeze in any order and the
+// state carried across calls.  A digest is 26 words: the 25 lanes, then absorb_pos (low half) and squeeze_pos (high
+// half).  Every sponge runs the same op script (device memory, read uniformly); keccak_duplex.cuh cuts each op into
+// segments that stay inside one rate block, and a segment touches the rate lanes it overlaps, byte by byte where it
+// starts or ends inside a lane or the row is not 8-byte aligned, one 64-bit access otherwise.
+constexpr int DIGEST_WORDS = 26;
+
+struct DuplexTag {
+  uint64_t lane[8];   // state lanes 17..24 of NewKeccakWithTag (the tag's bytes 136..199, zero-padded)
+  int use;            // 1: start every sponge from this state, 0: continue from its digest
+};
+
+__device__ __forceinline__ uint64_t duplex_positions(uint32_t absorb_pos, uint32_t squeeze_pos) {
+  return (uint64_t)absorb_pos | ((uint64_t)squeeze_pos << 32);
+}
+
+// bytes [lo, hi) of the lane whose byte 0 maps to p (only p[lo..hi) is touched)
+__device__ __forceinline__ uint64_t duplex_load(const uint8_t* p, uint32_t lo, uint32_t hi) {
+  if (lo == 0 && hi == 8 && ((uintptr_t)p & 7) == 0) return *reinterpret_cast<const uint64_t*>(p);
+  uint64_t v = 0;
+  for (uint32_t k = lo; k < hi; k++) v |= (uint64_t)p[k] << (8 * k);
+  return v;
+}
+
+__device__ __forceinline__ void duplex_store(uint8_t* p, uint64_t v, uint32_t lo, uint32_t hi) {
+  if (lo == 0 && hi == 8 && ((uintptr_t)p & 7) == 0) { *reinterpret_cast<uint64_t*>(p) = v; return; }
+  for (uint32_t k = lo; k < hi; k++) p[k] = (uint8_t)(v >> (8 * k));
+}
+
+__device__ __forceinline__ uint64_t duplex_mask(uint32_t lo, uint32_t hi) {
+  return (hi == 8 ? ~0ull : (1ull << (8 * hi)) - 1) & ~((1ull << (8 * lo)) - 1);
+}
+
+// One thread per sponge, 25 lanes in registers.  A warp stages its 32 digests (6656 contiguous bytes) through shared
+// memory in and out, as k_keccak_f_batch does, so the digest traffic is coalesced.
+constexpr int DUPLEX_THREADS = 128;
+__global__ void __launch_bounds__(DUPLEX_THREADS) k_duplex_thread(uint64_t* __restrict__ digests, size_t n, DuplexTag tag,
+                                                                  const b200g16_duplex_op* __restrict__ ops, size_t n_ops,
+                                                                  const uint8_t* __restrict__ in, size_t in_stride,
+                                                                  uint8_t* __restrict__ out, size_t out_stride) {
+  __shared__ uint64_t sm[DUPLEX_THREADS / 32][32 * DIGEST_WORDS];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const size_t warp_first = (size_t)blockIdx.x * DUPLEX_THREADS + (size_t)warp * 32;
+  if (warp_first >= n) return;   // whole warps leave together
+  const uint32_t in_warp = n - warp_first < 32 ? (uint32_t)(n - warp_first) : 32;
+  uint64_t* g = digests + warp_first * DIGEST_WORDS;
+  const uint32_t words = in_warp * DIGEST_WORDS;
+  uint64_t* mine = sm[warp] + lane * DIGEST_WORDS;
+  if (!tag.use) {
+#pragma unroll
+    for (int j = 0; j < DIGEST_WORDS; j++) {
+      const uint32_t w = lane + 32 * j;
+      if (w < words) sm[warp][w] = g[w];
+    }
+    __syncwarp();
+  }
+  if ((uint32_t)lane < in_warp) {
+    const size_t i = warp_first + lane;
+    uint64_t a[25];
+    DuplexWalk w;
+    if (tag.use) {
+#pragma unroll
+      for (int l = 0; l < 25; l++) a[l] = l < KECCAK_RATE_LANES ? 0 : tag.lane[l - KECCAK_RATE_LANES];
+      w.absorb_pos = 0;
+      w.squeeze_pos = DUPLEX_RATE;
+    } else {
+#pragma unroll
+      for (int l = 0; l < 25; l++) a[l] = mine[l];
+      w.absorb_pos = (uint32_t)mine[25];
+      w.squeeze_pos = (uint32_t)(mine[25] >> 32);
+    }
+    const uint8_t* in_row = in + i * in_stride;
+    uint8_t* out_row = out + i * out_stride;
+    uint64_t in_off = 0, out_off = 0;
+    for (size_t k = 0; k < n_ops; k++) {
+      const b200g16_duplex_op op = ops[k];
+      const bool sq = op.squeeze != 0;
+      duplex_op_begin(w, op.len, sq ? out_off : in_off);
+      while (w.left) {
+        const DuplexSeg s = duplex_next(w, sq);
+        if (s.permute) keccak_f1600(a);
+        // lane l's byte 0 sits at row byte s.row_off + 8l - s.rate_off (only its bytes inside the segment are touched)
+        const long long base = (long long)s.row_off - (long long)s.rate_off;
+#pragma unroll
+        for (int l = 0; l < KECCAK_RATE_LANES; l++) {
+          uint32_t lo, hi;
+          if (!duplex_lane_span(s, l, &lo, &hi)) continue;
+          if (sq) {
+            duplex_store(out_row + base + 8 * l, a[l], lo, hi);
+          } else {
+            const uint64_t m = duplex_mask(lo, hi);
+            a[l] = (a[l] & ~m) | (duplex_load(in_row + base + 8 * l, lo, hi) & m);
+          }
+        }
+      }
+      duplex_op_end(w, sq);
+      if (sq) out_off = w.row_off;
+      else in_off = w.row_off;
+    }
+#pragma unroll
+    for (int l = 0; l < 25; l++) mine[l] = a[l];
+    mine[25] = duplex_positions(w.absorb_pos, w.squeeze_pos);
+  }
+  __syncwarp();
+#pragma unroll
+  for (int j = 0; j < DIGEST_WORDS; j++) {
+    const uint32_t w = lane + 32 * j;
+    if (w < words) g[w] = sm[warp][w];
+  }
+}
+
+// One WARP per sponge, for the few sponges of a transcript replay: lane l = x + 5y holds state lane A[x, y] and the
+// permutation is keccak_f1600_warp (as k_merkle_paths_warp runs it); lane l < 17 overwrites or emits the bytes of its
+// lane that fall inside a segment.
+template <int WARPS, bool SMEM>
+__global__ void __launch_bounds__(32 * WARPS) k_duplex_warp(uint64_t* __restrict__ digests, size_t n, DuplexTag tag,
+                                                             const b200g16_duplex_op* __restrict__ ops, size_t n_ops,
+                                                             const uint8_t* __restrict__ in, size_t in_stride,
+                                                             uint8_t* __restrict__ out, size_t out_stride) {
+  __shared__ uint64_t sx[SMEM ? WARPS : 1][2][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const size_t i = (size_t)blockIdx.x * WARPS + warp;
+  if (i >= n) return;   // whole warps leave together
+  uint64_t* sA = sx[SMEM ? warp : 0][0];
+  uint64_t* sB = sx[SMEM ? warp : 0][1];
+  const KeccakLaneCtx c = keccak_lane_ctx(lane);
+  uint64_t* dg = digests + i * DIGEST_WORDS;
+  uint64_t a;
+  DuplexWalk w;
+  if (tag.use) {
+    a = 0;
+#pragma unroll
+    for (int j = 0; j < 8; j++)
+      if (lane == KECCAK_RATE_LANES + j) a = tag.lane[j];
+    w.absorb_pos = 0;
+    w.squeeze_pos = DUPLEX_RATE;
+  } else {
+    a = lane < 25 ? dg[lane] : 0;
+    const uint64_t pos = dg[25];
+    w.absorb_pos = (uint32_t)pos;
+    w.squeeze_pos = (uint32_t)(pos >> 32);
+  }
+  const uint8_t* in_row = in + i * in_stride;
+  uint8_t* out_row = out + i * out_stride;
+  uint64_t in_off = 0, out_off = 0;
+  for (size_t k = 0; k < n_ops; k++) {
+    const b200g16_duplex_op op = ops[k];
+    const bool sq = op.squeeze != 0;
+    duplex_op_begin(w, op.len, sq ? out_off : in_off);
+    while (w.left) {
+      const DuplexSeg s = duplex_next(w, sq);
+      if (s.permute) a = keccak_f1600_warp<SMEM>(a, c, lane, sA, sB);
+      uint32_t lo, hi;
+      if (lane < KECCAK_RATE_LANES && duplex_lane_span(s, lane, &lo, &hi)) {
+        const long long at = (long long)s.row_off - (long long)s.rate_off + 8 * lane;
+        if (sq) {
+          duplex_store(out_row + at, a, lo, hi);
+        } else {
+          const uint64_t m = duplex_mask(lo, hi);
+          a = (a & ~m) | (duplex_load(in_row + at, lo, hi) & m);
+        }
+      }
+    }
+    duplex_op_end(w, sq);
+    if (sq) out_off = w.row_off;
+    else in_off = w.row_off;
+  }
+  if (lane < 25) dg[lane] = a;
+  if (lane == 0) dg[25] = duplex_positions(w.absorb_pos, w.squeeze_pos);
+}
+
+// *bad = 1 if a digest holds a position above 136 (run before a continuing call changes any digest)
+__global__ void __launch_bounds__(256) k_duplex_check(const uint64_t* __restrict__ digests, size_t n,
+                                                      uint32_t* __restrict__ bad) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint64_t pos = digests[i * DIGEST_WORDS + 25];
+  if ((uint32_t)pos > DUPLEX_RATE || (uint32_t)(pos >> 32) > DUPLEX_RATE) *bad = 1;
+}
+
 // ------------------------------------------------------------------------------ host drivers
 int keccak_f_batch_device(b200g16_ctx* ctx, uint64_t* d_states, size_t n) {
   if (n == 0) return 0;
@@ -452,6 +635,57 @@ int merkle_paths_device(b200g16_ctx* ctx, const uint8_t* d_leaves, size_t leaf_l
                                                                         height, n, d_expected_root, d_roots, d_ok);
   ctx->launches++;
   B200_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// Up to here one warp per sponge; above, one thread per sponge.  Measured (profiles/r03c_keccak_duplex.jsonl, transcript
+// script, 6 permutations per sponge, device path, median call): the warp form takes 0.078-0.080 ms from 1 to 1024
+// sponges where the thread form takes 0.161-0.172 (one thread runs the 6 dependent permutations about twice as slowly
+// as a warp), 0.107 against 0.164 ms at 4096, 0.150 against 0.160 at 8192; at 16384 the warps no longer fit one wave
+// (148 SMs x 64 warps) and the thread form wins, 0.163 against 0.234 ms.
+constexpr size_t DUPLEX_WARP_MAX = 8192;
+
+// tag: NULL = continue from the digests, else tag_len (<= 64) bytes of NewKeccakWithTag.  d_ops in device memory.
+int keccak_duplex_device(b200g16_ctx* ctx, uint64_t* d_digests, size_t n, const uint8_t* tag, size_t tag_len,
+                         const b200g16_duplex_op* d_ops, size_t n_ops, const uint8_t* d_in, size_t in_stride,
+                         uint8_t* d_out, size_t out_stride) {
+  if (n == 0) return 0;
+  DuplexTag t = {};
+  t.use = tag != nullptr;
+  for (size_t j = 0; tag && j < tag_len; j++) t.lane[j / 8] |= (uint64_t)tag[j] << (8 * (j % 8));
+  // experiment knob (tools/duplex_bench.py): B200G16_DUPLEX_WARP = 1 forces the warp form, 0 the thread form
+  const char* e = getenv("B200G16_DUPLEX_WARP");
+  const bool warp = e && *e ? atoi(e) != 0 : n <= DUPLEX_WARP_MAX;
+  if (warp) {
+    // the exchange mechanism and CTA shape k_merkle_paths_warp measured best (profiles/r02o_merkle_warp_sweep.jsonl):
+    // shared memory with one warp per CTA up to 512 sponges, shuffles with two warps per CTA above
+    if (n <= 512)
+      k_duplex_warp<1, true><<<(unsigned)n, 32, 0, ctx->stream>>>(d_digests, n, t, d_ops, n_ops, d_in, in_stride, d_out,
+                                                                   out_stride);
+    else
+      k_duplex_warp<2, false><<<(unsigned)((n + 1) / 2), 64, 0, ctx->stream>>>(d_digests, n, t, d_ops, n_ops, d_in,
+                                                                                in_stride, d_out, out_stride);
+  } else {
+    k_duplex_thread<<<(unsigned)((n + DUPLEX_THREADS - 1) / DUPLEX_THREADS), DUPLEX_THREADS, 0, ctx->stream>>>(
+        d_digests, n, t, d_ops, n_ops, d_in, in_stride, d_out, out_stride);
+  }
+  ctx->launches++;
+  B200_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// *bad = whether a digest holds a position above 136; d_flag: 4 bytes of device scratch.  Synchronises the stream.
+int keccak_duplex_check_device(b200g16_ctx* ctx, const uint64_t* d_digests, size_t n, uint32_t* d_flag, bool* bad) {
+  *bad = false;
+  if (n == 0) return 0;
+  B200_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(uint32_t), ctx->stream));
+  k_duplex_check<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(d_digests, n, d_flag);
+  ctx->launches++;
+  B200_CUDA(cudaGetLastError());
+  uint32_t h = 0;
+  B200_CUDA(cudaMemcpyAsync(&h, d_flag, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+  B200_CUDA(cudaStreamSynchronize(ctx->stream));
+  *bad = h != 0;
   return 0;
 }
 

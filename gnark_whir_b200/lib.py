@@ -66,6 +66,8 @@ SIGNATURES = {
     "b200g16_keccak_f_batch": (C.c_int, [_vp, _vp, _sz]),
     "b200g16_keccak_f_batch_dev": (C.c_int, [_vp, _vp, _sz]),
     "b200g16_keccak_sponge_batch": (C.c_int, [_vp, _vp, _sz, _sz, _vp, _sz]),
+    "b200g16_keccak_duplex_batch": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp, _vp]),
+    "b200g16_keccak_duplex_batch_dev": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp, _vp]),
     "b200g16_keccak_merkle_paths": (C.c_int, [_vp, _vp, _sz, _vp, _vp, _vp, C.c_uint, _sz, _vp, _vp, _vp]),
     "b200g16_keccak_merkle_paths_dev": (C.c_int, [_vp, _vp, _sz, _vp, _vp, _vp, C.c_uint, _sz, _vp, _vp, _vp]),
     "b200g16_pk_upload": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
@@ -127,6 +129,42 @@ def load():
         fn.argtypes = args
     _lib = lib
     return lib
+
+
+# struct b200g16_keccak_digest: keccakSponge.Digest between calls (25 little-endian lanes, then the two positions)
+KECCAK_DIGEST = np.dtype([("state", "<u8", (25,)), ("absorb_pos", "<u4"), ("squeeze_pos", "<u4")])
+KECCAK_RATE = 136
+# sponges up to which b200g16_keccak_duplex_batch runs one warp per sponge (DUPLEX_WARP_MAX in csrc/keccak.cu)
+KECCAK_DUPLEX_WARP_MAX = 8192
+
+
+def keccak_digests(n, tags=None):
+    """n fresh digests: NewKeccak, or NewKeccakWithTag(tags[i]) for sponge i (tags: n byte strings of <= 64 bytes, or
+    one for all).  Pass them to keccak_duplex_batch with tag=None to start each sponge from its own tag."""
+    d = np.zeros(n, dtype=KECCAK_DIGEST)
+    d["squeeze_pos"] = KECCAK_RATE
+    if tags is not None:
+        if isinstance(tags, (bytes, bytearray)):
+            tags = [tags] * n
+        if len(tags) != n:
+            raise B200Error("keccak_digests: one tag per sponge")
+        raw = d.view(np.uint8).reshape(n, KECCAK_DIGEST.itemsize)
+        for i, t in enumerate(tags):
+            if len(t) > 64:
+                raise B200Error("keccak_digests: a tag has at most 64 bytes")
+            raw[i, KECCAK_RATE:KECCAK_RATE + len(t)] = np.frombuffer(bytes(t), dtype=np.uint8)
+    return d
+
+
+def duplex_script(ops):
+    """[("absorb", len) | ("squeeze", len), ...] -> (struct b200g16_duplex_op array, absorbed bytes, squeezed bytes)"""
+    kinds = {"absorb": 0, "squeeze": 1}
+    arr = np.zeros((len(ops), 2), dtype=np.uint32)
+    for k, (kind, n) in enumerate(ops):
+        if kind not in kinds or not 0 <= int(n) < 1 << 32:
+            raise B200Error(f"duplex op {k}: {kind!r}, {n!r}")
+        arr[k] = kinds[kind], int(n)
+    return arr, int(arr[arr[:, 0] == 0, 1].sum()), int(arr[arr[:, 0] == 1, 1].sum())
 
 
 # b200g16_set_msm_batch_affine(mode, levels, min_pairs) as a fresh ctx has it
@@ -501,6 +539,39 @@ class Context:
         out = np.zeros((n, out_len), dtype=np.uint8)
         _check(load().b200g16_keccak_sponge_batch(self.h, _ptr(a), in_len, n, _ptr(out), out_len))
         return out
+
+    def keccak_duplex_batch(self, ops, inputs, digests=None, tag=None):
+        """keccakSponge.Digest for n sponges running the same op script, state carried across calls.
+        ops: [("absorb", len) | ("squeeze", len), ...]; inputs: (n, A) uint8, A = the absorbed bytes of the script;
+        digests: (n,) KECCAK_DIGEST to continue from (None: start fresh); tag: bytes of NewKeccakWithTag for every
+        sponge (b"" = NewKeccak; ignored digests are not read).  -> (outputs (n, S) uint8, final digests)"""
+        script, A, S = duplex_script(ops)
+        inp = np.ascontiguousarray(inputs, dtype=np.uint8)
+        if inp.ndim != 2 or inp.shape[1] != A:
+            raise B200Error(f"keccak_duplex_batch: inputs must be (n, {A})")
+        n = inp.shape[0]
+        if digests is None:
+            dg = np.zeros(n, dtype=KECCAK_DIGEST)
+            tag = b"" if tag is None else tag
+        else:
+            dg = np.ascontiguousarray(digests, dtype=KECCAK_DIGEST).copy()
+            if dg.shape != (n,):
+                raise B200Error(f"keccak_duplex_batch: {n} digests expected")
+        tg = None if tag is None else np.frombuffer(bytes(tag) + b"\0", dtype=np.uint8)
+        out = np.zeros((n, S), dtype=np.uint8)
+        _check(load().b200g16_keccak_duplex_batch(self.h, _ptr(dg), n, _ptr(tg) if tg is not None else None,
+                                                  len(tg) - 1 if tg is not None else 0, _ptr(script), len(ops),
+                                                  _ptr(inp), _ptr(out)))
+        return out, dg
+
+    def keccak_duplex_batch_dev(self, d_digests, n, ops, d_inputs, d_outputs, tag=None):
+        """The same on device pointers: d_digests n x 208 bytes (8-byte aligned), d_inputs n x A and d_outputs n x S
+        bytes (any alignment); ops and tag as keccak_duplex_batch (tag None: continue from the digests)."""
+        script, _, _ = duplex_script(ops)
+        tg = None if tag is None else np.frombuffer(bytes(tag) + b"\0", dtype=np.uint8)
+        _check(load().b200g16_keccak_duplex_batch_dev(
+            self.h, _dp(d_digests), n, _ptr(tg) if tg is not None else None, len(tg) - 1 if tg is not None else 0,
+            _ptr(script), len(ops), _dp(d_inputs) if d_inputs else None, _dp(d_outputs) if d_outputs else None))
 
     def keccak_merkle_paths(self, leaves, siblings, auth_paths, indexes, expected_root=None):
         """leaves (n, leaf_len) u8; siblings (n, 32) u8; auth_paths (n, height-1, 32) u8;

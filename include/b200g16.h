@@ -263,6 +263,41 @@ int b200g16_keccak_f_batch_dev(b200g16_ctx* ctx, void* d_states, size_t n);
  * (keccakSponge.go:17-75): rate 136, overwrite-mode absorb, no padding. */
 int b200g16_keccak_sponge_batch(b200g16_ctx* ctx, const uint8_t* inputs, size_t in_len, size_t n,
                                 uint8_t* outputs, size_t out_len);
+/* keccakSponge.Digest between calls (keccakSponge.go:9-15): the 200-byte state as 25 little-endian lanes
+ * (lane x + 5y), then the two byte positions, each in 0..136.  NewKeccak = state all zero, absorb_pos 0,
+ * squeeze_pos 136.  NewKeccakWithTag(tag) is the same with tag[j] in state byte 136 + j (tag_len <= 64). */
+typedef struct b200g16_keccak_digest {
+  uint64_t state[25];
+  uint32_t absorb_pos;
+  uint32_t squeeze_pos;
+} b200g16_keccak_digest; /* 208 B */
+typedef struct b200g16_duplex_op {
+  uint32_t squeeze; /* 0: Absorb(len bytes), 1: Squeeze(len) */
+  uint32_t len;
+} b200g16_duplex_op;
+/* The whole Digest (keccakSponge.go:17-75: NewKeccak, NewKeccakWithTag, Absorb and Squeeze in any order) for n
+ * sponges that run the same script of n_ops ops, in order, with the state carried across calls:
+ *   inputs   n x A bytes, A = the sum of the absorb lengths; row i is sponge i's absorbed bytes in script order
+ *   outputs  n x S bytes, S = the sum of the squeeze lengths; row i receives sponge i's squeezed bytes
+ *   tag      non-NULL: every sponge starts from NewKeccakWithTag(tag[:tag_len]) (tag_len 0 = NewKeccak) and the
+ *            incoming digests are not read; NULL: every sponge continues from its digest (per-sponge tags: write
+ *            the bytes into fresh digests and pass tag = NULL)
+ *   digests  receive the final states either way.
+ * Byte rules exactly as the Digest: Absorb overwrites state byte absorb_pos (permuting first when it is 136) and
+ * sets squeeze_pos = 136 when it ends, also for len 0; Squeeze permutes first when squeeze_pos is 136 (both
+ * positions to 0) and emits byte squeeze_pos.  An absorbed full block stays unpermuted (absorb_pos 136) until the
+ * next byte or squeeze, across calls too.  ops and tag are host memory in both calls.
+ * B200G16_ERR_ARG, with nothing written: tag_len > 64, a digest position above 136 (tag == NULL), an op kind
+ * other than 0 / 1, NULL inputs with A > 0 or NULL outputs with S > 0, n x A or n x S overflowing size_t.
+ * n = 0 or n_ops = 0 returns 0. */
+int b200g16_keccak_duplex_batch(b200g16_ctx* ctx, b200g16_keccak_digest* digests, size_t n,
+                                const uint8_t* tag, size_t tag_len, const b200g16_duplex_op* ops, size_t n_ops,
+                                const uint8_t* inputs, uint8_t* outputs);
+/* Same with digests, inputs and outputs in DEVICE memory (d_digests 8-byte aligned; d_inputs and d_outputs
+ * may have any alignment). */
+int b200g16_keccak_duplex_batch_dev(b200g16_ctx* ctx, void* d_digests, size_t n,
+                                    const uint8_t* tag, size_t tag_len, const b200g16_duplex_op* ops, size_t n_ops,
+                                    const void* d_inputs, void* d_outputs);
 /* Recompute n_paths Merkle roots.  Mirrors VerifyMerkleTreeProofs
  * (/root/reference/mtUtilities.go:109-141) with the 2-to-1 hash instantiated by the Keccak
  * duplex above (leaf hash = sponge over the leaf's bytes, node = sponge over left||right,
