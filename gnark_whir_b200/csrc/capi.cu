@@ -5,12 +5,14 @@
 
 namespace b200 {
 // instantiated in msm_g1.cu / msm_g2.cu
-extern template int msm_enqueue<Fp>(b200g16_ctx*, const Affine<Fp>*, const MsmTable*, const Fr*, size_t, int, MsmCfg*, bool, bool);
-extern template int msm_collect<Fp>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp>*);
+extern template int msm_enqueue<Fp>(b200g16_ctx*, const Affine<Fp>*, const MsmTable*, const Fr*, size_t, size_t, size_t, int, MsmCfg*,
+                                   bool, bool);
+extern template int msm_collect<Fp>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp>*, size_t);
 extern template int msm_device<Fp>(b200g16_ctx*, const Affine<Fp>*, const MsmTable*, const Fr*, size_t, Affine<Fp>*);
 extern template int msm_build_table<Fp>(b200g16_ctx*, Affine<Fp>*, size_t, int, int);
-extern template int msm_enqueue<Fp2>(b200g16_ctx*, const Affine<Fp2>*, const MsmTable*, const Fr*, size_t, int, MsmCfg*, bool, bool);
-extern template int msm_collect<Fp2>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp2>*);
+extern template int msm_enqueue<Fp2>(b200g16_ctx*, const Affine<Fp2>*, const MsmTable*, const Fr*, size_t, size_t, size_t, int, MsmCfg*,
+                                   bool, bool);
+extern template int msm_collect<Fp2>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp2>*, size_t);
 extern template int msm_device<Fp2>(b200g16_ctx*, const Affine<Fp2>*, const MsmTable*, const Fr*, size_t, Affine<Fp2>*);
 extern template int msm_build_table<Fp2>(b200g16_ctx*, Affine<Fp2>*, size_t, int, int);
 
@@ -111,7 +113,7 @@ static int msm_entry(b200g16_ctx* ctx, const b200g16_bases* bases, int group, si
       B200_CUDA(cudaEventRecord(ctx->ev_copy[j], ctx->copy_stream));
       B200_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy[j], 0));
       const Affine<F>* pts = msm_operand<F>(bases, offset + lo[j], &tab, &tp);
-      B200_TRY(msm_enqueue<F>(ctx, pts, tp, d + lo[j], m, j, &cfg[j], false));
+      B200_TRY(msm_enqueue<F>(ctx, pts, tp, d + lo[j], m, 1, m, j, &cfg[j], false));
     }
     B200_TRY(msm_join(ctx));
     B200_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -133,6 +135,81 @@ static int msm_entry(b200g16_ctx* ctx, const b200g16_bases* bases, int group, si
     B200_TRY(msm_device<F>(ctx, pts, tp, d_scalars, n, &res));
   }
   memcpy(out, &res, sizeof(res));
+  return 0;
+}
+
+// k MSMs of n scalars each over the same resident bases: out[j] = sum_i scalars[j * n + i] * bases[offset + i].
+// Sub-batches of msm_batch_max vectors, up to MSM_BATCH_SLOTS of them enqueued back to back (each sub-batch's bucket
+// reduction runs under the next one's sort and accumulate), then one synchronisation and the host's Horner per vector.
+// k == 1, and a shape whose sub-batches hold one vector, take the single-MSM path.
+constexpr int MSM_BATCH_SLOTS = 5;   // result slots 0..4: 5..7 belong to open b200g16_msm_g1_begin tickets
+
+template <class F>
+static int msm_batch_entry(b200g16_ctx* ctx, const b200g16_bases* bases, int group, size_t offset, const void* scalars,
+                           bool scalars_on_device, size_t n, size_t k, uint64_t* out) {
+  if (!ctx || !bases || (k && (!out || (n && !scalars)))) return fail(B200G16_ERR_ARG, "msm_batch: null argument");
+  if (bases->group != group) return fail(B200G16_ERR_ARG, "msm_batch: bases are G%d, call is G%d", bases->group, group);
+  if (bases->device != ctx->device) return fail(B200G16_ERR_STATE, "msm_batch: bases live on another device");
+  if (offset > bases->n || n > bases->n - offset)
+    return fail(B200G16_ERR_ARG, "msm_batch: range [%zu,%zu) exceeds %zu bases", offset, offset + n, bases->n);
+  if (n >= (1ull << 31)) return fail(B200G16_ERR_ARG, "msm_batch: n=%zu too large", n);
+  if (n && k > SIZE_MAX / sizeof(Fr) / n) return fail(B200G16_ERR_ARG, "msm_batch: k x n overflows");
+  if (k == 0) return 0;
+  constexpr size_t words = sizeof(Affine<F>) / sizeof(uint64_t);
+  if (k == 1) return msm_entry<F>(ctx, bases, group, offset, scalars, scalars_on_device, n, out);
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  if (ctx->prove_active)
+    return fail(B200G16_ERR_STATE, "msm_batch: a prove is open on this ctx (b200g16_prove_begin_dev without _end_dev)");
+  B200_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  ctx->timings.n = 0;
+  B200_CUDA(cudaEventRecord(ctx->ev[0], st));
+  const Fr* d = reinterpret_cast<const Fr*>(scalars);
+  if (!scalars_on_device && n) {
+    B200_TRY(ctx->msm.scalars.ensure(k * n * sizeof(Fr)));
+    B200_TRY(h2d_copy(ctx, ctx->msm.scalars.p, scalars, k * n * sizeof(Fr), st));
+    d = ctx->msm.scalars.as<Fr>();
+  }
+  MsmTable tab;
+  const MsmTable* tp = nullptr;
+  const Affine<F>* pts = msm_operand<F>(bases, offset, &tab, &tp);
+  const int c = msm_window_for(ctx, tp, n);
+  const size_t ksub = std::min(k, msm_batch_max(c, tp != nullptr, n));
+  if (ksub > 1) B200_TRY(msm_batch_stage(ctx, ksub * (tp ? 1 : msm_num_windows(c)) * sizeof(XYZZ<F>)));
+  MsmCfg cfg[MSM_BATCH_SLOTS];
+  size_t first[MSM_BATCH_SLOTS];
+  int pending = 0;
+  auto run = [&]() -> int {
+    for (size_t j0 = 0; j0 < k;) {
+      pending = 0;
+      for (; pending < MSM_BATCH_SLOTS && j0 < k; pending++) {
+        const size_t m = std::min(ksub, k - j0);
+        first[pending] = j0;
+        B200_TRY(msm_enqueue<F>(ctx, pts, tp, d + j0 * n, n, m, n, pending, &cfg[pending], false));
+        j0 += m;
+      }
+      B200_TRY(msm_join(ctx));
+      B200_CUDA(cudaStreamSynchronize(st));
+      for (int q = 0; q < pending; q++)
+        for (size_t j = 0; j < std::max<size_t>(cfg[q].k, 1); j++) {
+          Affine<F> res;
+          B200_TRY(msm_collect<F>(ctx, q, cfg[q], &res, j));
+          memcpy(out + (first[q] + j) * words, &res, sizeof(res));
+        }
+      pending = 0;
+    }
+    return 0;
+  };
+  if (int status = run()) {   // leave the ctx usable: whatever is in flight is drained and forgotten
+    msm_join(ctx);
+    cudaStreamSynchronize(st);
+    cudaStreamSynchronize(ctx->tail_stream);
+    return status;
+  }
+  B200_CUDA(cudaEventRecord(ctx->ev[1], st));
+  B200_CUDA(cudaEventSynchronize(ctx->ev[1]));
+  cudaEventElapsedTime(&ctx->timings.ms[0], ctx->ev[0], ctx->ev[1]);
+  ctx->timings.n = 1;
   return 0;
 }
 
@@ -271,6 +348,7 @@ void b200g16_destroy(b200g16_ctx* ctx) {
     ctx->dist_h.slice[v].release();
   }
   if (ctx->msm.pinned) cudaFreeHost(ctx->msm.pinned);
+  if (ctx->msm.batch_pinned) cudaFreeHost(ctx->msm.batch_pinned);
   for (auto& ev : ctx->ev) cudaEventDestroy(ev);
   for (int i = 0; i < MSM_SETS; i++) { cudaEventDestroy(ctx->ev_front[i]); cudaEventDestroy(ctx->ev_tail[i]); }
   for (auto& ev : ctx->ev_copy) cudaEventDestroy(ev);
@@ -406,6 +484,23 @@ int b200g16_msm_g2_dev(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offs
   return msm_entry<Fp2>(ctx, bases, 2, offset, d_scalars, true, n, out);
 }
 
+int b200g16_msm_g1_batch(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const uint64_t* scalars, size_t n,
+                         size_t k, uint64_t* out) {
+  return msm_batch_entry<Fp>(ctx, bases, 1, offset, scalars, false, n, k, out);
+}
+int b200g16_msm_g2_batch(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const uint64_t* scalars, size_t n,
+                         size_t k, uint64_t* out) {
+  return msm_batch_entry<Fp2>(ctx, bases, 2, offset, scalars, false, n, k, out);
+}
+int b200g16_msm_g1_batch_dev(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const void* d_scalars, size_t n,
+                             size_t k, uint64_t* out) {
+  return msm_batch_entry<Fp>(ctx, bases, 1, offset, d_scalars, true, n, k, out);
+}
+int b200g16_msm_g2_batch_dev(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const void* d_scalars, size_t n,
+                             size_t k, uint64_t* out) {
+  return msm_batch_entry<Fp2>(ctx, bases, 2, offset, d_scalars, true, n, k, out);
+}
+
 // ---- asynchronous G1 MSM: enqueue now, take the result later.  gnark runs pedersen.ProveKnowledge after Solve and
 // before the five MSMs of Prove; nothing in between depends on its result, so a host can enqueue it, call
 // b200g16_prove, and collect it afterwards — its sort and accumulate run first, its bucket reduction hides under the
@@ -433,7 +528,7 @@ static int msm_begin(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset
   MsmTable tab;
   const MsmTable* tp = nullptr;
   const Affine<Fp>* pts = msm_operand<Fp>(bases, offset, &tab, &tp);
-  B200_TRY(msm_enqueue<Fp>(ctx, pts, tp, d_scalars, n, ASYNC_FIRST_SLOT + t, &ctx->async_cfg[t], false));
+  B200_TRY(msm_enqueue<Fp>(ctx, pts, tp, d_scalars, n, 1, n, ASYNC_FIRST_SLOT + t, &ctx->async_cfg[t], false));
   ctx->async_open[t] = true;
   *ticket = t;
   return 0;

@@ -78,6 +78,10 @@ struct MsmWorkspace {
   DevBuf aff_lvl[AFF_WS_LEVELS], aff_desc, aff_spill, aff_spill_task;
   void* pinned = nullptr;  // small host staging for window sums
   size_t pinned_cap = 0;
+  // window sums of batch MSMs (k vectors: k * Wr items per slot), MSM_SLOTS slots of batch_slot bytes.  Its own buffer:
+  // `pinned` is never reallocated while an asynchronous ticket (slots 5..7) may still be landing in it.
+  void* batch_pinned = nullptr;
+  size_t batch_slot = 0;
 };
 
 struct NttWorkspace {
@@ -99,14 +103,15 @@ struct MsmCfg {
   int c;          // window bits
   int W;          // windows
   uint32_t nbw;   // buckets per window = 2^(c-1)
-  uint32_t nb;    // buckets in total: W * nbw, or nbw when the bases carry a window table
-  int Wr;         // window sums produced by the reduction: W, or 1 with a window table
+  uint32_t nb;    // buckets in total: k * (W * nbw, or nbw when the bases carry a window table)
+  int Wr;         // window sums per vector produced by the reduction: W, or 1 with a window table
   uint32_t bstride;     // bucket-index stride between windows: nbw, or 0 with a window table
   uint32_t ent_stride;  // entry = w * ent_stride + ent_off + i  (index into the bases / the table)
   uint32_t ent_off;
   uint32_t target_tasks;  // accumulate tasks wanted even for skewed inputs (device picks the task size)
   uint32_t ch;    // buckets per reduce chunk
   uint32_t nch;   // chunks per window
+  uint32_t k;     // scalar vectors (1: one MSM); vector j's buckets are [j * nb / k, (j + 1) * nb / k)
 };
 
 // The sorted state (entries, counts, offsets, tasks) the last MSM left behind.  A following MSM over
@@ -114,7 +119,7 @@ struct MsmCfg {
 // wireValuesB — skips its sort phase and accumulates over these lists with its own bases.
 struct MsmSorted {
   const void* scalars = nullptr;
-  size_t n = 0;
+  size_t n = 0, k = 0, ld = 0;
   int c = 0;
   uint32_t bstride = 0, ent_stride = 0, ent_off = 0;
   int par = 0;

@@ -66,12 +66,14 @@ int msm_pick_table_window(size_t n) {
 // ------------------------------------------------------------------------------ kernels
 // The two-level counting sort (msm_sort.cuh): each kernel runs the header's steps thread by thread between barriers.
 
+// Passes 1 and 3 come in two instances: BATCH = false (one scalar vector) and true (k vectors, msm_sort.cuh).
 // pass 1: coarse count.  s[SORT_BINS] counts the CTA's entries (-> totals[3], which drives the task size)
+template <bool BATCH>
 __global__ void __launch_bounds__(SORT_CTA) k_sort_coarse_count(const SortArgs A) {
   __shared__ uint32_t s[SORT_BINS + 1];
   sort_coarse_init(A, threadIdx.x, s);
   __syncthreads();
-  sort_coarse_count(A, blockIdx.x, threadIdx.x, s);
+  sort_coarse_count<BATCH>(A, blockIdx.x, threadIdx.x, s);
   __syncthreads();
   sort_coarse_flush(A, threadIdx.x, s);
 }
@@ -116,6 +118,7 @@ __global__ void __launch_bounds__(SORT_CTA) k_sort_bins(const SortArgs A) {
 }
 
 // pass 3: coarse partition into part[] (bin order), staged in dynamic shared memory (sort_part_smem bytes)
+template <bool BATCH>
 __global__ void __launch_bounds__(SORT_CTA) k_sort_coarse_part(const SortArgs A) {
   extern __shared__ __align__(8) unsigned char sort_smem[];
   SortItem* stage = reinterpret_cast<SortItem*>(sort_smem);
@@ -124,12 +127,12 @@ __global__ void __launch_bounds__(SORT_CTA) k_sort_coarse_part(const SortArgs A)
   uint32_t* glob = loc + SORT_BINS;
   for (uint32_t b = threadIdx.x; b < SORT_BINS; b += SORT_CTA) s[b] = 0;
   __syncthreads();
-  sort_part_count(A, blockIdx.x, threadIdx.x, s);
+  sort_part_count<BATCH>(A, blockIdx.x, threadIdx.x, s);
   __syncthreads();
   sort_block_scan<SORT_BINS>(s);
   sort_part_reserve(A, threadIdx.x, s, loc, glob);
   __syncthreads();
-  sort_part_stage(A, blockIdx.x, threadIdx.x, s, stage);
+  sort_part_stage<BATCH>(A, blockIdx.x, threadIdx.x, s, stage);
   __syncthreads();
   sort_part_write(A, threadIdx.x, s[SORT_BINS], loc, glob, stage);
 }
@@ -372,10 +375,11 @@ __global__ void __launch_bounds__(TASK_CTA) k_task_order(const uint32_t* __restr
   if (valid) task_order[h[bin] + rank] = t;
 }
 
-int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, SortItem* part,
+int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, uint32_t ld, SortItem* part,
                    uint32_t* bins, uint32_t* counts, uint32_t* offsets, uint32_t* cursor, uint32_t* task_off,
                    uint32_t* totals, uint32_t* entries, uint32_t* task_bucket, uint32_t* task_order, uint32_t max_tasks,
                    uint32_t* scan_scratch, int* ev) {
+  const bool batch = cfg.k > 1;
   cudaStream_t st = ctx->stream;
   auto mark = [&]() { if (ev && *ev < 18) cudaEventRecord(ctx->ev[(*ev)++], st); };
   // B200G16_SORT_TRACE=1: an event after every operation of this phase, printed (and the stream drained) at its end —
@@ -389,7 +393,10 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
   auto tr = [&]() { if (trace && nt < 16) cudaEventRecord(tev[nt++], st); };
   SortArgs A;
   A.scalars = d_scalars;
-  A.n = n;
+  A.n = n * cfg.k;   // points of all vectors (msm_enqueue keeps n * k * W below 2^32)
+  A.vn = batch ? n : 0u;
+  A.ld = ld;
+  A.vstride = cfg.nb / cfg.k;
   A.c = cfg.c;
   A.W = cfg.W;
   A.bstride = cfg.bstride;
@@ -413,13 +420,14 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
   A.cursor = cursor;
   A.entries = entries;
   A.totals = totals;
-  const unsigned max_tiles = (unsigned)sort_max_tiles(A.nbins, (size_t)n * cfg.W);
+  const unsigned max_tiles = (unsigned)sort_max_tiles(A.nbins, (size_t)A.n * cfg.W);
   mark();
   tr();
   B200_CUDA(cudaMemsetAsync(counts, 0, (size_t)cfg.nb * sizeof(uint32_t), st));
   B200_CUDA(cudaMemsetAsync(totals, 0, 16 * sizeof(uint32_t), st));
   B200_CUDA(cudaMemsetAsync(A.bin_count, 0, SORT_BINS * sizeof(uint32_t), st));
-  k_sort_coarse_count<<<cdiv(n, SORT_POINTS), SORT_CTA, 0, st>>>(A);
+  if (batch) k_sort_coarse_count<true><<<cdiv(A.n, SORT_POINTS), SORT_CTA, 0, st>>>(A);
+  else k_sort_coarse_count<false><<<cdiv(A.n, SORT_POINTS), SORT_CTA, 0, st>>>(A);
   tr();
   k_pick_seg<<<1, 1, 0, st>>>(totals, cfg.nb, cfg.target_tasks);
   tr();
@@ -427,10 +435,12 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
   k_sort_bins<<<1, SORT_CTA, 0, st>>>(A);
   tr();
   if (!ctx->sort_smem_set) {   // once per context (= device)
-    B200_CUDA(cudaFuncSetAttribute(k_sort_coarse_part, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_part_smem()));
+    B200_CUDA(cudaFuncSetAttribute(k_sort_coarse_part<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_part_smem()));
+    B200_CUDA(cudaFuncSetAttribute(k_sort_coarse_part<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_part_smem()));
     ctx->sort_smem_set = true;
   }
-  k_sort_coarse_part<<<cdiv(n, A.part_points), SORT_CTA, sort_part_smem(), st>>>(A);
+  if (batch) k_sort_coarse_part<true><<<cdiv(A.n, A.part_points), SORT_CTA, sort_part_smem(), st>>>(A);
+  else k_sort_coarse_part<false><<<cdiv(A.n, A.part_points), SORT_CTA, sort_part_smem(), st>>>(A);
   tr();
   k_sort_fine_count<<<max_tiles, SORT_CTA, 0, st>>>(A);
   tr();
@@ -457,7 +467,7 @@ int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uin
     cudaStreamSynchronize(st);
     static const char* what[] = {"memsets + coarse count", "k_pick_seg", "bin scan", "coarse partition", "fine count",
                                  "scan x3", "fine place", "k_tasks", "memset + k_task_hist", "k_task_scan + k_task_order"};
-    fprintf(stderr, "[sort trace n=%u c=%d F=%d]", n, cfg.c, A.F);
+    fprintf(stderr, "[sort trace n=%u c=%d F=%d]", A.n, cfg.c, A.F);
     for (int i = 0; i + 1 < nt; i++) {
       float ms = 0;
       cudaEventElapsedTime(&ms, tev[i], tev[i + 1]);

@@ -38,9 +38,9 @@ namespace b200 {
 // msm_common.cu
 int msm_num_windows(int c);
 int msm_pick_window(size_t n);
-// two-level counting sort into bucket order + task table on ctx->stream (13 kernels + 4 memsets).
-// part: n * W items; bins: sort_bin_bytes(bins, n * W) bytes
-int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, SortItem* part,
+// two-level counting sort into bucket order + task table on ctx->stream (13 kernels + 4 memsets), for cfg.k vectors of
+// n scalars, vector j at d_scalars + j * ld.  part: k * n * W items; bins: sort_bin_bytes(bins, k * n * W) bytes
+int msm_sort_phase(b200g16_ctx* ctx, const MsmCfg& cfg, const Fr* d_scalars, uint32_t n, uint32_t ld, SortItem* part,
                    uint32_t* bins, uint32_t* counts, uint32_t* offsets, uint32_t* cursor, uint32_t* task_off,
                    uint32_t* totals, uint32_t* entries, uint32_t* task_bucket, uint32_t* task_order, uint32_t max_tasks,
                    uint32_t* scan_scratch, int* ev);
@@ -303,32 +303,74 @@ constexpr size_t AFF_AUTO_MIN_ENTRIES = (size_t)40 << 20;
 constexpr int MSM_SLOTS = 8;           // independent result slots (a prove enqueues 5 MSMs back to back); ctx->ev_slot has as many
 constexpr int MSM_MAX_WINDOWS = 130;
 
+// Batch MSMs (k scalar vectors over one bases vector, msm_enqueue with k > 1).  One call holds at most 2^23 buckets
+// (k * nb: sort_fine_bits <= 12, so the fine passes count in shared memory) and fewer than 2^32 entries (k * n * W:
+// offsets, cursors and tasks are 32-bit).  A larger k is split into sub-batches of msm_batch_max vectors.
+constexpr uint64_t MSM_BATCH_MAX_BUCKETS = 1ull << 23;
+constexpr uint64_t MSM_BATCH_MAX_ENTRIES = (1ull << 32) - 1;
+
+// window width and windows the library uses for an n-point MSM (with a table: the table's)
+inline int msm_window_for(const b200g16_ctx* ctx, const MsmTable* tab, size_t n) {
+  return tab ? tab->c : (ctx->msm_window_override ? ctx->msm_window_override : msm_pick_window(n));
+}
+
+// vectors of n points one batch enqueue may hold (>= 1; 1 means the single-MSM path)
+inline size_t msm_batch_max(int c, bool table, size_t n) {
+  if (c < 2 || c > 24) return 1;
+  const int W = msm_num_windows(c);
+  const uint64_t nb = (uint64_t)(table ? 1 : W) << (c - 1);
+  uint64_t k = MSM_BATCH_MAX_BUCKETS / nb;
+  if (n) k = std::min<uint64_t>(k, MSM_BATCH_MAX_ENTRIES / ((uint64_t)n * W));
+  return k < 1 ? 1 : (size_t)k;
+}
+
+// Grow-only pinned staging of batch window sums: MSM_SLOTS slots of `slot_bytes`.  Called by a batch entry point before
+// its first enqueue, when none of its slots is pending (every batch call drains its streams before it returns).
+inline int msm_batch_stage(b200g16_ctx* ctx, size_t slot_bytes) {
+  MsmWorkspace& ws = ctx->msm;
+  if (ws.batch_slot >= slot_bytes) return 0;
+  if (ws.batch_pinned) B200_CUDA(cudaFreeHost(ws.batch_pinned));
+  ws.batch_pinned = nullptr;
+  ws.batch_slot = 0;
+  B200_CUDA(cudaMallocHost(&ws.batch_pinned, MSM_SLOTS * slot_bytes));
+  ws.batch_slot = slot_bytes;
+  return 0;
+}
+
 // Enqueue one MSM on ctx->stream; its W window sums land in pinned slot `slot` once the stream
 // drains.  No host synchronisation.  record_events: fill ctx->ev for b200g16_last_timings.
 // share_sort: the caller guarantees that d_scalars still holds what the previous enqueue saw under the
 // same pointer; if that MSM used the same decomposition its sorted lists are reused (no sort phase).
+// k > 1: k MSMs of n scalars each over the same bases, vector j at d_scalars + j * ld, in one pass of every kernel:
+// vector j owns the bucket sets [j * Wr, (j + 1) * Wr) and its window sums land at items [j * Wr, (j + 1) * Wr) of slot
+// `slot` of the batch staging (msm_batch_stage: k * Wr items per slot).  k must not exceed msm_batch_max.
 template <class F>
-int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab, const Fr* d_scalars, size_t n, int slot,
-                MsmCfg* cfg_out, bool record_events, bool share_sort = false) {
+int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab, const Fr* d_scalars, size_t n, size_t k,
+                size_t ld, int slot, MsmCfg* cfg_out, bool record_events, bool share_sort = false) {
   MsmCfg cfg;
   memset(&cfg, 0, sizeof(cfg));
+  cfg.k = (uint32_t)k;
   *cfg_out = cfg;
   if (slot < 0 || slot >= MSM_SLOTS) return fail(B200G16_ERR_ARG, "msm: bad slot");
+  if (k == 0 || k >= (1ull << 32) || ld < n || ld >= (1ull << 32)) return fail(B200G16_ERR_ARG, "msm: bad batch shape");
   if (n == 0) return 0;  // cfg.W == 0 marks "infinity"
   if (n >= (1ull << 31)) return fail(B200G16_ERR_ARG, "msm: n=%zu too large", n);
-  cfg.c = tab ? tab->c : (ctx->msm_window_override ? ctx->msm_window_override : msm_pick_window(n));
+  cfg.c = msm_window_for(ctx, tab, n);
   if (cfg.c < 2 || cfg.c > 24) return fail(B200G16_ERR_ARG, "msm: window %d out of range", cfg.c);
   cfg.W = msm_num_windows(cfg.c);
   if (tab && tab->W != cfg.W) return fail(B200G16_ERR_STATE, "msm: window table has %d rows, want %d", tab->W, cfg.W);
   cfg.nbw = 1u << (cfg.c - 1);
   cfg.Wr = tab ? 1 : cfg.W;
-  cfg.nb = cfg.nbw * (uint32_t)cfg.Wr;
+  if (k > 1 && k > msm_batch_max(cfg.c, tab != nullptr, n))
+    return fail(B200G16_ERR_ARG, "msm: %zu vectors of %zu points exceed one batch call", k, n);
+  cfg.nb = cfg.nbw * (uint32_t)cfg.Wr * (uint32_t)k;
   cfg.bstride = tab ? 0u : cfg.nbw;
   cfg.ent_stride = tab ? tab->stride : 0u;
   cfg.ent_off = tab ? tab->off : 0u;
   if (tab && (double)tab->stride * cfg.W >= 2.0e9) return fail(B200G16_ERR_ARG, "msm: window table too large to index");
   if ((double)n * cfg.W >= 4.0e9) return fail(B200G16_ERR_ARG, "msm: n*W overflows 32-bit entry index");
-  size_t m_max = n * (size_t)cfg.W;
+  size_t m_max = n * k * (size_t)cfg.W;
+  const uint32_t R = (uint32_t)(k * cfg.Wr);   // bucket sets (window sums) of all vectors
   cfg.target_tasks = (uint32_t)ctx->sm_count * 2048u;  // ~4 waves of 512 resident threads per SM
   cfg.ch = 1;   // (unused since the tree reduction: one bucket per leaf)
   cfg.nch = cfg.nbw;
@@ -340,7 +382,7 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
   ctx->msm_parity = (par + 1) % MSM_SETS;
   const MsmSorted& ls = ctx->last_sort;
   const bool reuse = share_sort && ls.valid && ls.par != par && ls.scalars == (const void*)d_scalars && ls.n == n &&
-                     ls.c == cfg.c && ls.bstride == cfg.bstride && ls.ent_stride == cfg.ent_stride &&
+                     ls.k == k && ls.ld == ld && ls.c == cfg.c && ls.bstride == cfg.bstride && ls.ent_stride == cfg.ent_stride &&
                      ls.ent_off == cfg.ent_off;
   const int spar = reuse ? ls.par : par;  // set holding the sorted state: counts, offsets, tasks, totals
   const int sort_F = sort_fine_bits(cfg.nb);
@@ -357,7 +399,7 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
     B200_TRY(ws.tasks[q].ensure(2 * max_tasks * sizeof(uint32_t)));  // task_bucket, task_order
     B200_TRY(ws.partials[q].ensure(max_tasks * sizeof(XYZZ<F>)));
     // dense bucket array of the reduction tree + two ping-pong rows of c terms per window for the sum passes
-    B200_TRY(ws.chunks[q].ensure(((size_t)cfg.Wr * cfg.nbw + 2 * (size_t)cfg.Wr * (cfg.c + 1)) * sizeof(XYZZ<F>)));
+    B200_TRY(ws.chunks[q].ensure(((size_t)R * cfg.nbw + 2 * (size_t)R * (cfg.c + 1)) * sizeof(XYZZ<F>)));
   }
   const size_t slot_bytes = MSM_MAX_WINDOWS * sizeof(XYZZ<Fp2>);
   if (ws.pinned_cap < MSM_SLOTS * slot_bytes) {
@@ -366,6 +408,8 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
     ws.pinned_cap = MSM_SLOTS * slot_bytes;
   }
   if (cfg.W > MSM_MAX_WINDOWS - 2) return fail(B200G16_ERR_ARG, "msm: too many windows");
+  if (k > 1 && ws.batch_slot < (size_t)R * sizeof(XYZZ<F>)) return fail(B200G16_ERR_STATE, "msm: batch staging too small");
+  char* stage = k > 1 ? (char*)ws.batch_pinned + (size_t)slot * ws.batch_slot : (char*)ws.pinned + (size_t)slot * slot_bytes;
 
   uint32_t* counts = ws.counts[spar].as<uint32_t>();
   uint32_t* offsets = counts + cfg.nb;
@@ -393,12 +437,14 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
     if (rd >= 0 && ctx->tail_pending[rd]) B200_CUDA(cudaStreamWaitEvent(st, ctx->ev_tail[rd], 0));
     ctx->sort_reader[par] = -1;
     ctx->last_sort.valid = false;
-    B200_TRY(msm_sort_phase(ctx, cfg, d_scalars, n32, part, ws.bins.as<uint32_t>(), counts, offsets, cursor, task_off, totals, entries,
+    B200_TRY(msm_sort_phase(ctx, cfg, d_scalars, n32, (uint32_t)ld, part, ws.bins.as<uint32_t>(), counts, offsets, cursor, task_off, totals, entries,
                             task_bucket, task_order, (uint32_t)max_tasks,
                             reinterpret_cast<uint32_t*>(ws.misc[par].as<char>() + scan_off),
                             record_events ? &ev : nullptr));
     ctx->last_sort.scalars = d_scalars;
     ctx->last_sort.n = n;
+    ctx->last_sort.k = k;
+    ctx->last_sort.ld = ld;
     ctx->last_sort.c = cfg.c;
     ctx->last_sort.bstride = cfg.bstride;
     ctx->last_sort.ent_stride = cfg.ent_stride;
@@ -461,25 +507,25 @@ int msm_enqueue(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab,
   // threads per CTA measure 1.75 / 1.77 / 2.07 / 1.78 ms for the whole reduction at c = 20, profiles/r02w_g2_reduce_block.jsonl
   // — occupancy is not its lever.)
   constexpr unsigned rb = 128u;
-  const unsigned g1 = cdiv((size_t)cfg.Wr * (cfg.nbw >> 1), rb);
-  if (inl) k_reduce_first<F, CAN_INL><<<g1, rb, 0, tail>>>(partials, counts, task_off, (uint32_t)cfg.Wr, cfg.nbw, chunks);
-  else k_reduce_first<F, false><<<g1, rb, 0, tail>>>(partials, counts, task_off, (uint32_t)cfg.Wr, cfg.nbw, chunks);
+  // R = k * Wr bucket sets, nbw apart: vector j's set w is set j * Wr + w (key j * vstride + w * bstride + |d| - 1)
+  const unsigned g1 = cdiv((size_t)R * (cfg.nbw >> 1), rb);
+  if (inl) k_reduce_first<F, CAN_INL><<<g1, rb, 0, tail>>>(partials, counts, task_off, R, cfg.nbw, chunks);
+  else k_reduce_first<F, false><<<g1, rb, 0, tail>>>(partials, counts, task_off, R, cfg.nbw, chunks);
   int sum_levels = 2;
   for (uint32_t l = 2; l < l0 && l <= nlev; l++, sum_levels++) {
-    const unsigned gl = cdiv((size_t)cfg.Wr * l * (cfg.nbw >> l), rb);
-    if (inl) k_reduce_level<F, CAN_INL><<<gl, rb, 0, tail>>>(chunks, (uint32_t)cfg.Wr, cfg.nbw, l);
-    else k_reduce_level<F, false><<<gl, rb, 0, tail>>>(chunks, (uint32_t)cfg.Wr, cfg.nbw, l);
+    const unsigned gl = cdiv((size_t)R * l * (cfg.nbw >> l), rb);
+    if (inl) k_reduce_level<F, CAN_INL><<<gl, rb, 0, tail>>>(chunks, R, cfg.nbw, l);
+    else k_reduce_level<F, false><<<gl, rb, 0, tail>>>(chunks, R, cfg.nbw, l);
   }
-  XYZZ<F>* cur = chunks + (size_t)cfg.Wr * cfg.nbw;   // Wr window sums behind the tree
-  if (inl_tail) k_reduce_tail<F, CAN_INL><<<(unsigned)cfg.Wr, REDUCE_TAIL_THREADS, 0, tail>>>(chunks, cfg.nbw, nlev, l0 > nlev ? nlev + 1 : l0, cur);
-  else k_reduce_tail<F, false><<<(unsigned)cfg.Wr, REDUCE_TAIL_THREADS, 0, tail>>>(chunks, cfg.nbw, nlev, l0 > nlev ? nlev + 1 : l0, cur);
+  XYZZ<F>* cur = chunks + (size_t)R * cfg.nbw;   // R window sums behind the tree
+  if (inl_tail) k_reduce_tail<F, CAN_INL><<<R, REDUCE_TAIL_THREADS, 0, tail>>>(chunks, cfg.nbw, nlev, l0 > nlev ? nlev + 1 : l0, cur);
+  else k_reduce_tail<F, false><<<R, REDUCE_TAIL_THREADS, 0, tail>>>(chunks, cfg.nbw, nlev, l0 > nlev ? nlev + 1 : l0, cur);
   const int merge_levels = 3;
-  windows = cur;  // Wr items
+  windows = cur;  // R items
   if (record_events && ev < 18) cudaEventRecord(ctx->ev[ev++], tail);
   ctx->launches += merge_levels + sum_levels;
   B200_CUDA(cudaGetLastError());
-  B200_CUDA(cudaMemcpyAsync((char*)ws.pinned + (size_t)slot * slot_bytes, windows, (size_t)cfg.Wr * sizeof(XYZZ<F>),
-                            cudaMemcpyDeviceToHost, tail));
+  B200_CUDA(cudaMemcpyAsync(stage, windows, (size_t)R * sizeof(XYZZ<F>), cudaMemcpyDeviceToHost, tail));
   B200_CUDA(cudaEventRecord(ctx->ev_tail[par], tail));
   B200_CUDA(cudaEventRecord(ctx->ev_slot[slot], tail));
   ctx->tail_pending[par] = true;
@@ -499,13 +545,15 @@ inline int msm_join(b200g16_ctx* ctx) {
   return 0;
 }
 
-// After the stream has drained: Horner over the window sums of `slot` on the host,
+// After the stream has drained: Horner over the window sums of `slot` (vector j of a batch) on the host,
 // acc = sum_w 2^(c w) * S_w, then one inversion to the affine normal form.
 template <class F>
-int msm_collect(b200g16_ctx* ctx, int slot, const MsmCfg& cfg, Affine<F>* out) {
+int msm_collect(b200g16_ctx* ctx, int slot, const MsmCfg& cfg, Affine<F>* out, size_t j = 0) {
   if (cfg.W == 0) { *out = Affine<F>::inf(); return 0; }
   const size_t slot_bytes = MSM_MAX_WINDOWS * sizeof(XYZZ<Fp2>);
-  const XYZZ<F>* hw = reinterpret_cast<const XYZZ<F>*>((const char*)ctx->msm.pinned + (size_t)slot * slot_bytes);
+  const XYZZ<F>* hw = cfg.k > 1 ? reinterpret_cast<const XYZZ<F>*>((const char*)ctx->msm.batch_pinned + (size_t)slot * ctx->msm.batch_slot) +
+                                      j * cfg.Wr
+                                : reinterpret_cast<const XYZZ<F>*>((const char*)ctx->msm.pinned + (size_t)slot * slot_bytes);
   XYZZ<F> acc = hw[cfg.Wr - 1];
   for (int w = cfg.Wr - 2; w >= 0; w--) {
     for (int k = 0; k < cfg.c; k++) acc.dbl();
@@ -527,7 +575,7 @@ int msm_device(b200g16_ctx* ctx, const Affine<F>* d_bases, const MsmTable* tab, 
                Affine<F>* out) {
   MsmCfg cfg;
   ctx->timings.n = 0;
-  B200_TRY(msm_enqueue<F>(ctx, d_bases, tab, d_scalars, n, 0, &cfg, true));
+  B200_TRY(msm_enqueue<F>(ctx, d_bases, tab, d_scalars, n, 1, n, 0, &cfg, true));
   B200_TRY(msm_join(ctx));
   B200_CUDA(cudaStreamSynchronize(ctx->stream));
   msm_resolve_timings(ctx);

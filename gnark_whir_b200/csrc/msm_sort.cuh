@@ -29,8 +29,16 @@
 // With F > SORT_FINE_MAX_BITS (plain windows forced to c >= 20: tens of millions of buckets) passes 4 and 6 count
 // and place with one global atomic per entry; no width the library picks for itself goes there.
 //
+// Batch (BATCH = true, msm_enqueue with k > 1 scalar vectors over one bases vector): the point index q of passes 1 and
+// 3 runs over [0, k * vn) and splits as j = q / vn (vector) and i = q - j * vn (point); the scalar is scalars[j * ld + i]
+// and canon[q] its canonical form.  Every key gains j * vstride (vector j's own bucket sets, vstride = Wr * nbw), the
+// value is that of point i alone, so every vector gathers the same bases / table rows and passes 2, 4 and 6 (and
+// everything after the sort) see nothing but more buckets.  The single-vector kernels are the BATCH = false instances,
+// which read none of the batch fields (vn == 0 there means one vector).
+//
 // Everything below is plain C++ over field.cuh, run by the kernels thread by thread between barriers, so
-// tests/host_harness/sort_host.cc runs the same steps CTA by CTA on the CPU against a direct counting sort.
+// tests/host_harness/sort_host.cc and sort_batch_host.cc run the same steps CTA by CTA on the CPU against a direct
+// counting sort.
 #pragma once
 #include "field.cuh"
 
@@ -73,6 +81,10 @@ struct SortArgs {
   uint32_t* cursor;      // per bucket: offsets, advanced by pass 6
   uint32_t* entries;     // [n * W]: values in bucket order
   uint32_t* totals;
+  // batch fields (read by the BATCH instances only; appended so the single-vector kernels' parameters keep their offsets)
+  uint32_t vn;       // points per vector (0: one vector, n points)
+  uint32_t ld;       // scalar row stride in elements (>= vn)
+  uint32_t vstride;  // buckets per vector
 };
 
 // smallest F with at most SORT_BINS bins
@@ -121,9 +133,23 @@ B200_HD void sort_recode(const uint32_t limbs[9], int c, int W, Fn&& fn) {
   }
 }
 
-// fn(key, val) for every nonzero digit of scalar i, given in canonical form
-template <class Fn>
-B200_HD void sort_entries(const SortArgs& A, const Fr& s, uint32_t i, Fn&& fn) {
+// point q -> (vector j, point i of that vector) and the scalar's index in A.scalars
+template <bool BATCH>
+B200_HD size_t sort_point(const SortArgs& A, uint32_t q, uint32_t& i, uint32_t& j) {
+  if constexpr (BATCH) {
+    j = q / A.vn;
+    i = q - j * A.vn;
+    return (size_t)j * A.ld + i;
+  } else {
+    j = 0;
+    i = q;
+    return q;
+  }
+}
+
+// fn(key, val) for every nonzero digit of scalar i of vector j, given in canonical form
+template <bool BATCH = false, class Fn>
+B200_HD void sort_entries(const SortArgs& A, const Fr& s, uint32_t i, uint32_t j, Fn&& fn) {
   uint32_t limbs[9];
 #pragma unroll
   for (int k = 0; k < 8; k++) limbs[k] = s.l[k];
@@ -132,8 +158,13 @@ B200_HD void sort_entries(const SortArgs& A, const Fr& s, uint32_t i, Fn&& fn) {
     if (d == 0) return;
     const uint32_t neg = d < 0;
     const uint32_t mag = neg ? (uint32_t)(-d) : (uint32_t)d;
-    fn((uint32_t)w * A.bstride + mag - 1, (((uint32_t)w * A.ent_stride + A.ent_off + i) << 1) | neg);
+    const uint32_t key = (uint32_t)w * A.bstride + mag - 1;
+    fn(BATCH ? j * A.vstride + key : key, (((uint32_t)w * A.ent_stride + A.ent_off + i) << 1) | neg);
   });
+}
+template <class Fn>
+B200_HD void sort_entries(const SortArgs& A, const Fr& s, uint32_t i, Fn&& fn) {
+  sort_entries<false>(A, s, i, 0u, fn);
 }
 
 // ---- pass 1: CTA `blk` owns points [blk * SORT_POINTS, +SORT_POINTS); s[SORT_BINS + 1] in shared memory
@@ -143,14 +174,16 @@ B200_HD void sort_coarse_init(const SortArgs& A, uint32_t tid, uint32_t* s) {
 }
 
 // s[bin] += entries;  s[SORT_BINS] += all entries
+template <bool BATCH = false>
 B200_HD void sort_coarse_count(const SortArgs& A, uint32_t blk, uint32_t tid, uint32_t* s) {
   uint32_t nz = 0;
   for (int k = 0; k < SORT_PPT; k++) {
-    const uint32_t i = blk * SORT_POINTS + (uint32_t)k * SORT_CTA + tid;
-    if (i >= A.n) break;
-    const Fr sc = Fr::from_mont(A.scalars[i]);
-    A.canon[i] = sc;
-    sort_entries(A, sc, i, [&](uint32_t key, uint32_t) { sort_add(&s[key >> A.F], 1u); nz++; });
+    const uint32_t q = blk * SORT_POINTS + (uint32_t)k * SORT_CTA + tid;
+    if (q >= A.n) break;
+    uint32_t i, j;
+    const Fr sc = Fr::from_mont(A.scalars[sort_point<BATCH>(A, q, i, j)]);
+    A.canon[q] = sc;
+    sort_entries<BATCH>(A, sc, i, j, [&](uint32_t key, uint32_t) { sort_add(&s[key >> A.F], 1u); nz++; });
   }
   if (nz) sort_add(&s[SORT_BINS], nz);
 }
@@ -171,11 +204,14 @@ constexpr uint32_t SORT_STAGE = 10240;   // staged entries per CTA: 80 KB, two C
 inline uint32_t sort_part_points(int W) { return SORT_STAGE / (uint32_t)W; }
 inline size_t sort_part_smem() { return (3 * (size_t)SORT_BINS + 1) * 4 + SORT_STAGE * sizeof(SortItem); }
 
+template <bool BATCH = false>
 B200_HD void sort_part_count(const SortArgs& A, uint32_t blk, uint32_t tid, uint32_t* s) {
   for (uint32_t k = tid; k < A.part_points; k += SORT_CTA) {
-    const uint32_t i = blk * A.part_points + k;
-    if (i >= A.n) break;
-    sort_entries(A, A.canon[i], i, [&](uint32_t key, uint32_t) { sort_add(&s[key >> A.F], 1u); });
+    const uint32_t q = blk * A.part_points + k;
+    if (q >= A.n) break;
+    uint32_t i, j;
+    sort_point<BATCH>(A, q, i, j);
+    sort_entries<BATCH>(A, A.canon[q], i, j, [&](uint32_t key, uint32_t) { sort_add(&s[key >> A.F], 1u); });
   }
 }
 
@@ -188,11 +224,15 @@ B200_HD void sort_part_reserve(const SortArgs& A, uint32_t tid, const uint32_t* 
   }
 }
 
+template <bool BATCH = false>
 B200_HD void sort_part_stage(const SortArgs& A, uint32_t blk, uint32_t tid, uint32_t* s, SortItem* stage) {
   for (uint32_t k = tid; k < A.part_points; k += SORT_CTA) {
-    const uint32_t i = blk * A.part_points + k;
-    if (i >= A.n) break;
-    sort_entries(A, A.canon[i], i, [&](uint32_t key, uint32_t val) { stage[sort_add(&s[key >> A.F], 1u)] = SortItem{key, val}; });
+    const uint32_t q = blk * A.part_points + k;
+    if (q >= A.n) break;
+    uint32_t i, j;
+    sort_point<BATCH>(A, q, i, j);
+    sort_entries<BATCH>(A, A.canon[q], i, j,
+                        [&](uint32_t key, uint32_t val) { stage[sort_add(&s[key >> A.F], 1u)] = SortItem{key, val}; });
   }
 }
 

@@ -15,6 +15,9 @@
 //   Ar  = A + alpha + r*delta
 //   Bs1 = B1 + beta + s*delta           Bs = B2 + beta2 + s*delta2
 //   Krs = K + Z + (-rs)*delta + s*Ar + r*Bs1
+#include <algorithm>
+#include <thread>
+
 #include "prove.cuh"
 #include "host_copy.cuh"
 
@@ -26,6 +29,17 @@ __global__ void __launch_bounds__(256) k_gather_fr(const Fr* __restrict__ src, c
   if (i >= n) return;
   const uint4* s = reinterpret_cast<const uint4*>(src + idx[i]);
   uint4* d = reinterpret_cast<uint4*>(dst + i);
+  d[0] = __ldg(s);
+  d[1] = __ldg(s + 1);
+}
+
+// Batch prove: row y of the (proof) grid gathers proof y's scalar vector from its witness row.
+__global__ void __launch_bounds__(256) k_gather_fr_rows(const Fr* __restrict__ src, size_t src_stride,
+                                                         const uint32_t* __restrict__ idx, uint32_t n, Fr* __restrict__ dst) {
+  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint4* s = reinterpret_cast<const uint4*>(src + blockIdx.y * src_stride + idx[i]);
+  uint4* d = reinterpret_cast<uint4*>(dst + (size_t)blockIdx.y * n + i);
   d[0] = __ldg(s);
   d[1] = __ldg(s + 1);
 }
@@ -178,10 +192,10 @@ static int prove_enqueue_one(b200g16_ctx* ctx, const b200g16_pk* pk, int i, cons
   if (i < 4) {
     const G1Affine* pts = msm_operand<Fp>(pk->vec[i], 0, &tab, &tp);
     // Bs1 runs over the same scalar vector as Bs2 (wireValuesB): it reuses Bs2's sorted lists
-    return msm_enqueue<Fp>(ctx, pts, tp, scalars, count, i, cfg, false, /*share_sort=*/i == 1);
+    return msm_enqueue<Fp>(ctx, pts, tp, scalars, count, 1, count, i, cfg, false, /*share_sort=*/i == 1);
   }
   const G2Affine* pts = msm_operand<Fp2>(pk->vec[i], 0, &tab, &tp);
-  return msm_enqueue<Fp2>(ctx, pts, tp, scalars, count, i, cfg, false);
+  return msm_enqueue<Fp2>(ctx, pts, tp, scalars, count, 1, count, i, cfg, false);
 }
 
 // Gathers + the four MSMs over witness values — G2 leading: its bucket reduction is the longest tail and
@@ -283,6 +297,189 @@ static int prove_device(b200g16_ctx* ctx, const b200g16_pk* pk, const Fr* d_wire
   return prove_back(ctx, pk, d_a, r, s, out, ev_io);
 }
 
+// ---- batch prove: k proofs of one circuit against one resident pk, in sub-batches of m proofs.  Per sub-batch:
+// gathers of the m x (A, B, K) scalar rows, the four witness MSMs as batch MSMs (k = m, B1 on B2's sorted lists),
+// computeH per proof on rows j * N of m x N buffers, one batch Z MSM over the m h rows (ld = N), one synchronisation,
+// then the host assembly spread over threads.  The delta multiples of all k proofs start on those threads before any
+// GPU work is enqueued.
+
+// fn(i) for i < count on min(count, hardware threads, 16) threads (the caller's thread included); false when a thread
+// could not be started (the started ones are joined, and the work is not complete).
+template <class Fn>
+static bool host_parallel(size_t count, Fn fn) {
+  const size_t hw = std::max(1u, std::thread::hardware_concurrency());
+  const size_t T = std::min<size_t>({count, hw, 16});
+  if (T <= 1) { for (size_t i = 0; i < count; i++) fn(i); return true; }
+  std::vector<std::thread> th;
+  bool ok = true;
+  try {
+    for (size_t t = 1; t < T; t++)
+      th.emplace_back([&, t]() { for (size_t i = t; i < count; i += T) fn(i); });
+  } catch (...) {
+    ok = false;
+  }
+  if (ok)
+    for (size_t i = 0; i < count; i += T) fn(i);
+  for (auto& x : th) x.join();
+  return ok;
+}
+
+// proofs per sub-batch: every one of the five MSMs fits one batch call (msm_batch_max); 1 = the single-prove path.
+// *slot_bytes: the batch staging one of those MSMs needs per proof at most.
+static size_t prove_batch_max(const b200g16_ctx* ctx, const b200g16_pk* pk, size_t* slot_bytes) {
+  const size_t n[5] = {pk->n_idx[0], pk->n_idx[1], pk->n_idx[2], pk->n_z, pk->n_idx[1]};
+  size_t m = SIZE_MAX;
+  *slot_bytes = 0;
+  for (int i = 0; i < 5; i++) {
+    MsmTable tab;
+    const MsmTable* tp = nullptr;
+    if (i < 4) msm_operand<Fp>(pk->vec[i], 0, &tab, &tp);
+    else msm_operand<Fp2>(pk->vec[i], 0, &tab, &tp);
+    const int c = msm_window_for(ctx, tp, n[i]);
+    m = std::min(m, msm_batch_max(c, tp != nullptr, n[i]));
+    const size_t wr = tp ? 1 : (size_t)msm_num_windows(c);
+    *slot_bytes = std::max(*slot_bytes, wr * (i < 4 ? sizeof(XYZZ<Fp>) : sizeof(XYZZ<Fp2>)));
+  }
+  return m;
+}
+
+// One sub-batch of m >= 2 proofs on device rows: d_wires m x n_wires, d_a/b/c m x N (h is left in the d_a rows).
+// abc(&ready) runs once the witness MSMs are enqueued: the host path starts the a, b, c uploads there, under those
+// MSMs, and returns the event after which the rows are in place (nullptr: already there).  dm: the proofs' delta
+// multiples (threads still filling them are joined by `dm_wait` before the assembly).  ms[4] accumulates the phase times.
+template <class Abc, class Wait>
+static int prove_batch_sub(b200g16_ctx* ctx, const b200g16_pk* pk, size_t m, const Fr* d_wires, Fr* d_a, Fr* d_b,
+                           Fr* d_c, Abc&& abc, const Fr* r, const Fr* s, const DeltaMultiples* dm,
+                           Wait&& dm_wait, b200g16_proof* out, float* ms) {
+  cudaStream_t st = ctx->stream;
+  const size_t N = (size_t)1 << pk->log2n;
+  cudaEventRecord(ctx->ev[0], st);
+  const size_t tot = pk->n_idx[0] + pk->n_idx[1] + pk->n_idx[2];
+  B200_TRY(ctx->io_b.ensure((tot ? tot * m : 1) * sizeof(Fr)));
+  Fr* sv[3];
+  sv[0] = ctx->io_b.as<Fr>();
+  sv[1] = sv[0] + m * pk->n_idx[0];
+  sv[2] = sv[1] + m * pk->n_idx[1];
+  for (int i = 0; i < 3; i++)
+    if (pk->n_idx[i]) {
+      k_gather_fr_rows<<<dim3(cdiv(pk->n_idx[i], 256), (unsigned)m), 256, 0, st>>>(d_wires, pk->n_wires, pk->d_idx[i],
+                                                                                   (uint32_t)pk->n_idx[i], sv[i]);
+      ctx->launches++;
+    }
+  cudaEventRecord(ctx->ev[1], st);
+  MsmCfg cfg[5];
+  const size_t cnt[5] = {pk->n_idx[0], pk->n_idx[1], pk->n_idx[2], 0, pk->n_idx[1]};
+  const Fr* scal[5] = {sv[0], sv[1], sv[2], nullptr, sv[1]};
+  for (int i : {4, 1, 0, 2}) {
+    MsmTable tab;
+    const MsmTable* tp = nullptr;
+    if (i < 4) {
+      const G1Affine* pts = msm_operand<Fp>(pk->vec[i], 0, &tab, &tp);
+      B200_TRY(msm_enqueue<Fp>(ctx, pts, tp, scal[i], cnt[i], m, cnt[i], i, &cfg[i], false, /*share_sort=*/i == 1));
+    } else {
+      const G2Affine* pts = msm_operand<Fp2>(pk->vec[i], 0, &tab, &tp);
+      B200_TRY(msm_enqueue<Fp2>(ctx, pts, tp, scal[i], cnt[i], m, cnt[i], i, &cfg[i], false));
+    }
+  }
+  cudaEventRecord(ctx->ev[2], st);
+  cudaEvent_t abc_ready = nullptr;
+  B200_TRY(abc(&abc_ready));
+  if (abc_ready) B200_CUDA(cudaStreamWaitEvent(st, abc_ready, 0));
+  for (size_t j = 0; j < m; j++) B200_TRY(compute_h_device(ctx, d_a + j * N, d_b + j * N, d_c + j * N, (int)pk->log2n, false));
+  cudaEventRecord(ctx->ev[3], st);
+  {
+    MsmTable tab;
+    const MsmTable* tp = nullptr;
+    const G1Affine* pts = msm_operand<Fp>(pk->vec[3], 0, &tab, &tp);
+    B200_TRY(msm_enqueue<Fp>(ctx, pts, tp, d_a + pk->off_z, pk->n_z, m, N, 3, &cfg[3], false));
+  }
+  B200_TRY(msm_join(ctx));
+  cudaEventRecord(ctx->ev[4], st);
+  B200_CUDA(cudaStreamSynchronize(st));
+  for (int i = 0; i < 4; i++) {
+    float t = 0;
+    cudaEventElapsedTime(&t, ctx->ev[i], ctx->ev[i + 1]);
+    ms[i] += t;
+  }
+  dm_wait();
+  const bool ok = host_parallel(m, [&](size_t j) {
+    G1Affine A, B1, K, Z;
+    G2Affine B2;
+    msm_collect<Fp>(ctx, 0, cfg[0], &A, j);
+    msm_collect<Fp>(ctx, 1, cfg[1], &B1, j);
+    msm_collect<Fp>(ctx, 2, cfg[2], &K, j);
+    msm_collect<Fp>(ctx, 3, cfg[3], &Z, j);
+    msm_collect<Fp2>(ctx, 4, cfg[4], &B2, j);
+    b200g16_proof* o = out + j;
+    memset(o, 0, sizeof(*o));
+    prove_finish_host(pk, dm[j], A, B1, K, Z, B2, r[j], s[j], o);
+    memcpy(o->msm_a, &A, 64);
+    memcpy(o->msm_b1, &B1, 64);
+    memcpy(o->msm_k, &K, 64);
+    memcpy(o->msm_z, &Z, 64);
+    memcpy(o->msm_b2, &B2, 128);
+  });
+  if (!ok) return fail(B200G16_ERR_STATE, "prove_batch: could not start the host assembly threads");
+  return 0;
+}
+
+// The shared body of both entry points.  rows(j0, m, &wires, &a, &b, &c) gives the device rows of proofs [j0, j0 + m)
+// (the host path uploads the wires there); abc(j0, m, &ready) is prove_batch_sub's abc for that sub-batch.
+template <class Rows, class Abc>
+static int prove_batch_run(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, size_t m_max, size_t slot_bytes,
+                           const uint64_t* r, const uint64_t* s, b200g16_proof* out, Rows&& rows, Abc&& abc) {
+  B200_TRY(msm_batch_stage(ctx, m_max * slot_bytes));
+  std::vector<Fr> fr_r(k), fr_s(k);
+  memcpy(fr_r.data(), r, k * sizeof(Fr));
+  memcpy(fr_s.data(), s, k * sizeof(Fr));
+  std::vector<DeltaMultiples> dm(k);
+  // the delta multiples of all k proofs, on host threads under the GPU's work
+  const size_t T = std::max<size_t>(1, std::min<size_t>({k, (size_t)std::max(1u, std::thread::hardware_concurrency()), 16}));
+  std::vector<std::thread> th;
+  bool started = true;
+  try {
+    for (size_t t = 0; t < T; t++)
+      th.emplace_back([&, t]() { for (size_t i = t; i < k; i += T) dm[i] = delta_multiples(pk, fr_r[i], fr_s[i]); });
+  } catch (...) {
+    started = false;
+  }
+  bool joined = false;
+  auto dm_wait = [&]() { if (!joined) { for (auto& x : th) x.join(); joined = true; } };
+  if (!started) { dm_wait(); return fail(B200G16_ERR_STATE, "prove_batch: could not start the host threads"); }
+  float ms[4] = {0, 0, 0, 0};
+  auto body = [&]() -> int {
+    for (size_t j0 = 0; j0 < k;) {
+      const size_t m = std::min(m_max, k - j0);
+      const Fr *w = nullptr;
+      Fr *a = nullptr, *b = nullptr, *c = nullptr;
+      B200_TRY(rows(j0, m, &w, &a, &b, &c));
+      B200_TRY(prove_batch_sub(ctx, pk, m, w, a, b, c, [&](cudaEvent_t* ready) { return abc(j0, m, ready); },
+                               fr_r.data() + j0, fr_s.data() + j0, dm.data() + j0, dm_wait, out + j0, ms));
+      j0 += m;
+    }
+    return 0;
+  };
+  const int status = body();
+  dm_wait();
+  if (status) {   // leave the ctx usable: whatever is in flight is drained and forgotten
+    msm_join(ctx);
+    cudaStreamSynchronize(ctx->stream);
+    cudaStreamSynchronize(ctx->tail_stream);
+    cudaStreamSynchronize(ctx->copy_stream);
+    ctx->last_sort.valid = false;
+    return status;
+  }
+  for (int i = 0; i < 4; i++) ctx->timings.ms[i] = ms[i];
+  ctx->timings.n = 4;
+  return 0;
+}
+
+static int prove_batch_check(b200g16_ctx* ctx, const b200g16_pk* pk, const char* what) {
+  if (pk->device != ctx->device) return fail(B200G16_ERR_STATE, "%s: pk lives on another device", what);
+  if (pk->partial) return fail(B200G16_ERR_ARG, "%s: a partial (sharded) pk cannot be batch-proved", what);
+  return 0;
+}
+
 }  // namespace b200
 
 using namespace b200;
@@ -344,6 +541,103 @@ int b200g16_prove(b200g16_ctx* ctx, const b200g16_pk* pk, const uint64_t* wires,
   for (int i = 0; i + 1 < ev; i++) cudaEventElapsedTime(&ctx->timings.ms[i], ctx->ev[i], ctx->ev[i + 1]);
   if (h_out) B200_TRY(d2h_copy(ctx, h_out, ctx->ntt.a.p, N * sizeof(Fr), ctx->stream));
   return 0;
+}
+
+int b200g16_prove_batch(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const uint64_t* wires, size_t n_wires,
+                        const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints, const uint64_t* r,
+                        const uint64_t* s, b200g16_proof* proofs_out) {
+  if (!ctx || !pk) return fail(B200G16_ERR_ARG, "prove_batch: null");
+  if (k && (!wires || !a || !b || !c || !r || !s || !proofs_out)) return fail(B200G16_ERR_ARG, "prove_batch: null");
+  B200_TRY(prove_batch_check(ctx, pk, "prove_batch"));
+  if (n_wires != pk->n_wires) return fail(B200G16_ERR_ARG, "prove_batch: %zu wires, pk expects %zu", n_wires, pk->n_wires);
+  const size_t N = (size_t)1 << pk->log2n;
+  if (n_constraints > N) return fail(B200G16_ERR_ARG, "prove_batch: %zu constraints > domain %zu", n_constraints, N);
+  if (k && (n_wires > SIZE_MAX / sizeof(Fr) / k || N > SIZE_MAX / sizeof(Fr) / k))
+    return fail(B200G16_ERR_ARG, "prove_batch: k x n_wires or k x N overflows");
+  if (k == 0) return 0;
+  size_t m_max, slot_bytes;
+  {
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (ctx->prove_active) return fail(B200G16_ERR_STATE, "prove_batch: a prove is open on this ctx");
+    m_max = std::min(k, prove_batch_max(ctx, pk, &slot_bytes));
+  }
+  if (m_max <= 1) {   // one proof per sub-batch: the single prove, proof by proof
+    for (size_t j = 0; j < k; j++)
+      B200_TRY(b200g16_prove(ctx, pk, wires + j * n_wires * 4, n_wires, a + j * n_constraints * 4, b + j * n_constraints * 4,
+                             c + j * n_constraints * 4, n_constraints, r + 4 * j, s + 4 * j, proofs_out + j, nullptr));
+    return 0;
+  }
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  if (ctx->prove_active) return fail(B200G16_ERR_STATE, "prove_batch: a prove is open on this ctx");
+  B200_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream, cs = ctx->copy_stream;
+  B200_TRY(ctx->io_a.ensure((n_wires ? m_max * n_wires : 1) * sizeof(Fr)));
+  DevBuf* bufs[3] = {&ctx->ntt.a, &ctx->ntt.b, &ctx->ntt.c};
+  for (int i = 0; i < 3; i++) B200_TRY(bufs[i]->ensure(m_max * N * sizeof(Fr)));
+  const uint64_t* src[3] = {a, b, c};
+  // As b200g16_prove: the wires first on the main stream (they gate the witness MSMs), and a, b, c on the copy stream
+  // only once those MSMs are enqueued — a copy from pageable memory occupies this thread while it is staged.
+  auto rows = [&](size_t j0, size_t m, const Fr** w, Fr** da, Fr** db, Fr** dc) -> int {
+    if (n_wires) B200_TRY(h2d_copy(ctx, ctx->io_a.p, wires + j0 * n_wires * 4, m * n_wires * sizeof(Fr), st));
+    B200_CUDA(cudaEventRecord(ctx->ev_copy[1], st));
+    *w = ctx->io_a.as<Fr>();
+    *da = ctx->ntt.a.as<Fr>();
+    *db = ctx->ntt.b.as<Fr>();
+    *dc = ctx->ntt.c.as<Fr>();
+    return 0;
+  };
+  auto abc = [&](size_t j0, size_t m, cudaEvent_t* ready) -> int {
+    B200_CUDA(cudaStreamWaitEvent(cs, ctx->ev_copy[1], 0));   // the rows' previous readers (the sub-batch before) are done
+    for (int i = 0; i < 3; i++)
+      for (size_t j = 0; j < m; j++) {
+        char* row = (char*)bufs[i]->p + j * N * sizeof(Fr);
+        if (n_constraints)
+          B200_TRY(h2d_copy(ctx, row, src[i] + (j0 + j) * n_constraints * 4, n_constraints * sizeof(Fr), cs));
+        if (N > n_constraints)
+          B200_CUDA(cudaMemsetAsync(row + n_constraints * sizeof(Fr), 0, (N - n_constraints) * sizeof(Fr), cs));
+      }
+    B200_CUDA(cudaEventRecord(ctx->ev_copy[0], cs));
+    *ready = ctx->ev_copy[0];
+    return 0;
+  };
+  return prove_batch_run(ctx, pk, k, m_max, slot_bytes, r, s, proofs_out, rows, abc);
+}
+
+int b200g16_prove_batch_dev(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const void* d_wires, void* d_a, void* d_b,
+                            void* d_c, const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out) {
+  if (!ctx || !pk) return fail(B200G16_ERR_ARG, "prove_batch_dev: null");
+  if (k && (!d_wires || !d_a || !d_b || !d_c || !r || !s || !proofs_out)) return fail(B200G16_ERR_ARG, "prove_batch_dev: null");
+  B200_TRY(prove_batch_check(ctx, pk, "prove_batch_dev"));
+  const size_t N = (size_t)1 << pk->log2n;
+  if (k && (pk->n_wires > SIZE_MAX / sizeof(Fr) / k || N > SIZE_MAX / sizeof(Fr) / k))
+    return fail(B200G16_ERR_ARG, "prove_batch_dev: k x n_wires or k x N overflows");
+  if (k == 0) return 0;
+  size_t m_max, slot_bytes;
+  {
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (ctx->prove_active) return fail(B200G16_ERR_STATE, "prove_batch_dev: a prove is open on this ctx");
+    m_max = std::min(k, prove_batch_max(ctx, pk, &slot_bytes));
+  }
+  const Fr* W = (const Fr*)d_wires;
+  Fr *A = (Fr*)d_a, *B = (Fr*)d_b, *C = (Fr*)d_c;
+  if (m_max <= 1) {
+    for (size_t j = 0; j < k; j++)
+      B200_TRY(b200g16_prove_dev(ctx, pk, W + j * pk->n_wires, A + j * N, B + j * N, C + j * N, r + 4 * j, s + 4 * j,
+                                 proofs_out + j));
+    return 0;
+  }
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  if (ctx->prove_active) return fail(B200G16_ERR_STATE, "prove_batch_dev: a prove is open on this ctx");
+  B200_CUDA(cudaSetDevice(ctx->device));
+  auto rows = [&](size_t j0, size_t, const Fr** w, Fr** da, Fr** db, Fr** dc) -> int {
+    *w = W + j0 * pk->n_wires;
+    *da = A + j0 * N;
+    *db = B + j0 * N;
+    *dc = C + j0 * N;
+    return 0;
+  };
+  auto abc = [](size_t, size_t, cudaEvent_t* ready) -> int { *ready = nullptr; return 0; };
+  return prove_batch_run(ctx, pk, k, m_max, slot_bytes, r, s, proofs_out, rows, abc);
 }
 
 int b200g16_prove_finish(const b200g16_pk* pk, const uint64_t msm_a[8], const uint64_t msm_b1[8],

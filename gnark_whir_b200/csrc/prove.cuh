@@ -10,10 +10,12 @@ int ntt_coset_pair_device(b200g16_ctx* ctx, Fr* const* vecs, int batch, int L, c
 int h_pointwise_plain_device(b200g16_ctx* ctx, Fr* a, const Fr* b, const Fr* c, int L);
 int compute_h_dist_phase(b200g16_ctx* ctx, Fr* const (*peers)[8], int g, int me, int L, int phase);
 // instantiated in msm_g1.cu / msm_g2.cu
-extern template int msm_enqueue<Fp>(b200g16_ctx*, const Affine<Fp>*, const MsmTable*, const Fr*, size_t, int, MsmCfg*, bool, bool);
-extern template int msm_collect<Fp>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp>*);
-extern template int msm_enqueue<Fp2>(b200g16_ctx*, const Affine<Fp2>*, const MsmTable*, const Fr*, size_t, int, MsmCfg*, bool, bool);
-extern template int msm_collect<Fp2>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp2>*);
+extern template int msm_enqueue<Fp>(b200g16_ctx*, const Affine<Fp>*, const MsmTable*, const Fr*, size_t, size_t, size_t, int, MsmCfg*,
+                                   bool, bool);
+extern template int msm_collect<Fp>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp>*, size_t);
+extern template int msm_enqueue<Fp2>(b200g16_ctx*, const Affine<Fp2>*, const MsmTable*, const Fr*, size_t, size_t, size_t, int, MsmCfg*,
+                                   bool, bool);
+extern template int msm_collect<Fp2>(b200g16_ctx*, int, const MsmCfg&, Affine<Fp2>*, size_t);
 }  // namespace b200
 
 struct b200g16_pk {

@@ -540,6 +540,49 @@ def Prove(ctx, r1cs, pk, witness, r=None, s=None, resolve=None, want_h=False):
     return Proof(out["ar"], out["krs"], out["bs"], proof_commitments, pok, dbg)
 
 
+def BatchProve(ctx, r1cs, pk, witnesses, rs=None, ss=None, resolve=None):
+    """k proofs of one circuit in one b200g16_prove_batch call -> list of k Proofs, proof j equal to
+    Prove(ctx, r1cs, pk, witnesses[j], rs[j], ss[j], resolve).
+
+    With a commitment, the Pedersen Commit of all k witnesses is one batch MSM over the commitment basis; each
+    witness's commitment wire is then filled from its own commitment (and `resolve` finishes that witness), and
+    ProveKnowledge is one batch MSM over BasisExpSigma.  rs, ss: k blinding scalars each; drawn like Prove draws
+    them when omitted."""
+    ws = [list(w) for w in witnesses]
+    k = len(ws)
+    rs = [secrets.randbelow(R_MOD) for _ in range(k)] if rs is None else list(rs)
+    ss = [secrets.randbelow(R_MOD) for _ in range(k)] if ss is None else list(ss)
+    if len(rs) != k or len(ss) != k:
+        raise ValueError("groth16.BatchProve: one r and one s per witness")
+    if k == 0:
+        return []
+    coms, poks = [[] for _ in range(k)], [None] * k
+    if r1cs.commitment_wire >= 0:
+        ck = pk.CommitmentKeys[0]
+        if ck.basis_dev is None:
+            ck.basis_dev = ctx.upload_g1(ck.Basis)
+            ck.basis_exp_sigma_dev = ctx.upload_g1(ck.BasisExpSigma)
+        vals = np.stack([fr_array([w[i] for i in r1cs.private_committed]).reshape(-1, 4) for w in ws])
+        com = ctx.msm_batch(ck.basis_dev, vals)                     # pedersen Commit of every witness
+        for j, w in enumerate(ws):
+            w[r1cs.commitment_wire] = commitment_challenge(com[j], [w[i] for i in r1cs.public_committed])
+            if resolve is not None:
+                resolve(w)
+        pok = ctx.msm_batch(ck.basis_exp_sigma_dev, vals)           # pedersen ProveKnowledge of every witness
+        coms = [[com[j]] for j in range(k)]
+        poks = [pok[j] for j in range(k)]
+    abc = [solve_abc(r1cs, w) for w in ws]
+    outs = ctx.prove_batch(pk.device_handle(ctx), np.stack([fr_array(w).reshape(-1, 4) for w in ws]),
+                           *[np.stack([fr_array(t[i]).reshape(-1, 4) for t in abc]) for i in range(3)],
+                           fr_array(rs).reshape(k, 4), fr_array(ss).reshape(k, 4))
+    proofs = []
+    for j, out in enumerate(outs):
+        dbg = dict(out)
+        dbg["witness"] = ws[j]
+        proofs.append(Proof(out["ar"], out["krs"], out["bs"], coms[j], poks[j], dbg))
+    return proofs
+
+
 def _verify_inputs(proof, vk, public_witness):
     """The public inputs b200g16_verify takes for one proof (the public witness, then the BSB22 challenge when the
     circuit has a commitment) and the proof's commitment and proof of knowledge (None without one)."""

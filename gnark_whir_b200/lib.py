@@ -59,6 +59,10 @@ SIGNATURES = {
     "b200g16_msm_g1_begin_dev": (C.c_int, [_vp, _vp, _sz, _vp, _sz, C.POINTER(C.c_int)]),
     "b200g16_msm_g1_end": (C.c_int, [_vp, C.c_int, _vp]),
     "b200g16_msm_g2_dev": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _vp]),
+    "b200g16_msm_g1_batch": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _sz, _vp]),
+    "b200g16_msm_g2_batch": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _sz, _vp]),
+    "b200g16_msm_g1_batch_dev": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _sz, _vp]),
+    "b200g16_msm_g2_batch_dev": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _sz, _vp]),
     "b200g16_ntt": (C.c_int, [_vp, _vp, C.c_uint, C.c_int, C.c_int, C.c_int]),
     "b200g16_ntt_dev": (C.c_int, [_vp, _vp, C.c_uint, C.c_uint, C.c_int, C.c_int, C.c_int]),
     "b200g16_compute_h": (C.c_int, [_vp, _vp, _vp, _vp, _sz, C.c_uint, _vp]),
@@ -74,6 +78,8 @@ SIGNATURES = {
     "b200g16_pk_free": (None, [_vp]),
     "b200g16_prove": (C.c_int, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp]),
     "b200g16_prove_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200g16_prove_batch": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
+    "b200g16_prove_batch_dev": (C.c_int, [_vp, _vp, _sz, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "b200g16_prove_h_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "b200g16_h_pointwise_dev": (C.c_int, [_vp, _vp, _vp, _vp, C.c_uint]),
     "b200g16_prove_begin_dev": (C.c_int, [_vp, _vp, _vp]),
@@ -631,6 +637,30 @@ class Context:
                                         _ptr(r), _ptr(s), C.byref(out)))
         return out.as_dict()
 
+    def prove_batch(self, pk, wires, a, b, c, r, s):
+        """b200g16_prove_batch: k proves of one circuit.  wires (k, n_wires, 4), a/b/c (k, n_constraints, 4), r/s (k, 4),
+        all Montgomery -> list of k dicts as prove() returns them."""
+        wires, a, b, c = [np.ascontiguousarray(x, dtype=np.uint64) for x in (wires, a, b, c)]
+        k = wires.shape[0]
+        if wires.ndim != 3 or any(x.ndim != 3 or x.shape[0] != k for x in (a, b, c)) or not a.shape == b.shape == c.shape:
+            raise B200Error("prove_batch: wires must be (k, n_wires, 4), a/b/c (k, n_constraints, 4)")
+        r, s = _u64(r, 4), _u64(s, 4)
+        if r.shape[0] != k or s.shape[0] != k:
+            raise B200Error("prove_batch: one r and one s per proof")
+        out = (ProofOut * max(k, 1))()
+        _check(load().b200g16_prove_batch(self.h, pk, k, _ptr(wires), wires.shape[1], _ptr(a), _ptr(b), _ptr(c),
+                                          a.shape[1], _ptr(r), _ptr(s), out))
+        return [out[j].as_dict() for j in range(k)]
+
+    def prove_batch_dev(self, pk, k, d_wires, d_a, d_b, d_c, r, s):
+        """b200g16_prove_batch_dev: device pointers to k x n_wires wires and k x N a/b/c rows (zero padded, clobbered;
+        h is left in the d_a rows); r/s (k, 4) host -> list of k dicts."""
+        r, s = _u64(r, 4), _u64(s, 4)
+        out = (ProofOut * max(k, 1))()
+        _check(load().b200g16_prove_batch_dev(self.h, pk, k, _dp(d_wires), _dp(d_a), _dp(d_b), _dp(d_c),
+                                              _ptr(r), _ptr(s), out))
+        return [out[j].as_dict() for j in range(k)]
+
     # -- pairing / verify (mirror bn254.PairingCheck, bn254.Pair, groth16.Verify)
     def pairing_check(self, g1_points, g2_points):
         p, q = _u64(g1_points, 8), _u64(g2_points, 16)
@@ -780,6 +810,26 @@ class Context:
         else:  # raw device pointer (e.g. torch tensor .data_ptr())
             fn = lib.b200g16_msm_g1_dev if bases.group == 1 else lib.b200g16_msm_g2_dev
             _check(fn(self.h, bases.handle, offset, _dp(scalars), n, _ptr(out)))
+        return out
+
+    def msm_batch(self, bases, scalars, offset=0, n=None, k=None):
+        """k MSMs over the same bases (b200g16_msm_g1_batch / _g2_batch): scalars (k, n, 4) uint64 Montgomery, or a device
+        pointer to k x n scalars with n and k given.  -> (k, 8) or (k, 16) affine points, row j = msm(bases, scalars[j])"""
+        lib = load()
+        if isinstance(scalars, np.ndarray):
+            sc = np.ascontiguousarray(scalars, dtype=np.uint64)
+            if sc.ndim != 3 or sc.shape[2] != 4:
+                raise B200Error("msm_batch: scalars must be (k, n, 4)")
+            k, n = sc.shape[0], sc.shape[1]
+            fn = lib.b200g16_msm_g1_batch if bases.group == 1 else lib.b200g16_msm_g2_batch
+            ptr = _ptr(sc)
+        else:
+            if n is None or k is None:
+                raise B200Error("msm_batch: a device pointer needs n and k")
+            fn = lib.b200g16_msm_g1_batch_dev if bases.group == 1 else lib.b200g16_msm_g2_batch_dev
+            ptr = _dp(scalars)
+        out = np.zeros((k, 8 if bases.group == 1 else 16), dtype=np.uint64)
+        _check(fn(self.h, bases.handle, offset, ptr, n, k, _ptr(out) if k else None))
         return out
 
     def msm_begin(self, bases, scalars, offset=0, n=None):

@@ -211,6 +211,26 @@ int b200g16_msm_g1_dev(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offs
                        const void* d_scalars, size_t n, uint64_t out_affine[8]);
 int b200g16_msm_g2_dev(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset,
                        const void* d_scalars, size_t n, uint64_t out_affine[16]);
+/* k MultiExps over ONE resident bases vector: out[j] = sum_i scalars[j*n + i] * bases[offset + i], j < k.
+ * scalars: k x n fr.Elements (Montgomery), row j contiguous; out: k affine points (k x 8 words for G1, k x 16 for
+ * G2).  Each out[j] equals the b200g16_msm_g1 / _g2 result on row j.  The k rows run through one pass of every MSM
+ * kernel (vector j has its own bucket sets), so the sort, accumulate and bucket-reduction launches are paid once per
+ * batch instead of once per vector.  One pass holds at most 2^23 buckets (k x buckets per vector) and fewer than 2^32
+ * digit entries (k x n x windows); a larger k is split into sub-batches of that many vectors, run back to back in
+ * one call.  k = 1, and a shape where a sub-batch would hold one vector, run the single-MSM path.
+ * B200G16_ERR_ARG: NULL buffers with k > 0, k x n overflowing size_t, n >= 2^31, and the checks of b200g16_msm_g1.
+ * B200G16_ERR_STATE between b200g16_prove_begin_dev and _end_dev.  k = 0 returns 0 and writes nothing.
+ * b200g16_last_timings (k > 1): one value, the device time of the whole call.  Open b200g16_msm_g1_begin tickets
+ * are unaffected. */
+int b200g16_msm_g1_batch(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const uint64_t* scalars,
+                         size_t n, size_t k, uint64_t* out);
+int b200g16_msm_g2_batch(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const uint64_t* scalars,
+                         size_t n, size_t k, uint64_t* out);
+/* Same with the k x n scalars in DEVICE memory. */
+int b200g16_msm_g1_batch_dev(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const void* d_scalars,
+                             size_t n, size_t k, uint64_t* out);
+int b200g16_msm_g2_batch_dev(b200g16_ctx* ctx, const b200g16_bases* bases, size_t offset, const void* d_scalars,
+                             size_t n, size_t k, uint64_t* out);
 
 /* Asynchronous G1 MSM: _begin enqueues it and returns a ticket (0..2; three can be open per ctx), _end waits for that
  * MSM alone and returns its result.  Calls made in between on the same ctx (b200g16_prove*, b200g16_msm_*, NTTs) run
@@ -346,6 +366,26 @@ int b200g16_prove_finish(const b200g16_pk* pk, const uint64_t msm_a[8], const ui
  * clobbered; h is left in d_a). */
 int b200g16_prove_dev(b200g16_ctx* ctx, const b200g16_pk* pk, const void* d_wires, void* d_a, void* d_b,
                       void* d_c, const uint64_t r[4], const uint64_t s[4], b200g16_proof* proof_out);
+/* k proves of one circuit against one resident pk: proof j from wires[j] (k x n_wires), a/b/c[j] (k x n_constraints
+ * each), r[j], s[j] (k x 4 each), into proofs_out[j]; every field is bit-identical to b200g16_prove on those inputs.
+ * The proofs run in sub-batches: the five MSMs of a sub-batch are batch MSMs (see b200g16_msm_g1_batch; a
+ * sub-batch holds as many proofs as the most constrained of the five allows), computeH runs once per proof, and
+ * one synchronisation per sub-batch is followed by the host assembly on up to 16 threads.  Sub-batches of one
+ * proof (k = 1, or a key whose MSMs allow no more) run b200g16_prove proof by proof.
+ * B200G16_ERR_ARG: NULL buffers with k > 0, n_wires != the pk's, n_constraints > N, k x n_wires or k x N
+ * overflowing, a partial (sharded) pk.  B200G16_ERR_STATE: pk on another device, between
+ * b200g16_prove_begin_dev and _end_dev, or host threads that could not be started.  Any error leaves the ctx
+ * usable.  k = 0 returns 0 and writes nothing.
+ * b200g16_last_timings (sub-batches of more than one proof): 4 device phases summed over the sub-batches:
+ * uploads of the witness rows + gathers, the four witness MSMs, computeH (with the wait for a, b, c), and the Z MSM
+ * with the remaining bucket reductions. */
+int b200g16_prove_batch(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const uint64_t* wires, size_t n_wires,
+                        const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints,
+                        const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out);
+/* Same with wires (k x n_wires) and a, b, c (k x N each, zero padded, clobbered; h is left in the d_a rows) in DEVICE
+ * memory. */
+int b200g16_prove_batch_dev(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const void* d_wires, void* d_a,
+                            void* d_b, void* d_c, const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out);
 
 /* ---- pairing / Groth16 verify ----------------------------------------------------------- */
 /* groth16_bn254.VerifyingKey as Verify needs it (gnark backend/groth16/bn254/verify.go). */

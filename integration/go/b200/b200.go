@@ -160,6 +160,48 @@ func msmG1(ctx *C.b200g16_ctx, bases *C.b200g16_bases, scalars []fr.Element) (cu
 	return out, err
 }
 
+// solve runs gnark's solver with the BSB22 hint overridden: identical to gnark's, except Commit() is the GPU MSM on the
+// resident basis.  commitments receives one point per commitment; the committed private values are returned for the
+// proofs of knowledge.
+func solve(r1cs *cs.R1CS, pk *ProvingKey, opt backend.ProverConfig, fullWitness witness.Witness,
+	commitments []curve.G1Affine) (*cs.R1CSSolution, [][]fr.Element, error) {
+	commitmentInfo := r1cs.CommitmentInfo.(constraint.Groth16Commitments)
+	privateCommittedValues := make([][]fr.Element, len(commitmentInfo))
+	solverOpts := opt.SolverOpts[:len(opt.SolverOpts):len(opt.SolverOpts)]
+	bsb22ID := solver.GetHintID(fcs.Bsb22CommitmentComputePlaceholder)
+	solverOpts = append(solverOpts, solver.OverrideHint(bsb22ID, func(_ *big.Int, in []*big.Int, out []*big.Int) error {
+		i := int(in[0].Int64())
+		in = in[1:]
+		privateCommittedValues[i] = make([]fr.Element, len(commitmentInfo[i].PrivateCommitted))
+		hashed := in[:len(commitmentInfo[i].PublicAndCommitmentCommitted)]
+		committed := in[len(hashed):]
+		for j, inJ := range committed {
+			privateCommittedValues[i][j].SetBigInt(inJ)
+		}
+		var err error
+		if commitments[i], err = msmG1(pk.ctx, pk.pedBasis[i], privateCommittedValues[i]); err != nil {
+			return err
+		}
+		opt.HashToFieldFn.Write(constraint.SerializeCommitment(commitments[i].Marshal(), hashed, (fr.Bits-1)/8+1))
+		hashBts := opt.HashToFieldFn.Sum(nil)
+		opt.HashToFieldFn.Reset()
+		nbBuf := fr.Bytes
+		if opt.HashToFieldFn.Size() < fr.Bytes {
+			nbBuf = opt.HashToFieldFn.Size()
+		}
+		var res fr.Element
+		res.SetBytes(hashBts[:nbBuf])
+		res.BigInt(out[0])
+		return nil
+	}))
+
+	_solution, err := r1cs.Solve(fullWitness, solverOpts...) // Go, CPU (out of scope)
+	if err != nil {
+		return nil, nil, err
+	}
+	return _solution.(*cs.R1CSSolution), privateCommittedValues, nil
+}
+
 // Prove has gnark's signature: groth16.Prove(ccs, pk, fullWitness, opts...) at mt.go:496.  The body follows gnark
 // v0.11.0 backend/groth16/bn254/prove.go; what changes is where the arithmetic runs.
 func Prove(r1cs *cs.R1CS, pk *ProvingKey, fullWitness witness.Witness, opts ...backend.ProverOption) (*groth16_bn254.Proof, error) {
@@ -176,42 +218,10 @@ func Prove(r1cs *cs.R1CS, pk *ProvingKey, fullWitness witness.Witness, opts ...b
 
 	commitmentInfo := r1cs.CommitmentInfo.(constraint.Groth16Commitments)
 	proof := &groth16_bn254.Proof{Commitments: make([]curve.G1Affine, len(commitmentInfo))}
-	privateCommittedValues := make([][]fr.Element, len(commitmentInfo))
-
-	// BSB22 hint override: identical to gnark's, except Commit() is the GPU MSM on the resident basis
-	solverOpts := opt.SolverOpts[:len(opt.SolverOpts):len(opt.SolverOpts)]
-	bsb22ID := solver.GetHintID(fcs.Bsb22CommitmentComputePlaceholder)
-	solverOpts = append(solverOpts, solver.OverrideHint(bsb22ID, func(_ *big.Int, in []*big.Int, out []*big.Int) error {
-		i := int(in[0].Int64())
-		in = in[1:]
-		privateCommittedValues[i] = make([]fr.Element, len(commitmentInfo[i].PrivateCommitted))
-		hashed := in[:len(commitmentInfo[i].PublicAndCommitmentCommitted)]
-		committed := in[len(hashed):]
-		for j, inJ := range committed {
-			privateCommittedValues[i][j].SetBigInt(inJ)
-		}
-		var err error
-		if proof.Commitments[i], err = msmG1(pk.ctx, pk.pedBasis[i], privateCommittedValues[i]); err != nil {
-			return err
-		}
-		opt.HashToFieldFn.Write(constraint.SerializeCommitment(proof.Commitments[i].Marshal(), hashed, (fr.Bits-1)/8+1))
-		hashBts := opt.HashToFieldFn.Sum(nil)
-		opt.HashToFieldFn.Reset()
-		nbBuf := fr.Bytes
-		if opt.HashToFieldFn.Size() < fr.Bytes {
-			nbBuf = opt.HashToFieldFn.Size()
-		}
-		var res fr.Element
-		res.SetBytes(hashBts[:nbBuf])
-		res.BigInt(out[0])
-		return nil
-	}))
-
-	_solution, err := r1cs.Solve(fullWitness, solverOpts...) // Go, CPU (out of scope)
+	solution, privateCommittedValues, err := solve(r1cs, pk, opt, fullWitness, proof.Commitments)
 	if err != nil {
 		return nil, err
 	}
-	solution := _solution.(*cs.R1CSSolution)
 	wireValues := []fr.Element(solution.W)
 
 	// Pedersen proofs of knowledge (gnark: ProveKnowledge per key): one MSM per commitment on BasisExpSigma,
@@ -290,6 +300,106 @@ func Prove(r1cs *cs.R1CS, pk *ProvingKey, fullWitness witness.Witness, opts ...b
 	proof.Bs = *(*curve.G2Affine)(unsafe.Pointer(&out.bs))
 	proof.Krs = *(*curve.G1Affine)(unsafe.Pointer(&out.krs))
 	return proof, nil
+}
+
+// BatchProve proves k witnesses of one circuit: proof j equals Prove(r1cs, pk, witnesses[j], opts...) with the same
+// r, s.  Each witness is solved as Prove solves it (the BSB22 commitment stays one GPU MSM inside each solve, since the
+// hint's answer feeds the rest of that solve); the proofs of knowledge of all k witnesses are one
+// b200g16_msm_g1_batch per commitment key, and the k proves one b200g16_prove_batch call.
+func BatchProve(r1cs *cs.R1CS, pk *ProvingKey, witnesses []witness.Witness, opts ...backend.ProverOption) ([]*groth16_bn254.Proof, error) {
+	opt, err := backend.NewProverConfig(opts...)
+	if err != nil {
+		return nil, fmt.Errorf("new prover config: %w", err)
+	}
+	if opt.HashToFieldFn == nil {
+		opt.HashToFieldFn = hash_to_field.New([]byte(constraint.CommitmentDst))
+	}
+	if err := pk.setup(r1cs); err != nil {
+		return nil, err
+	}
+	k := len(witnesses)
+	if k == 0 {
+		return nil, nil
+	}
+	commitmentInfo := r1cs.CommitmentInfo.(constraint.Groth16Commitments)
+	proofs := make([]*groth16_bn254.Proof, k)
+	committed := make([][][]fr.Element, k)
+	var wires, A, B, Cv []fr.Element
+	for j, w := range witnesses {
+		proofs[j] = &groth16_bn254.Proof{Commitments: make([]curve.G1Affine, len(commitmentInfo))}
+		solution, pcv, err := solve(r1cs, pk, opt, w, proofs[j].Commitments)
+		if err != nil {
+			return nil, err
+		}
+		committed[j] = pcv
+		wires = append(wires, solution.W...)
+		A = append(A, solution.A...)
+		B = append(B, solution.B...)
+		Cv = append(Cv, solution.C...)
+	}
+	nWires, nCons := len(wires)/k, len(A)/k
+
+	// proofs of knowledge: for each commitment key, the k witnesses' committed values as one batch MSM
+	poks := make([][]curve.G1Affine, k)
+	for j := range poks {
+		poks[j] = make([]curve.G1Affine, len(pk.CommitmentKeys))
+	}
+	for i := range pk.CommitmentKeys {
+		n := len(committed[0][i])
+		if n == 0 {
+			continue
+		}
+		rows := make([]fr.Element, 0, k*n)
+		for j := 0; j < k; j++ {
+			rows = append(rows, committed[j][i]...)
+		}
+		out := make([]curve.G1Affine, k)
+		if err := call(func() C.int {
+			return C.b200g16_msm_g1_batch(pk.ctx, pk.pedSigma[i], 0, u64(unsafe.Pointer(&rows[0])), C.size_t(n), C.size_t(k),
+				u64(unsafe.Pointer(&out[0])))
+		}); err != nil {
+			return nil, err
+		}
+		for j := 0; j < k; j++ {
+			poks[j][i] = out[j]
+		}
+	}
+
+	rs, ss := make([]fr.Element, k), make([]fr.Element, k)
+	for j := 0; j < k; j++ {
+		if _, err := rs[j].SetRandom(); err != nil {
+			return nil, err
+		}
+		if _, err := ss[j].SetRandom(); err != nil {
+			return nil, err
+		}
+	}
+	out := make([]C.b200g16_proof, k)
+	err = call(func() C.int {
+		return C.b200g16_prove_batch(pk.ctx, pk.dev, C.size_t(k), u64(unsafe.Pointer(&wires[0])), C.size_t(nWires),
+			u64(unsafe.Pointer(&A[0])), u64(unsafe.Pointer(&B[0])), u64(unsafe.Pointer(&Cv[0])), C.size_t(nCons),
+			u64(unsafe.Pointer(&rs[0])), u64(unsafe.Pointer(&ss[0])), &out[0])
+	})
+	if err != nil {
+		return nil, err
+	}
+	for j := 0; j < k; j++ {
+		commitmentsSerialized := make([]byte, fr.Bytes*len(commitmentInfo))
+		for i := range commitmentInfo {
+			copy(commitmentsSerialized[fr.Bytes*i:], wires[j*nWires+commitmentInfo[i].CommitmentIndex].Marshal())
+		}
+		challenge, err := fr.Hash(commitmentsSerialized, []byte("G16-BSB22"), 1)
+		if err != nil {
+			return nil, err
+		}
+		if _, err = proofs[j].CommitmentPok.Fold(poks[j], challenge[0], ecc.MultiExpConfig{NbTasks: 1}); err != nil {
+			return nil, err
+		}
+		proofs[j].Ar = *(*curve.G1Affine)(unsafe.Pointer(&out[j].ar))
+		proofs[j].Bs = *(*curve.G2Affine)(unsafe.Pointer(&out[j].bs))
+		proofs[j].Krs = *(*curve.G1Affine)(unsafe.Pointer(&out[j].krs))
+	}
+	return proofs, nil
 }
 
 // Pin registers the witness-sized Go slices once (cudaHostRegister): H2D copies from unregistered (pageable) Go
