@@ -200,10 +200,8 @@ static int msm_batch_entry(b200g16_ctx* ctx, const b200g16_bases* bases, int gro
     }
     return 0;
   };
-  if (int status = run()) {   // leave the ctx usable: whatever is in flight is drained and forgotten
-    msm_join(ctx);
-    cudaStreamSynchronize(st);
-    cudaStreamSynchronize(ctx->tail_stream);
+  if (int status = run()) {
+    msm_drain(ctx);
     return status;
   }
   B200_CUDA(cudaEventRecord(ctx->ev[1], st));

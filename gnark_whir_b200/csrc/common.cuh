@@ -190,6 +190,19 @@ struct b200g16_ctx {
   bool sort_smem_set = false;   // k_sort_coarse_part's dynamic shared-memory limit raised on this device
 };
 
+namespace b200 {
+// ctx->timings from the events ctx->ev[0 .. ev) a call recorded, all complete: interval i = ev[i] -> ev[i + 1].
+// add: sum onto the intervals already there (the sub-batches of one call).
+inline void events_to_timings(b200g16_ctx* ctx, int ev, bool add = false) {
+  for (int i = 0; i + 1 < ev; i++) {
+    float t = 0;
+    cudaEventElapsedTime(&t, ctx->ev[i], ctx->ev[i + 1]);
+    ctx->timings.ms[i] = add ? ctx->timings.ms[i] + t : t;
+  }
+  ctx->timings.n = ev - 1;
+}
+}  // namespace b200
+
 struct b200g16_bases {
   int group = 1;  // 1 = G1, 2 = G2
   size_t n = 0;

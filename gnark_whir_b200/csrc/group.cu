@@ -377,12 +377,11 @@ static int group_prove_dist(b200g16_group* g, const b200g16_group_pk* gpk, const
     if (!st) st = [&]() -> int {
       B200_CUDA(cudaStreamWaitEvent(stm, ctx->ev_copy[1], 0));
       cudaEventRecord(ctx->ev[ev++], stm);
-      B200_TRY(prove_front(ctx, pk, ctx->io_a.as<Fr>(), &ev));
+      B200_TRY(prove_front(ctx, pk, ctx->io_a.as<Fr>(), n_wires, 1, &ev));
       if (ev < 18) cudaEventRecord(ctx->ev[ev++], stm);
       const Fr* d_h = reinterpret_cast<const Fr*>(ctx->dist_h.slice[0].p) - pk->off_z;  // prove_back reads d_h[off_z, off_z + n_z)
-      B200_TRY(prove_back(ctx, pk, d_h, fr_r, fr_s, &parts[i], &ev));
-      ctx->timings.n = ev - 1;
-      for (int k = 0; k + 1 < ev; k++) cudaEventElapsedTime(&ctx->timings.ms[k], ctx->ev[k], ctx->ev[k + 1]);
+      B200_TRY(prove_back(ctx, pk, d_h, (size_t)1 << L, 1, &fr_r, &fr_s, &parts[i], &ev));
+      events_to_timings(ctx, ev);
       return 0;
     }();
     if (st) ctx->prove_active = false;
@@ -470,7 +469,7 @@ int b200g16_group_prove(b200g16_group* g, const b200g16_group_pk* gpk, const uin
       }
       B200_CUDA(cudaStreamWaitEvent(stm, ctx->ev_copy[1], 0));
       cudaEventRecord(ctx->ev[ev++], stm);
-      B200_TRY(prove_front(ctx, pk, ctx->io_a.as<Fr>(), &ev));
+      B200_TRY(prove_front(ctx, pk, ctx->io_a.as<Fr>(), n_wires, 1, &ev));
       if (i != root) {
         B200_TRY(ctx->io_c.ensure((pk->n_z ? pk->n_z : 1) * sizeof(Fr)));
         if (int ws = h_ready.wait()) { ctx->prove_active = false; return fail(ws, "group_prove: the root device failed"); }
@@ -481,9 +480,8 @@ int b200g16_group_prove(b200g16_group* g, const b200g16_group_pk* gpk, const uin
         d_h = ctx->io_c.as<Fr>() - pk->off_z;  // prove_back reads d_h[off_z, off_z + n_z)
       }
       if (ev < 18) cudaEventRecord(ctx->ev[ev++], stm);
-      B200_TRY(prove_back(ctx, pk, d_h, fr_r, fr_s, &parts[i], &ev));
-      ctx->timings.n = ev - 1;
-      for (int k = 0; k + 1 < ev; k++) cudaEventElapsedTime(&ctx->timings.ms[k], ctx->ev[k], ctx->ev[k + 1]);
+      B200_TRY(prove_back(ctx, pk, d_h, N, 1, &fr_r, &fr_s, &parts[i], &ev));
+      events_to_timings(ctx, ev);
       return 0;
     };
     int rc = body();

@@ -545,6 +545,17 @@ inline int msm_join(b200g16_ctx* ctx) {
   return 0;
 }
 
+// After a failed call: wait for everything in flight on the ctx's streams and forget it (no open prove, no sorted lists
+// to share), so that the ctx is usable again.
+inline void msm_drain(b200g16_ctx* ctx) {
+  msm_join(ctx);
+  cudaStreamSynchronize(ctx->stream);
+  cudaStreamSynchronize(ctx->tail_stream);
+  cudaStreamSynchronize(ctx->copy_stream);
+  ctx->prove_active = false;
+  ctx->last_sort.valid = false;
+}
+
 // After the stream has drained: Horner over the window sums of `slot` (vector j of a batch) on the host,
 // acc = sum_w 2^(c w) * S_w, then one inversion to the affine normal form.
 template <class F>
@@ -564,10 +575,7 @@ int msm_collect(b200g16_ctx* ctx, int slot, const MsmCfg& cfg, Affine<F>* out, s
 }
 
 inline void msm_resolve_timings(b200g16_ctx* ctx) {
-  if (ctx->timings.n >= 0) return;
-  int n = -ctx->timings.n;
-  for (int i = 0; i < n; i++) cudaEventElapsedTime(&ctx->timings.ms[i], ctx->ev[i], ctx->ev[i + 1]);
-  ctx->timings.n = n;
+  if (ctx->timings.n < 0) events_to_timings(ctx, 1 - ctx->timings.n);
 }
 
 template <class F>

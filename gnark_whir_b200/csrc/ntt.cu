@@ -574,8 +574,7 @@ int compute_h_device(b200g16_ctx* ctx, Fr* a, Fr* b, Fr* c, int L, bool sync_and
   B200_CUDA(cudaGetLastError());
   if (!sync_and_time) return 0;
   B200_CUDA(cudaStreamSynchronize(ctx->stream));
-  ctx->timings.n = ev - 1;
-  for (int i = 0; i + 1 < ev; i++) cudaEventElapsedTime(&ctx->timings.ms[i], ctx->ev[i], ctx->ev[i + 1]);
+  events_to_timings(ctx, ev);
   return 0;
 }
 

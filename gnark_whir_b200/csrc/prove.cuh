@@ -47,11 +47,13 @@ void prove_finish_host(const b200g16_pk* pk, const DeltaMultiples& dm, const G1A
                        b200g16_proof* out);
 int pk_build(b200g16_ctx* ctx, const b200g16_pk_desc* d, b200g16_pk** out);
 void pk_release(b200g16_pk* pk);
-// gathers + the four witness MSMs enqueued on ctx->stream (no synchronisation); ev_io: next free ctx->ev slot
-int prove_front(b200g16_ctx* ctx, const b200g16_pk* pk, const Fr* d_wires, int* ev_io);
-// Z MSM over d_h[off_z, off_z + n_z), join, host assembly (or the five partial sums for a partial pk)
-int prove_back(b200g16_ctx* ctx, const b200g16_pk* pk, const Fr* d_h, const Fr& r, const Fr& s, b200g16_proof* out,
-               int* ev_io);
+// m proofs (a single prove: m = 1).  Gathers from the m witness rows d_wires[j * wire_stride ..) + the four witness MSMs
+// enqueued on ctx->stream (no synchronisation); ev_io: next free ctx->ev slot
+int prove_front(b200g16_ctx* ctx, const b200g16_pk* pk, const Fr* d_wires, size_t wire_stride, size_t m, int* ev_io);
+// Z MSM over the m rows d_h[j * h_stride + off_z, + n_z), join, host assembly of out[0 .. m) with r[j], s[j] (or the
+// five partial sums for a partial pk, m = 1)
+int prove_back(b200g16_ctx* ctx, const b200g16_pk* pk, const Fr* d_h, size_t h_stride, size_t m, const Fr* r,
+               const Fr* s, b200g16_proof* out, int* ev_io);
 template <class F>
 Affine<F> host_sum_points(const Affine<F>* pts, int n);
 }  // namespace b200

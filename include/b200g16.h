@@ -370,15 +370,14 @@ int b200g16_prove_dev(b200g16_ctx* ctx, const b200g16_pk* pk, const void* d_wire
  * each), r[j], s[j] (k x 4 each), into proofs_out[j]; every field is bit-identical to b200g16_prove on those inputs.
  * The proofs run in sub-batches: the five MSMs of a sub-batch are batch MSMs (see b200g16_msm_g1_batch; a
  * sub-batch holds as many proofs as the most constrained of the five allows), computeH runs once per proof, and
- * one synchronisation per sub-batch is followed by the host assembly on up to 16 threads.  Sub-batches of one
- * proof (k = 1, or a key whose MSMs allow no more) run b200g16_prove proof by proof.
+ * the host assembly runs on up to 16 threads, each step as soon as the MSM results it needs have landed.  A
+ * sub-batch of one proof runs exactly as b200g16_prove.
  * B200G16_ERR_ARG: NULL buffers with k > 0, n_wires != the pk's, n_constraints > N, k x n_wires or k x N
  * overflowing, a partial (sharded) pk.  B200G16_ERR_STATE: pk on another device, between
  * b200g16_prove_begin_dev and _end_dev, or host threads that could not be started.  Any error leaves the ctx
  * usable.  k = 0 returns 0 and writes nothing.
- * b200g16_last_timings (sub-batches of more than one proof): 4 device phases summed over the sub-batches:
- * uploads of the witness rows + gathers, the four witness MSMs, computeH (with the wait for a, b, c), and the Z MSM
- * with the remaining bucket reductions. */
+ * b200g16_last_timings: the 8 device phases of b200g16_prove, summed over the sub-batches: upload of the witness
+ * rows, gathers, MSM B2, B1, A, K, computeH (with the wait for a, b, c), and the Z MSM. */
 int b200g16_prove_batch(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const uint64_t* wires, size_t n_wires,
                         const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints,
                         const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out);

@@ -43,6 +43,7 @@ def test_host_path_closed_form_and_single_prove(ctx, keys, log2n, k):
     wires, a, b, c, r, s = inputs(key, k, ncons)
     got = ctx.prove_batch(key.handle, wires, a, b, c, r, s)
     assert len(got) == k
+    assert len(ctx.last_timings()) == 8          # a single prove's phases, summed over the sub-batches
     for j in range(k):
         exp, _ = key.expected(wires[j], a[j], b[j], c[j], r[j], s[j])
         assert check_proof(got[j], exp) == [], f"proof {j}"
