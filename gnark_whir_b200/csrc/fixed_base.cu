@@ -46,22 +46,47 @@ __global__ void __launch_bounds__(128) k_fb_mul(const Affine<F>* __restrict__ ta
   out[i] = acc.to_affine();
 }
 
+// Enqueue the window table of `base` (fixed_base_table_points() points) on ctx->stream.
+template <class F>
+int fixed_base_table_device(b200g16_ctx* ctx, const Affine<F>& base, Affine<F>* d_table) {
+  k_fb_table<F><<<FB_W, 256, 0, ctx->stream>>>(base, d_table);
+  ctx->launches++;
+  B200_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// Enqueue out[i] = scalars[i] * base over a table built by fixed_base_table_device (no synchronisation).
+template <class F>
+int fixed_base_mul_table_device(b200g16_ctx* ctx, const Affine<F>* d_table, const Fr* d_scalars, size_t n,
+                                Affine<F>* d_out) {
+  if (n == 0) return 0;
+  if (n >= (1ull << 32)) return fail(B200G16_ERR_ARG, "fixed_base: n too large");
+  k_fb_mul<F><<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(d_table, d_scalars, (uint32_t)n, d_out);
+  ctx->launches++;
+  B200_CUDA(cudaGetLastError());
+  return 0;
+}
+
+size_t fixed_base_table_points() { return (size_t)FB_W * FB_ROW; }
+
 template <class F>
 int fixed_base_mul_device(b200g16_ctx* ctx, const Affine<F>& base, const Fr* d_scalars, size_t n, Affine<F>* d_out) {
   if (n == 0) return 0;
   if (n >= (1ull << 32)) return fail(B200G16_ERR_ARG, "fixed_base: n too large");
-  B200_TRY(ctx->io_c.ensure((size_t)FB_W * FB_ROW * sizeof(Affine<F>)));
+  B200_TRY(ctx->io_c.ensure(fixed_base_table_points() * sizeof(Affine<F>)));
   Affine<F>* table = ctx->io_c.as<Affine<F>>();
-  k_fb_table<F><<<FB_W, 256, 0, ctx->stream>>>(base, table);
-  k_fb_mul<F><<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(table, d_scalars, (uint32_t)n, d_out);
-  ctx->launches += 2;
-  B200_CUDA(cudaGetLastError());
+  B200_TRY(fixed_base_table_device<F>(ctx, base, table));
+  B200_TRY(fixed_base_mul_table_device<F>(ctx, table, d_scalars, n, d_out));
   B200_CUDA(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
 
 template int fixed_base_mul_device<Fp>(b200g16_ctx*, const Affine<Fp>&, const Fr*, size_t, Affine<Fp>*);
 template int fixed_base_mul_device<Fp2>(b200g16_ctx*, const Affine<Fp2>&, const Fr*, size_t, Affine<Fp2>*);
+template int fixed_base_table_device<Fp>(b200g16_ctx*, const Affine<Fp>&, Affine<Fp>*);
+template int fixed_base_table_device<Fp2>(b200g16_ctx*, const Affine<Fp2>&, Affine<Fp2>*);
+template int fixed_base_mul_table_device<Fp>(b200g16_ctx*, const Affine<Fp>*, const Fr*, size_t, Affine<Fp>*);
+template int fixed_base_mul_table_device<Fp2>(b200g16_ctx*, const Affine<Fp2>*, const Fr*, size_t, Affine<Fp2>*);
 
 // ---- integer-pipe probe: `chains` independent dependent-multiply chains per thread ----------
 template <int CHAINS>

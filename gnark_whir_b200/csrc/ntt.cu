@@ -332,7 +332,7 @@ static Fr fr_from_u64(uint64_t v) {
 static Fr coset_denominator_inv(size_t n);
 
 // Build t[0..count) = first * ratio^i on the device.
-static int build_geometric(b200g16_ctx* ctx, Fr* d_t, size_t count, const Fr& first, Fr ratio) {
+int build_geometric(b200g16_ctx* ctx, Fr* d_t, size_t count, const Fr& first, Fr ratio) {
   B200_CUDA(cudaMemcpyAsync(d_t, &first, sizeof(Fr), cudaMemcpyHostToDevice, ctx->stream));
   B200_CUDA(cudaStreamSynchronize(ctx->stream));  // `first` is a host temporary
   Fr step = ratio;                                // ratio^s

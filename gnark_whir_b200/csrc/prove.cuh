@@ -9,6 +9,16 @@ int h_pointwise_device(b200g16_ctx* ctx, Fr* a, const Fr* b, const Fr* c, int L)
 int ntt_coset_pair_device(b200g16_ctx* ctx, Fr* const* vecs, int batch, int L, const bool* with_den);
 int h_pointwise_plain_device(b200g16_ctx* ctx, Fr* a, const Fr* b, const Fr* c, int L);
 int compute_h_dist_phase(b200g16_ctx* ctx, Fr* const (*peers)[8], int g, int me, int L, int phase);
+// t[0 .. count) = first * ratio^i on the device (ntt.cu)
+int build_geometric(b200g16_ctx* ctx, Fr* d_t, size_t count, const Fr& first, Fr ratio);
+// fixed-base multiples (fixed_base.cu): one window table per base, then any number of vectors over it, enqueued on
+// ctx->stream without synchronisation
+size_t fixed_base_table_points();
+template <class F>
+int fixed_base_table_device(b200g16_ctx* ctx, const Affine<F>& base, Affine<F>* d_table);
+template <class F>
+int fixed_base_mul_table_device(b200g16_ctx* ctx, const Affine<F>* d_table, const Fr* d_scalars, size_t n,
+                                Affine<F>* d_out);
 // instantiated in msm_g1.cu / msm_g2.cu
 extern template int msm_enqueue<Fp>(b200g16_ctx*, const Affine<Fp>*, const MsmTable*, const Fr*, size_t, size_t, size_t, int, MsmCfg*,
                                    bool, bool);

@@ -7,6 +7,7 @@ restated.  What runs where:
 
   Setup   host: toxic waste, per-wire A_i(tau), B_i(tau), C_i(tau), K_i, Z_i scalars (python ints)
           GPU : every group element, through b200g16_fixed_base_mul_g1/g2
+  DeviceSetup  the same key, all of it on the GPU (b200g16_setup), point vectors left resident
   Prove   host: the constraint "solver" (here: L.w, R.w, O.w from a full assignment), the BSB22
                 challenge hash, sampling r, s
           GPU : Pedersen commit + PoK (b200g16_msm_g1), computeH, the five MSMs, via b200g16_prove
@@ -22,6 +23,7 @@ every group operation below goes through the CUDA library.
 """
 from __future__ import annotations
 
+import functools
 import hashlib
 import secrets
 from dataclasses import dataclass, field
@@ -84,6 +86,70 @@ class R1CS:
     commitment_wire: int = -1
 
 
+@dataclass
+class SparseR1CS:
+    """A constraint system as gnark stores it (constraint/r1cs.go): an interned coefficient table and, per matrix,
+    CSR arrays by constraint of Term{CID, VID} (provekit.InternedR1CS has the same shape).  Constraint j of L holds
+    the terms l_wire[l_row[j]:l_row[j+1]] with coefficients coeffs[l_coeff[...]]; likewise R and O.  This is what
+    b200g16_setup takes (struct b200g16_r1cs_desc)."""
+    nb_wires: int
+    nb_public: int
+    coeffs: np.ndarray             # (n, 4) fr.Element, Montgomery
+    l_row: np.ndarray              # uint64, n_constraints + 1
+    l_wire: np.ndarray             # uint32
+    l_coeff: np.ndarray            # uint32
+    r_row: np.ndarray
+    r_wire: np.ndarray
+    r_coeff: np.ndarray
+    o_row: np.ndarray
+    o_wire: np.ndarray
+    o_coeff: np.ndarray
+    private_committed: np.ndarray = field(default_factory=lambda: np.zeros(0, dtype=np.uint32))
+    public_committed: list = field(default_factory=list)
+    commitment_wire: int = -1
+
+    def __getitem__(self, name):   # the mapping lib.Context.setup reads
+        return getattr(self, name)
+
+    @staticmethod
+    def from_r1cs(r1cs):
+        """Intern the coefficients of a Python R1CS and lay its three matrices out as CSR; every term is kept, in
+        order (repeated wires and zero coefficients included)."""
+        ids = {}
+        out = {}
+        for k, p in enumerate("lro"):
+            row, wires, cids = [0], [], []
+            for con in r1cs.constraints:
+                for i, c in con[k]:
+                    wires.append(i)
+                    cids.append(ids.setdefault(c % R_MOD, len(ids)))
+                row.append(len(wires))
+            out[p + "_row"] = np.array(row, dtype=np.uint64)
+            out[p + "_wire"] = np.array(wires, dtype=np.uint32)
+            out[p + "_coeff"] = np.array(cids, dtype=np.uint32)
+        table = sorted(ids, key=ids.get)
+        return SparseR1CS(r1cs.nb_wires, r1cs.nb_public, fr_array(table) if table else np.zeros((0, 4), np.uint64),
+                          private_committed=np.array(r1cs.private_committed, dtype=np.uint32),
+                          public_committed=list(r1cs.public_committed), commitment_wire=r1cs.commitment_wire, **out)
+
+    @functools.cached_property
+    def constraints(self):
+        """[(L, R, O)] with [(wire, coeff)] terms, as R1CS.constraints (what solve_abc reads).  Built from the arrays on
+        first access and kept: the host prover walks it once per solve_abc, and rebuilding it per access costs seconds
+        at 2^16 constraints.  Change the arrays of a SparseR1CS before that first access, not after."""
+        cf = [_fr_from(c) for c in np.asarray(self.coeffs, dtype=np.uint64).reshape(-1, 4)]
+        mats = []
+        for p in "lro":
+            row, wire, cid = getattr(self, p + "_row"), getattr(self, p + "_wire").tolist(), getattr(self, p + "_coeff").tolist()
+            mats.append([[(wire[e], cf[cid[e]]) for e in range(int(row[j]), int(row[j + 1]))] for j in range(len(row) - 1)])
+        return list(zip(*mats))
+
+
+def _fr_from(limbs):
+    v = int(limbs[0]) | int(limbs[1]) << 64 | int(limbs[2]) << 128 | int(limbs[3]) << 192
+    return v * pow(_MONT, -1, R_MOD) % R_MOD
+
+
 def _lc(lc, w):
     return sum(c * w[i] for i, c in lc) % R_MOD
 
@@ -123,6 +189,7 @@ class ProvingKey:                  # groth16_bn254.ProvingKey
     CommitmentKeys: list = field(default_factory=list)
     _dev: object = None            # device handle, filled lazily on first Prove (like gnark's icicle pk)
     _ctx: object = None
+    _owned: list = field(default_factory=list)   # resident vectors DeviceSetup made; free() releases them
 
     def device_handle(self, ctx, precompute=False):
         """precompute=True: attach window tables to the resident point vectors at upload time
@@ -144,6 +211,9 @@ class ProvingKey:                  # groth16_bn254.ProvingKey
                 if b is not None:
                     b.free()
             ck.basis_dev = ck.basis_exp_sigma_dev = None
+        for b in self._owned:
+            b.free()
+        self._owned = []
 
 
 @dataclass
@@ -499,6 +569,39 @@ def Setup(ctx, r1cs, toxic=None):
         vk.PedersenG = g2
         vk.PedersenGSigmaNeg = ctx.fixed_base_mul(g2, fr_array([(-tw.sigma) % R_MOD]), group=2)[0]
         vk.PublicAndCommitmentCommitted = list(r1cs.public_committed)
+        vk.has_commitment = True
+    return pk, vk
+
+
+def DeviceSetup(ctx, r1cs, toxic=None, precompute=False):
+    """groth16.Setup(ccs) -> (pk, vk) computed on the GPU by b200g16_setup: the same key as Setup for the same toxic
+    waste, bit for bit.  r1cs: an R1CS or a SparseR1CS.  The proving key's point vectors stay resident (G1_A, G1_B,
+    G1_K, G1_Z, G2_B and the Pedersen basis_dev / basis_exp_sigma_dev are Bases); Prove, BatchProve, pk_write_to and
+    the verifier take the key as it is.  precompute=True attaches window tables to the five prove vectors.
+    pk.free() releases them."""
+    tw = toxic or ToxicWaste.random()
+    sp = r1cs if isinstance(r1cs, SparseR1CS) else SparseR1CS.from_r1cs(r1cs)
+    t = fr_array([tw.tau, tw.alpha, tw.beta, tw.gamma, tw.delta, tw.sigma])
+    o = ctx.setup(sp, *t)
+    owned = [o[n] for n in lib.SETUP_VECTORS if o[n] is not None]
+    vk_k = o["vk_k"].download()
+    o["vk_k"].free()
+    owned.remove(o["vk_k"])
+    if precompute:
+        for n in ("a", "b", "k", "z", "b2"):
+            if len(o[n]):
+                o[n].precompute(0)
+    pk = ProvingKey(o["log2_domain"], o["g1_alpha"], o["g1_beta"], o["g1_delta"], o["a"], o["b"], o["z"], o["k"],
+                    o["g2_beta"], o["g2_delta"], o["b2"], o["infinity_a"], o["infinity_b"], o["k_skip"], _owned=owned)
+    vk = VerifyingKey(o["g1_alpha"], vk_k, o["g2_beta"], o["g2_gamma"], o["g2_delta"], G1_Beta=o["g1_beta"],
+                      G1_Delta=o["g1_delta"])
+    if sp.commitment_wire >= 0:
+        basis, bes = o["ped_basis"], o["ped_basis_exp_sigma"]
+        pk.CommitmentKeys = [PedersenProvingKey(basis, bes, basis_dev=basis, basis_exp_sigma_dev=bes)]
+        owned.remove(basis)
+        owned.remove(bes)
+        vk.PedersenG, vk.PedersenGSigmaNeg = o["ped_g"], o["ped_g_sigma_neg"]
+        vk.PublicAndCommitmentCommitted = list(sp.public_committed)
         vk.has_commitment = True
     return pk, vk
 

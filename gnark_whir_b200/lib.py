@@ -85,6 +85,8 @@ SIGNATURES = {
     "b200g16_prove_begin_dev": (C.c_int, [_vp, _vp, _vp]),
     "b200g16_prove_end_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "b200g16_prove_finish": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200g16_setup": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b200g16_setup_wire_polys": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "b200g16_pairing_check": (C.c_int, [_vp, _vp, _vp, _sz, C.POINTER(C.c_int)]),
     "b200g16_pair": (C.c_int, [_vp, _vp, _vp, _sz, _vp]),
     "b200g16_verify": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(C.c_int)]),
@@ -229,6 +231,10 @@ def g2_scalar_mul(p, k):
     return out
 
 
+# bases handles of struct b200g16_setup_out, in field order
+SETUP_VECTORS = ("a", "b", "k", "z", "b2", "vk_k", "ped_basis", "ped_basis_exp_sigma")
+
+
 class PkDesc(C.Structure):
     """struct b200g16_pk_desc (include/b200g16.h)"""
     _fields_ = [
@@ -241,6 +247,51 @@ class PkDesc(C.Structure):
         ("partial", C.c_int), ("off_a", _sz), ("off_b", _sz), ("off_k", _sz), ("off_z", _sz),
         ("precompute", C.c_int),
     ]
+
+
+class R1csDesc(C.Structure):
+    """struct b200g16_r1cs_desc (include/b200g16.h)"""
+    _fields_ = [("n_constraints", _sz), ("n_wires", _sz), ("n_public", _sz), ("coeffs", _vp), ("n_coeffs", _sz),
+                ("l_row", _vp), ("l_wire", _vp), ("l_coeff", _vp), ("r_row", _vp), ("r_wire", _vp), ("r_coeff", _vp),
+                ("o_row", _vp), ("o_wire", _vp), ("o_coeff", _vp), ("private_committed", _vp),
+                ("n_private_committed", _sz), ("commitment_wire", C.c_int64)]
+
+
+class Toxic(C.Structure):
+    """struct b200g16_toxic (include/b200g16.h)"""
+    _fields_ = [(n, C.c_uint64 * 4) for n in ("tau", "alpha", "beta", "gamma", "delta", "sigma")]
+
+
+class SetupOut(C.Structure):
+    """struct b200g16_setup_out (include/b200g16.h)"""
+    _fields_ = ([("log2_domain", C.c_uint)] + [(n, _vp) for n in SETUP_VECTORS]
+                + [(n, C.c_uint64 * 8) for n in ("g1_alpha", "g1_beta", "g1_delta")]
+                + [(n, C.c_uint64 * 16) for n in ("g2_beta", "g2_delta", "g2_gamma", "ped_g", "ped_g_sigma_neg")])
+
+
+def _r1cs_desc(r):
+    """struct b200g16_r1cs_desc from a mapping with the fields of groth16.SparseR1CS -> (desc, arrays to keep alive)"""
+    keep = {"coeffs": _u64(r["coeffs"], 4), "private_committed": np.ascontiguousarray(r["private_committed"], np.uint32)}
+    for p in "lro":
+        keep[p + "_row"] = np.ascontiguousarray(r[p + "_row"], dtype=np.uint64)
+        keep[p + "_wire"] = np.ascontiguousarray(r[p + "_wire"], dtype=np.uint32)
+        keep[p + "_coeff"] = np.ascontiguousarray(r[p + "_coeff"], dtype=np.uint32)
+    m = len(keep["l_row"]) - 1
+    for p in "lro":    # the library reads row[0 .. m] and the first row[m] terms of every matrix
+        row = keep[p + "_row"]
+        if m < 0 or len(row) != m + 1:
+            raise B200Error(f"r1cs: {p}_row has {len(row)} entries, l_row {m + 1}: one row array per matrix, same length")
+        if len(keep[p + "_wire"]) < row[-1] or len(keep[p + "_coeff"]) < row[-1]:
+            raise B200Error(f"r1cs: {p}_row ends at {int(row[-1])} but {p}_wire / {p}_coeff hold fewer terms")
+    d = R1csDesc()
+    d.n_constraints = m
+    d.n_wires, d.n_public = int(r["nb_wires"]), int(r["nb_public"])
+    d.n_coeffs = keep["coeffs"].shape[0]
+    d.n_private_committed = keep["private_committed"].shape[0]
+    d.commitment_wire = int(r["commitment_wire"])
+    for name, a in keep.items():
+        setattr(d, name, _ptr(a) if a.size else None)
+    return d, keep
 
 
 class VkDesc(C.Structure):
@@ -488,6 +539,39 @@ class Context:
         fn = lib.b200g16_fixed_base_mul_g1 if group == 1 else lib.b200g16_fixed_base_mul_g2
         _check(fn(self.h, _ptr(base), _ptr(sc), n, _ptr(out)))
         return out
+
+    # -- Groth16 setup (b200g16_setup)
+    def setup(self, r1cs, tau, alpha, beta, gamma, delta, sigma):
+        """The key of a constraint system (a mapping with groth16.SparseR1CS's fields) for the given toxic waste
+        (Montgomery fr.Elements, 4 limbs each) -> dict: log2_domain, the resident vectors as Bases (a, b, k, z, b2,
+        vk_k, ped_basis, ped_basis_exp_sigma; the last two None without a commitment), the small points
+        (g1_alpha ... ped_g_sigma_neg) and the host flags infinity_a, infinity_b, k_skip."""
+        d, keep = _r1cs_desc(r1cs)
+        t = Toxic()
+        for name, v in zip(("tau", "alpha", "beta", "gamma", "delta", "sigma"), (tau, alpha, beta, gamma, delta, sigma)):
+            getattr(t, name)[:] = [int(x) for x in _u64(v).reshape(4)]
+        nw = int(d.n_wires)
+        flags = [np.zeros(nw, dtype=np.uint8) for _ in range(3)]
+        out = SetupOut()
+        _check(load().b200g16_setup(self.h, C.byref(d), C.byref(t), *[_ptr(f) for f in flags], C.byref(out)))
+        del keep
+        res = {"log2_domain": int(out.log2_domain), "infinity_a": flags[0], "infinity_b": flags[1], "k_skip": flags[2]}
+        for name in SETUP_VECTORS:
+            h = getattr(out, name)
+            res[name] = None if not h else Bases(self, _vp(h), 2 if name == "b2" else 1,
+                                                 int(load().b200g16_bases_len(_vp(h))))
+        for name, _ in SetupOut._fields_[1 + len(SETUP_VECTORS):]:
+            res[name] = np.array(getattr(out, name)[:], dtype=np.uint64)
+        return res
+
+    def setup_wire_polys(self, r1cs, tau):
+        """gnark's setupABC on the GPU: (A, B, C) per wire at tau, each (n_wires, 4) Montgomery."""
+        d, keep = _r1cs_desc(r1cs)
+        out = [np.zeros((int(d.n_wires), 4), dtype=np.uint64) for _ in range(3)]
+        tau = _u64(tau).reshape(4)
+        _check(load().b200g16_setup_wire_polys(self.h, C.byref(d), _ptr(tau), *[_ptr(o) for o in out]))
+        del keep
+        return tuple(out)
 
     def modmul_probe(self, blocks_per_sm=4, chains=4, iters=2000):
         rate = C.c_double()

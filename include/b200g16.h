@@ -116,7 +116,7 @@ void b200g16_destroy(b200g16_ctx* ctx);
 /* Number of CUDA kernels this ctx has launched so far (bench.py's gpu_launches). */
 uint64_t b200g16_launch_count(const b200g16_ctx* ctx);
 /* Device time (ms, CUDA events on the ctx stream) of the phases of the last MSM /
- * computeH call: writes up to `cap` floats, returns how many. */
+ * computeH / prove / setup call: writes up to `cap` floats, returns how many. */
 int b200g16_last_timings(const b200g16_ctx* ctx, float* out_ms, int cap);
 /* Force the Pippenger window width (0 = automatic). Testing / tuning only. */
 int b200g16_set_msm_window(b200g16_ctx* ctx, int c);
@@ -385,6 +385,72 @@ int b200g16_prove_batch(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const 
  * memory. */
 int b200g16_prove_batch_dev(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const void* d_wires, void* d_a,
                             void* d_b, void* d_c, const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out);
+
+/* ---- Groth16 setup ----------------------------------------------------------------------- */
+/* A rank-1 constraint system as gnark's R1CS stores it (constraint/r1cs.go: a Coefficients table and, per
+ * constraint, the terms Term{CID, VID} of L, R and O).  Each matrix is CSR by constraint: constraint j has the
+ * entries [row[j], row[j+1]) of wire[] / coeff[]; row has n_constraints + 1 entries, row[0] = 0, and
+ * nnz = row[n_constraints] is that matrix's number of terms.  A wire may appear more than once in a row (the terms
+ * add up); zero coefficients and empty rows are allowed.  At most one BSB22 commitment. */
+typedef struct b200g16_r1cs_desc {
+  size_t n_constraints, n_wires, n_public;   /* n_public counts wire 0 (the constant one)             */
+  const uint64_t* coeffs;                    /* coefficient table: n_coeffs fr.Elements (Montgomery)  */
+  size_t n_coeffs;
+  const uint64_t* l_row; const uint32_t* l_wire; const uint32_t* l_coeff;
+  const uint64_t* r_row; const uint32_t* r_wire; const uint32_t* r_coeff;
+  const uint64_t* o_row; const uint32_t* o_wire; const uint32_t* o_coeff;
+  const uint32_t* private_committed;         /* committed private wires, strictly increasing          */
+  size_t n_private_committed;
+  int64_t commitment_wire;                   /* wire receiving the BSB22 challenge; -1: no commitment */
+} b200g16_r1cs_desc;
+/* The toxic waste, fr.Elements (Montgomery). */
+typedef struct b200g16_toxic {
+  uint64_t tau[4], alpha[4], beta[4], gamma[4], delta[4], sigma[4];
+} b200g16_toxic;
+/* The key b200g16_setup produces.  Point vectors are new resident bases handles the caller frees with
+ * b200g16_bases_free (an empty vector is a valid n = 0 handle); they go straight into b200g16_pk_desc.res_*. */
+typedef struct b200g16_setup_out {
+  unsigned log2_domain;                      /* N = 2^log2_domain                                     */
+  b200g16_bases* a;                          /* pk.G1.A  (G1)                                         */
+  b200g16_bases* b;                          /* pk.G1.B  (G1)                                         */
+  b200g16_bases* k;                          /* pk.G1.K  (G1)                                         */
+  b200g16_bases* z;                          /* pk.G1.Z  (G1, N - 1 points)                           */
+  b200g16_bases* b2;                         /* pk.G2.B  (G2)                                         */
+  b200g16_bases* vk_k;                       /* vk.G1.K  (G1): public wires, then the commitment wire  */
+  b200g16_bases* ped_basis;                  /* pedersen Basis, BasisExpSigma (G1); NULL without a     */
+  b200g16_bases* ped_basis_exp_sigma;        /*   commitment                                          */
+  uint64_t g1_alpha[8], g1_beta[8], g1_delta[8];
+  uint64_t g2_beta[16], g2_delta[16], g2_gamma[16];
+  uint64_t ped_g[16], ped_g_sigma_neg[16];   /* pedersen G = the G2 generator, GSigmaNeg = [-sigma] G  */
+} b200g16_setup_out;
+/* groth16.Setup (gnark backend/groth16/bn254/setup.go; reference mt.go:448) with explicit toxic waste, on the GPU
+ * from the constraint matrices to the resident proving key.  The key is bit-identical to gnark's for the same toxic
+ * waste:
+ *   N = 2^ceil(log2 n_constraints); A_i, B_i, C_i = sum of coeff * L_j(tau) over wire i's terms of L, R, O
+ *   K_i = beta A_i + alpha B_i + C_i:  public wires and then the commitment wire: K_i / gamma -> vk.G1.K;
+ *     committed private wires: K_i / gamma -> pedersen Basis (committed-list order), sigma times that -> BasisExpSigma;
+ *     every other wire: K_i / delta -> pk.G1.K (wire order)
+ *   pk.G1.A, pk.G1.B, pk.G2.B: the wires with A_i != 0 (B_i != 0), in wire order
+ *   pk.G1.Z[i] = (tau^N - 1) / delta * tau^bitrev(i), i < N - 1
+ * infinity_a[i] = (A_i == 0), infinity_b[i] = (B_i == 0), k_skip[i] = 1 for public, committed and commitment wires
+ * (as b200g16_pk_desc takes it): n_wires bytes each, host, written on success.
+ * B200G16_ERR_ARG, with nothing left allocated: NULL arguments, n_constraints = 0 or N > 2^28, n_wires >= 2^32,
+ * n_public = 0 or > n_wires, a row array that does not start at 0 or decreases, more than 15 * 2^28 terms in one matrix, a wire
+ * >= n_wires, a coefficient id >= n_coeffs, a committed list that is not strictly increasing inside
+ * [n_public, n_wires), a commitment wire < n_public, >= n_wires or in that list (or committed wires without one),
+ * gamma = 0, delta = 0, and tau^N = 1.  The last is a deliberate deviation: gnark divides by tau - w^j and
+ * would fail or produce a degenerate key; a sampled tau never hits it.  The index arrays are checked on the
+ * GPU (one flag read back).  B200G16_ERR_STATE between b200g16_prove_begin_dev and _end_dev.  Any error leaves
+ * the ctx usable.  The setup's scratch is its own and is released on return.
+ * b200g16_last_timings: upload + checks, tau powers + Lagrange values, accumulation of L, R, O, K values +
+ * compaction + Z scalars, G1 points, G2 points, flags and small points to the host. */
+int b200g16_setup(b200g16_ctx* ctx, const b200g16_r1cs_desc* r1cs, const b200g16_toxic* toxic,
+                  uint8_t* infinity_a, uint8_t* infinity_b, uint8_t* k_skip, b200g16_setup_out* out);
+/* gnark's setupABC alone: A_i(tau), B_i(tau), C_i(tau) for every wire, n_wires fr.Elements each (host; any of the
+ * three may be NULL).  The same checks as b200g16_setup on the system, except that tau^N = 1 is accepted (the
+ * Lagrange values are then 0 / 1). */
+int b200g16_setup_wire_polys(b200g16_ctx* ctx, const b200g16_r1cs_desc* r1cs, const uint64_t tau[4],
+                             uint64_t* a_out, uint64_t* b_out, uint64_t* c_out);
 
 /* ---- pairing / Groth16 verify ----------------------------------------------------------- */
 /* groth16_bn254.VerifyingKey as Verify needs it (gnark backend/groth16/bn254/verify.go). */

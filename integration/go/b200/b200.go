@@ -40,6 +40,7 @@ type ProvingKey struct {
 	dev       *C.b200g16_pk
 	pedBasis  []*C.b200g16_bases // pk.CommitmentKeys[i].Basis
 	pedSigma  []*C.b200g16_bases // pk.CommitmentKeys[i].BasisExpSigma
+	owned     []*C.b200g16_bases // resident vectors Setup made and the device key borrows
 }
 
 func u64(p unsafe.Pointer) *C.uint64_t { return (*C.uint64_t)(p) }
@@ -429,6 +430,10 @@ func (pk *ProvingKey) Free() {
 		C.b200g16_pk_free(pk.dev)
 		pk.dev = nil
 	}
+	for _, b := range pk.owned {
+		C.b200g16_bases_free(b)
+	}
+	pk.owned = nil
 	if pk.ctx != nil {
 		C.b200g16_destroy(pk.ctx)
 		pk.ctx = nil
