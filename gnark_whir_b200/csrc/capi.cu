@@ -282,6 +282,32 @@ static void host_scalar_mul(const uint64_t* p, const uint64_t* k, uint64_t* out)
   Affine<F> r = acc.to_affine();
   memcpy(out, &r, sizeof(r));
 }
+
+// A new vector on `device` with src's points (its window table included), the copy enqueued on `st` (a stream of
+// that device, which must be current) and not waited for.  A resident vector is complete once the call that made it
+// returned (upload, precompute, setup and fixed-base calls all synchronise), so the copy needs no wait on src.
+int bases_copy_enqueue(int device, cudaStream_t st, const b200g16_bases* src, b200g16_bases** out) {
+  const size_t sz = src->group == 1 ? sizeof(G1Affine) : sizeof(G2Affine);
+  const size_t rows = src->tab_c ? (size_t)src->tab_W : 1;
+  const size_t bytes = src->n * rows * sz;
+  b200g16_bases* b = new b200g16_bases();
+  b->group = src->group;
+  b->n = src->n;
+  b->device = device;
+  b->tab_c = src->tab_c;
+  b->tab_W = src->tab_W;
+  cudaError_t e = cudaMalloc(&b->d_points, bytes ? bytes : sz);
+  if (e == cudaSuccess && bytes) e = cudaMemcpyPeerAsync(b->d_points, device, src->d_points, src->device, bytes, st);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    if (b->d_points) cudaFree(b->d_points);
+    delete b;
+    return fail(B200G16_ERR_CUDA, "bases_copy: %zu bytes from device %d to %d: %s", bytes, src->device, device,
+                cudaGetErrorString(e));
+  }
+  *out = b;
+  return 0;
+}
 }  // namespace b200
 
 using namespace b200;
@@ -421,6 +447,21 @@ int b200g16_bases_download(const b200g16_bases* b, size_t offset, size_t n, uint
   size_t sz = b->group == 1 ? sizeof(G1Affine) : sizeof(G2Affine);
   B200_CUDA(cudaSetDevice(b->device));
   B200_CUDA(cudaMemcpy(out, (const char*)b->d_points + offset * sz, n * sz, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+int b200g16_bases_copy(b200g16_ctx* ctx, const b200g16_bases* src, b200g16_bases** out) {
+  if (!ctx || !src || !out) return fail(B200G16_ERR_ARG, "bases_copy: null");
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  B200_CUDA(cudaSetDevice(ctx->device));
+  b200g16_bases* b = nullptr;
+  B200_TRY(bases_copy_enqueue(ctx->device, ctx->stream, src, &b));
+  cudaError_t e = cudaStreamSynchronize(ctx->stream);
+  if (e != cudaSuccess) {
+    b200g16_bases_free(b);
+    return fail(B200G16_ERR_CUDA, "bases_copy: %s", cudaGetErrorString(e));
+  }
+  *out = b;
   return 0;
 }
 

@@ -12,6 +12,8 @@
 //     host: the n x 5 partial points are added (n - 1 additions each) and the proof is assembled
 // No NCCL, no collective library: the only data crossing devices are two vectors into the root, one slice of h
 // out to each device, and 5 points per device back to the host.
+#include <algorithm>
+#include <array>
 #include <condition_variable>
 #include <thread>
 
@@ -37,10 +39,16 @@ struct b200g16_group_bases {
   std::vector<size_t> lo;
 };
 
+// sharded (b200g16_group_pk_upload): shard[i] holds a point range of every vector; replicated
+// (b200g16_group_pk_replicate): shard[i] is the whole key on member i's device, its vectors borrowed from the source
+// or from `copies` (one set per distinct device other than the source's, shared by the members on that device)
 struct b200g16_group_pk {
   unsigned log2n = 0;
   size_t n_wires = 0;
   std::vector<b200g16_pk*> shard;
+  bool replicated = false;
+  const b200g16_group* group = nullptr;   // the group that built it
+  std::vector<b200g16_bases*> copies;
 };
 
 namespace {
@@ -276,6 +284,7 @@ int b200g16_group_pk_upload(b200g16_group* g, const b200g16_pk_desc* d, b200g16_
   b200g16_group_pk* pk = new b200g16_group_pk();
   pk->log2n = d->log2_domain;
   pk->n_wires = d->n_wires;
+  pk->group = g;
   pk->shard.assign(g->n, nullptr);
   int st = run_on_all(g, [&](int i) {
     b200g16_pk_desc s = *d;
@@ -303,7 +312,97 @@ int b200g16_group_pk_upload(b200g16_group* g, const b200g16_pk_desc* d, b200g16_
 void b200g16_group_pk_free(b200g16_group_pk* pk) {
   if (!pk) return;
   for (auto* s : pk->shard) pk_release(s);
+  for (auto* b : pk->copies) b200g16_bases_free(b);
   delete pk;
+}
+
+// ---- replicated proving key: the whole key on every device, for whole proofs per device
+int b200g16_group_pk_replicate(b200g16_group* g, const b200g16_pk* src, b200g16_group_pk** out) {
+  if (!g || !src || !out) return fail(B200G16_ERR_ARG, "group_pk_replicate: null");
+  if (src->partial) return fail(B200G16_ERR_ARG, "group_pk_replicate: a partial (sharded) key cannot be replicated");
+  std::lock_guard<std::mutex> glock(g->mu);
+  const int n = g->n;
+  // the distinct devices in group order; the first member on each lends its ctx (stream, lock) to the copies
+  std::vector<int> dev, lead, slot(n);
+  for (int i = 0; i < n; i++) {
+    const auto it = std::find(dev.begin(), dev.end(), g->devices[i]);
+    slot[i] = (int)(it - dev.begin());
+    if (it == dev.end()) { dev.push_back(g->devices[i]); lead.push_back(i); }
+  }
+  const int D = (int)dev.size();
+  std::vector<std::unique_lock<std::mutex>> locks;
+  for (int d = 0; d < D; d++) locks.emplace_back(g->ctx[lead[d]]->mu);
+  b200g16_group_pk* gpk = new b200g16_group_pk();
+  gpk->log2n = src->log2n;
+  gpk->n_wires = src->n_wires;
+  gpk->replicated = true;
+  gpk->group = g;
+  gpk->shard.assign(n, nullptr);
+  std::vector<std::array<b200g16_bases*, 5>> vecs(D);
+  std::vector<cudaEvent_t> ready(D, nullptr);   // ready[d]: the copies onto dev[d] are complete
+  std::vector<int> holders, todo;               // holders: devices that can serve a copy (-1: src, off the group)
+  for (int d = 0; d < D; d++) {
+    if (dev[d] == src->device) {
+      for (int v = 0; v < 5; v++) vecs[d][v] = src->vec[v];
+      holders.push_back(d);
+    } else {
+      todo.push_back(d);
+    }
+  }
+  if (holders.empty()) holders.push_back(-1);
+  auto body = [&]() -> int {
+    // doubling broadcast: each round, every holder serves one device that has no copy yet
+    for (size_t next = 0; next < todo.size();) {
+      std::vector<int> fresh;
+      for (int h : holders) {
+        if (next == todo.size()) break;
+        const int d = todo[next++];
+        b200g16_ctx* c = g->ctx[lead[d]];
+        B200_CUDA(cudaSetDevice(c->device));
+        if (h >= 0 && ready[h]) B200_CUDA(cudaStreamWaitEvent(c->stream, ready[h], 0));
+        for (int v = 0; v < 5; v++) {
+          B200_TRY(bases_copy_enqueue(c->device, c->stream, h >= 0 ? vecs[h][v] : src->vec[v], &vecs[d][v]));
+          gpk->copies.push_back(vecs[d][v]);
+        }
+        B200_CUDA(cudaEventCreateWithFlags(&ready[d], cudaEventDisableTiming));
+        B200_CUDA(cudaEventRecord(ready[d], c->stream));
+        fresh.push_back(d);
+      }
+      holders.insert(holders.end(), fresh.begin(), fresh.end());
+    }
+    // every member: the key's small points and sizes, the vectors of its device, its own gather lists
+    for (int i = 0; i < n; i++) {
+      const int d = slot[i];
+      b200g16_ctx* c = g->ctx[lead[d]];
+      B200_CUDA(cudaSetDevice(c->device));
+      b200g16_pk* pk = new b200g16_pk(*src);
+      for (int t = 0; t < 3; t++) pk->d_idx[t] = nullptr;
+      for (int v = 0; v < 5; v++) { pk->vec[v] = vecs[d][v]; pk->owned[v] = false; }
+      pk->device = c->device;
+      gpk->shard[i] = pk;
+      for (int t = 0; t < 3; t++) {
+        B200_CUDA(cudaMalloc(&pk->d_idx[t], (pk->n_idx[t] ? pk->n_idx[t] : 1) * sizeof(uint32_t)));
+        if (pk->n_idx[t])
+          B200_CUDA(cudaMemcpyPeerAsync(pk->d_idx[t], c->device, src->d_idx[t], src->device, pk->n_idx[t] * sizeof(uint32_t),
+                                        c->stream));
+      }
+    }
+    return 0;
+  };
+  int st = body();
+  for (int d = 0; d < D; d++) {   // every copy complete (or, after a failure, nothing in flight any more)
+    b200g16_ctx* c = g->ctx[lead[d]];
+    cudaSetDevice(c->device);
+    cudaError_t e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess && !st) st = fail(B200G16_ERR_CUDA, "group_pk_replicate: device %d: %s", c->device, cudaGetErrorString(e));
+    if (ready[d]) cudaEventDestroy(ready[d]);
+  }
+  if (st) {
+    b200g16_group_pk_free(gpk);
+    return st;
+  }
+  *out = gpk;
+  return 0;
 }
 
 static int dist_h_alloc(b200g16_ctx* ctx, unsigned log2n, int n_peers, int me);
@@ -397,6 +496,8 @@ int b200g16_group_prove(b200g16_group* g, const b200g16_group_pk* gpk, const uin
                         const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints, const uint64_t r[4],
                         const uint64_t s[4], b200g16_proof* proof_out, uint64_t* h_out) {
   if (!g || !gpk || !wires || !a || !b || !c || !r || !s || !proof_out) return fail(B200G16_ERR_ARG, "group_prove: null");
+  if (gpk->replicated)
+    return fail(B200G16_ERR_ARG, "group_prove: a replicated key proves whole proofs per device (b200g16_group_prove_batch)");
   if ((int)gpk->shard.size() != g->n) return fail(B200G16_ERR_STATE, "group_prove: pk belongs to another group");
   if (n_wires != gpk->n_wires) return fail(B200G16_ERR_ARG, "group_prove: %zu wires, pk expects %zu", n_wires, gpk->n_wires);
   const int L = (int)gpk->log2n;
@@ -521,6 +622,41 @@ int b200g16_group_prove(b200g16_group* g, const b200g16_group_pk* gpk, const uin
     B200_CUDA(cudaMemcpy(h_out, g->ctx[root]->ntt.a.p, N * sizeof(Fr), cudaMemcpyDeviceToHost));
   }
   return 0;
+}
+
+// ---- k proofs over the group with a replicated key: contiguous ranges of proofs, b200g16_prove_batch's pipeline on
+// every member from its own host thread, no data across devices
+int b200g16_group_prove_batch(b200g16_group* g, const b200g16_group_pk* gpk, size_t k, const uint64_t* wires,
+                              size_t n_wires, const uint64_t* a, const uint64_t* b, const uint64_t* c,
+                              size_t n_constraints, const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out) {
+  if (!g || !gpk) return fail(B200G16_ERR_ARG, "group_prove_batch: null");
+  if (k && (!wires || !a || !b || !c || !r || !s || !proofs_out)) return fail(B200G16_ERR_ARG, "group_prove_batch: null");
+  if (gpk->group != g || (int)gpk->shard.size() != g->n)
+    return fail(B200G16_ERR_STATE, "group_prove_batch: pk belongs to another group");
+  if (!gpk->replicated)
+    return fail(B200G16_ERR_ARG, "group_prove_batch: a sharded key proves one proof over the group (b200g16_group_prove)");
+  if (n_wires != gpk->n_wires)
+    return fail(B200G16_ERR_ARG, "group_prove_batch: %zu wires, pk expects %zu", n_wires, gpk->n_wires);
+  const size_t N = (size_t)1 << gpk->log2n;
+  if (n_constraints > N) return fail(B200G16_ERR_ARG, "group_prove_batch: %zu constraints > domain %zu", n_constraints, N);
+  if (k && (n_wires > SIZE_MAX / sizeof(Fr) / k || N > SIZE_MAX / sizeof(Fr) / k))
+    return fail(B200G16_ERR_ARG, "group_prove_batch: k x n_wires or k x N overflows");
+  if (k == 0) return 0;
+  std::lock_guard<std::mutex> glock(g->mu);
+  const int st = run_on_all(g, [&](int i) -> int {
+    size_t lo, hi;
+    shard_range(k, i, g->n, &lo, &hi);
+    if (lo == hi) return 0;
+    b200g16_ctx* ctx = g->ctx[i];
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    B200_CUDA(cudaSetDevice(ctx->device));
+    return prove_from_host(ctx, gpk->shard[i], hi - lo, wires + lo * n_wires * 4, n_wires, a + lo * n_constraints * 4,
+                           b + lo * n_constraints * 4, c + lo * n_constraints * 4, n_constraints, r + lo * 4, s + lo * 4,
+                           proofs_out + lo);
+  });
+  if (st)   // (the failing member has drained its own streams; nothing of the others may still run either)
+    for (int i = 0; i < g->n; i++) { cudaSetDevice(g->ctx[i]->device); cudaStreamSynchronize(g->ctx[i]->stream); }
+  return st;
 }
 
 // ---- computeH split over 2 / 4 / 8 GPUs, one PROCESS per GPU (torch.distributed ranks): CUDA IPC maps every

@@ -401,7 +401,7 @@ static int prove_batch_check(b200g16_ctx* ctx, const b200g16_pk* pk, const char*
 // first: it gates the four MSMs, which are enqueued BEFORE a, b, c are touched — a copy from pageable memory (a Go
 // slice) occupies the calling thread while it is staged, and the GPU should already be busy.  a, b, c then cross PCIe
 // on the copy stream under those MSMs.
-static int prove_from_host(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const uint64_t* wires, size_t n_wires,
+int prove_from_host(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const uint64_t* wires, size_t n_wires,
                            const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints,
                            const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out) {
   const size_t N = (size_t)1 << pk->log2n;

@@ -66,4 +66,10 @@ int prove_back(b200g16_ctx* ctx, const b200g16_pk* pk, const Fr* d_h, size_t h_s
                const Fr* s, b200g16_proof* out, int* ev_io);
 template <class F>
 Affine<F> host_sum_points(const Affine<F>* pts, int n);
+// The host path of b200g16_prove_batch, called under ctx->mu on ctx's device: k proofs of a whole pk from host rows
+int prove_from_host(b200g16_ctx* ctx, const b200g16_pk* pk, size_t k, const uint64_t* wires, size_t n_wires,
+                    const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints,
+                    const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out);
+// a copy of src on `device` enqueued on st (capi.cu); complete once st has passed it
+int bases_copy_enqueue(int device, cudaStream_t st, const b200g16_bases* src, b200g16_bases** out);
 }  // namespace b200

@@ -686,6 +686,129 @@ def BatchProve(ctx, r1cs, pk, witnesses, rs=None, ss=None, resolve=None):
     return proofs
 
 
+class GroupProvingKey:
+    """A ProvingKey (from Setup or DeviceSetup) on every device of a lib.Group, for GroupBatchProve.
+
+    The key is first made resident on one device: where its vectors already are (DeviceSetup, or a key Prove has
+    uploaded), else on `ctx` (default: the group's first member).  It is then replicated over the group
+    (b200g16_group_pk_replicate: device-to-device copies, window tables included).  With a commitment, the Pedersen
+    bases reach each member's device the same way (b200g16_bases_copy).  free() releases the replica and the copies,
+    never pk itself; call it before the group is closed."""
+
+    def __init__(self, group, pk, ctx=None, precompute=False):
+        self.group, self.pk = group, pk
+        if pk._dev is not None:
+            src_ctx = pk._ctx
+        elif isinstance(pk.G1_A, lib.Bases):
+            src_ctx = pk.G1_A.ctx
+        else:
+            src_ctx = ctx if ctx is not None else group.ctx(0)
+        self.ctxs = [group.ctx(i) for i in range(len(group))]
+        self.handle = group.pk_replicate(pk.device_handle(src_ctx, precompute=precompute))
+        self._copies = []
+        self.pedersen = None        # per member: (Basis, BasisExpSigma) on its device
+        if pk.CommitmentKeys:
+            ck = pk.CommitmentKeys[0]
+            if ck.basis_dev is None:
+                ck.basis_dev = src_ctx.upload_g1(ck.Basis)
+                ck.basis_exp_sigma_dev = src_ctx.upload_g1(ck.BasisExpSigma)
+            on_device = {}
+            for c in self.ctxs:
+                if c.device not in on_device:
+                    if c.device == ck.basis_dev.ctx.device:
+                        on_device[c.device] = (ck.basis_dev, ck.basis_exp_sigma_dev)
+                    else:
+                        on_device[c.device] = (c.bases_copy(ck.basis_dev), c.bases_copy(ck.basis_exp_sigma_dev))
+                        self._copies += on_device[c.device]
+            self.pedersen = [on_device[c.device] for c in self.ctxs]
+
+    @property
+    def log2_domain(self):
+        return self.pk.log2_domain
+
+    def free(self):
+        if self.handle is not None:
+            self.group.pk_free(self.handle)
+            self.handle = None
+        for b in self._copies:
+            b.free()
+        self._copies = []
+        self.pedersen = None
+
+
+def _ranges(k, n):
+    """Contiguous ranges of k items over n members, sizes differing by at most one (the library's split)."""
+    base, rem = divmod(k, n)
+    out, lo = [], 0
+    for i in range(n):
+        hi = lo + base + (1 if i < rem else 0)
+        out.append((lo, hi))
+        lo = hi
+    return out
+
+
+def _on_members(ctxs, k, fn):
+    """fn(i, lo, hi) for every member with a non-empty range, one thread per member (the library calls release the
+    GIL); the first exception is raised."""
+    import threading
+    errs = []
+
+    def run(i, lo, hi):
+        try:
+            fn(i, lo, hi)
+        except BaseException as e:   # noqa: BLE001 - re-raised below
+            errs.append(e)
+    th = [threading.Thread(target=run, args=(i, lo, hi)) for i, (lo, hi) in enumerate(_ranges(k, len(ctxs))) if hi > lo]
+    for t in th:
+        t.start()
+    for t in th:
+        t.join()
+    if errs:
+        raise errs[0]
+
+
+def GroupBatchProve(group, r1cs, gpk, witnesses, rs=None, ss=None, resolve=None):
+    """BatchProve over the devices of a group with a GroupProvingKey: the same k proofs, bit for bit, in one
+    b200g16_group_prove_batch call (contiguous ranges of proofs per member).  With a commitment, the Pedersen Commit
+    and ProveKnowledge batch MSMs are split over the members the same way, one thread each."""
+    ws = [list(w) for w in witnesses]
+    k = len(ws)
+    rs = [secrets.randbelow(R_MOD) for _ in range(k)] if rs is None else list(rs)
+    ss = [secrets.randbelow(R_MOD) for _ in range(k)] if ss is None else list(ss)
+    if len(rs) != k or len(ss) != k:
+        raise ValueError("groth16.GroupBatchProve: one r and one s per witness")
+    if k == 0:
+        return []
+    coms, poks = [[] for _ in range(k)], [None] * k
+    if r1cs.commitment_wire >= 0:
+        vals = np.stack([fr_array([w[i] for i in r1cs.private_committed]).reshape(-1, 4) for w in ws])
+        com, pok = [None] * k, [None] * k
+
+        def commit(i, lo, hi):
+            com[lo:hi] = list(gpk.ctxs[i].msm_batch(gpk.pedersen[i][0], vals[lo:hi]))
+        _on_members(gpk.ctxs, k, commit)                            # pedersen Commit of every witness
+        for j, w in enumerate(ws):
+            w[r1cs.commitment_wire] = commitment_challenge(com[j], [w[i] for i in r1cs.public_committed])
+            if resolve is not None:
+                resolve(w)
+
+        def knowledge(i, lo, hi):
+            pok[lo:hi] = list(gpk.ctxs[i].msm_batch(gpk.pedersen[i][1], vals[lo:hi]))
+        _on_members(gpk.ctxs, k, knowledge)                         # pedersen ProveKnowledge of every witness
+        coms = [[com[j]] for j in range(k)]
+        poks = pok
+    abc = [solve_abc(r1cs, w) for w in ws]
+    outs = group.prove_batch(gpk.handle, np.stack([fr_array(w).reshape(-1, 4) for w in ws]),
+                             *[np.stack([fr_array(t[i]).reshape(-1, 4) for t in abc]) for i in range(3)],
+                             fr_array(rs).reshape(k, 4), fr_array(ss).reshape(k, 4))
+    proofs = []
+    for j, out in enumerate(outs):
+        dbg = dict(out)
+        dbg["witness"] = ws[j]
+        proofs.append(Proof(out["ar"], out["krs"], out["bs"], coms[j], poks[j], dbg))
+    return proofs
+
+
 def _verify_inputs(proof, vk, public_witness):
     """The public inputs b200g16_verify takes for one proof (the public witness, then the BSB22 challenge when the
     circuit has a commitment) and the proof's commitment and proof of knowledge (None without one)."""

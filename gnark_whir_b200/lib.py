@@ -45,6 +45,7 @@ SIGNATURES = {
     "b200g16_bases_window": (C.c_int, [_vp]),
     "b200g16_msm_plan": (C.c_int, [_vp, _vp, _sz, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "b200g16_bases_download": (C.c_int, [_vp, _sz, _sz, _vp]),
+    "b200g16_bases_copy": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
     "b200g16_fixed_base_mul_g1": (C.c_int, [_vp, _vp, _vp, _sz, _vp]),
     "b200g16_fixed_base_mul_g2": (C.c_int, [_vp, _vp, _vp, _sz, _vp]),
     "b200g16_bases_from_scalars_g1": (C.c_int, [_vp, _vp, _vp, _sz, C.POINTER(_vp)]),
@@ -110,6 +111,8 @@ SIGNATURES = {
     "b200g16_group_pk_upload": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
     "b200g16_group_pk_free": (None, [_vp]),
     "b200g16_group_prove": (C.c_int, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp]),
+    "b200g16_group_pk_replicate": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
+    "b200g16_group_prove_batch": (C.c_int, [_vp, _vp, _sz, _vp, _sz, _vp, _vp, _vp, _sz, _vp, _vp, _vp]),
     "b200g16_dist_h_init": (C.c_int, [_vp, C.c_uint, C.c_int, C.c_int, _vp]),
     "b200g16_dist_h_open": (C.c_int, [_vp, _vp]),
     "b200g16_dist_h_load": (C.c_int, [_vp, _vp, _vp, _vp]),
@@ -362,6 +365,19 @@ def _pk_desc(log2_domain, n_wires, A, B, K, Z, B2, alpha, beta, delta, beta2, de
     return d, keep
 
 
+def _batch_rows(what, wires, a, b, c, r, s):
+    """The host rows of a batch prove as the library reads them -> (k, wires, a, b, c, r, s); refuses shapes that would
+    let it read past a buffer, before any library call."""
+    wires, a, b, c = [np.ascontiguousarray(x, dtype=np.uint64) for x in (wires, a, b, c)]
+    k = wires.shape[0]
+    if wires.ndim != 3 or any(x.ndim != 3 or x.shape[0] != k for x in (a, b, c)) or not a.shape == b.shape == c.shape:
+        raise B200Error(f"{what}: wires must be (k, n_wires, 4), a/b/c (k, n_constraints, 4)")
+    r, s = _u64(r, 4), _u64(s, 4)
+    if r.shape[0] != k or s.shape[0] != k:
+        raise B200Error(f"{what}: one r and one s per proof")
+    return k, wires, a, b, c, r, s
+
+
 def host_register(arr):
     """Page-lock a numpy array in place (b200g16_host_register); returns the array."""
     _check(load().b200g16_host_register(_ptr(arr), arr.nbytes))
@@ -432,7 +448,16 @@ class Group:
         del keep
         return h
 
+    def pk_replicate(self, pk):
+        """A whole single-device key (a Context.pk_upload handle, on any device) on every device of the group
+        (b200g16_group_pk_replicate): members on the key's device borrow its vectors, every other device gets one
+        copy, window tables included.  The source must outlive the returned key; prove with prove_batch."""
+        h = _vp()
+        _check(load().b200g16_group_pk_replicate(self.h, pk, C.byref(h)))
+        return h
+
     def pk_free(self, pk):
+        """Releases a sharded (pk_upload) or a replicated (pk_replicate) key."""
         load().b200g16_group_pk_free(pk)
 
     def prove(self, pk, wires, a, b, c, r, s, want_h=False, log2_domain=None):
@@ -443,6 +468,15 @@ class Group:
         _check(load().b200g16_group_prove(self.h, pk, _ptr(wires), wires.shape[0], _ptr(a), _ptr(b), _ptr(c), a.shape[0],
                                           _ptr(r), _ptr(s), C.byref(out), _ptr(h) if want_h else None))
         return out.as_dict(), h
+
+    def prove_batch(self, pk, wires, a, b, c, r, s):
+        """b200g16_group_prove_batch with a replicated key: Context.prove_batch's arguments and results, the k proofs
+        split into contiguous ranges over the members."""
+        k, wires, a, b, c, r, s = _batch_rows("group prove_batch", wires, a, b, c, r, s)
+        out = (ProofOut * max(k, 1))()
+        _check(load().b200g16_group_prove_batch(self.h, pk, k, _ptr(wires), wires.shape[1], _ptr(a), _ptr(b), _ptr(c),
+                                                a.shape[1], _ptr(r), _ptr(s), out))
+        return [out[j].as_dict() for j in range(k)]
 
 
 class Bases:
@@ -522,6 +556,13 @@ class Context:
         h = _vp()
         _check(load().b200g16_bases_upload_g2(self.h, _ptr(pts), pts.shape[0], C.byref(h)))
         return Bases(self, h, 2, pts.shape[0])
+
+    def bases_copy(self, bases):
+        """A copy of a resident vector (on any device) on this ctx's device, its window table included
+        (b200g16_bases_copy, device to device); independent of the source."""
+        h = _vp()
+        _check(load().b200g16_bases_copy(self.h, bases.handle, C.byref(h)))
+        return Bases(self, h, bases.group, bases.n)
 
     # -- fixed-base batch scalar multiplication (BatchScalarMultiplicationG1/G2)
     def fixed_base_mul(self, base, scalars, group=1, resident=False):
@@ -724,13 +765,7 @@ class Context:
     def prove_batch(self, pk, wires, a, b, c, r, s):
         """b200g16_prove_batch: k proves of one circuit.  wires (k, n_wires, 4), a/b/c (k, n_constraints, 4), r/s (k, 4),
         all Montgomery -> list of k dicts as prove() returns them."""
-        wires, a, b, c = [np.ascontiguousarray(x, dtype=np.uint64) for x in (wires, a, b, c)]
-        k = wires.shape[0]
-        if wires.ndim != 3 or any(x.ndim != 3 or x.shape[0] != k for x in (a, b, c)) or not a.shape == b.shape == c.shape:
-            raise B200Error("prove_batch: wires must be (k, n_wires, 4), a/b/c (k, n_constraints, 4)")
-        r, s = _u64(r, 4), _u64(s, 4)
-        if r.shape[0] != k or s.shape[0] != k:
-            raise B200Error("prove_batch: one r and one s per proof")
+        k, wires, a, b, c, r, s = _batch_rows("prove_batch", wires, a, b, c, r, s)
         out = (ProofOut * max(k, 1))()
         _check(load().b200g16_prove_batch(self.h, pk, k, _ptr(wires), wires.shape[1], _ptr(a), _ptr(b), _ptr(c),
                                           a.shape[1], _ptr(r), _ptr(s), out))

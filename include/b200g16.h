@@ -157,6 +157,14 @@ int b200g16_msm_plan(const b200g16_ctx* ctx, const b200g16_bases* bases, size_t 
 /* Copy points [offset, offset+n) of a resident vector back to the host (tests / sampling). */
 int b200g16_bases_download(const b200g16_bases* bases, size_t offset, size_t n, uint64_t* out_points);
 
+/* A new resident vector on ctx's device with the points of `src` (which may live on any device), including its
+ * window table (the tab_W rows of a b200g16_bases_precompute'd vector) when it has one, so the copy needs no
+ * precompute of its own.  The copy is device to device (cudaMemcpyPeerAsync on ctx's stream): over NVLink where the
+ * devices are peers, staged by the driver otherwise; the call returns once it is complete.  The copy is independent
+ * of src: either may be freed first.  A vector from setup or from a multi-device key can so reach another device
+ * without a round trip through the host. */
+int b200g16_bases_copy(b200g16_ctx* ctx, const b200g16_bases* src, b200g16_bases** out);
+
 /* ---- batch fixed-base scalar multiplication (Setup's hot loop) --------------------- */
 /* out_points[i] = scalars[i] * base.  Replaces gnark-crypto ecc/bn254
  * BatchScalarMultiplicationG1 / BatchScalarMultiplicationG2 as used by gnark
@@ -603,6 +611,30 @@ void b200g16_group_pk_free(b200g16_group_pk* pk);
 int b200g16_group_prove(b200g16_group* g, const b200g16_group_pk* pk, const uint64_t* wires, size_t n_wires,
                         const uint64_t* a, const uint64_t* b, const uint64_t* c, size_t n_constraints,
                         const uint64_t r[4], const uint64_t s[4], b200g16_proof* proof_out, uint64_t* h_out);
+
+/* ---- batch prove over a group: a whole key on every device, whole proofs per device ----------------------
+ * A replicated key: the whole (non-partial) resident key `src` (b200g16_pk_upload, with or without precompute, or
+ * b200g16_setup's vectors through res_*), on any device, made available on every device of the group.  Members on
+ * src's device use src's point vectors without copying (src must then outlive the group key, as res_* vectors must
+ * outlive a pk); every other distinct device receives one owned copy of the five vectors, window tables included,
+ * shared by the members that name that device.  The copies run as a doubling broadcast: in each round every device
+ * that already holds the key serves one that does not, one cudaMemcpyPeerAsync per vector on the receiver's stream
+ * after a cross-device event from its source.  Every member gets its own gather lists.  Returns once every copy has
+ * completed.  B200G16_ERR_ARG: NULL, a partial src.  A failed copy releases everything created so far.
+ * b200g16_group_pk_free releases either kind of group key (never src). */
+int b200g16_group_pk_replicate(b200g16_group* g, const b200g16_pk* src, b200g16_group_pk** out);
+/* k proves of one circuit over the group, with a replicated key: the arguments, the layout (wires k x n_wires,
+ * a / b / c k x n_constraints, r / s k x 4) and the per-proof results of b200g16_prove_batch, every proof
+ * bit-identical to it.  Proofs are split into contiguous ranges, one per member, sizes differing by at most one; each
+ * member runs b200g16_prove_batch's pipeline (with its sub-batching) on its range from its own host thread, and the
+ * proofs land at their own indexes.  No data crosses devices.  Errors: those of b200g16_prove_batch (k = 0 returns 0
+ * and writes nothing); a sharded key is B200G16_ERR_ARG (b200g16_group_prove likewise refuses a replicated key:
+ * summing the replicas' partial proofs would give a wrong proof); a key built by another group is
+ * B200G16_ERR_STATE.  A failure on one device drains every device and names that device; every ctx stays usable.
+ * b200g16_last_timings on each member ctx that proved: its 8 phases, as b200g16_prove_batch reports them. */
+int b200g16_group_prove_batch(b200g16_group* g, const b200g16_group_pk* pk, size_t k, const uint64_t* wires,
+                              size_t n_wires, const uint64_t* a, const uint64_t* b, const uint64_t* c,
+                              size_t n_constraints, const uint64_t* r, const uint64_t* s, b200g16_proof* proofs_out);
 
 /* ---- computeH split over 2 / 4 / 8 GPUs, one PROCESS per GPU ---------------------------------------
  * (b200g16_group_prove does the same inside one process.)  Rank `me` of n_peers holds positions

@@ -11,6 +11,7 @@ package b200
 import "C"
 
 import (
+	"errors"
 	"math/bits"
 	"runtime"
 	"unsafe"
@@ -92,5 +93,94 @@ func (pk *GroupProvingKey) Free() {
 	if pk.grp != nil {
 		C.b200g16_group_destroy(pk.grp)
 		pk.grp = nil
+	}
+}
+
+// ReplicatedKey = a whole resident single-GPU key on every GPU of a group, for throughput: each device proves whole
+// proofs of its own share of a batch, with no data crossing devices.
+type ReplicatedKey struct {
+	grp *C.b200g16_group
+	dev *C.b200g16_group_pk
+}
+
+// Replicate starts a group over devices (CUDA ordinals) and makes pk's resident key (from Setup, or uploaded by a
+// first Prove / BatchProve) available on every one of them: devices other than pk's receive device-to-device
+// copies of the point vectors, window tables included.  pk must outlive the replicated key.
+func Replicate(pk *ProvingKey, devices []int) (*ReplicatedKey, error) {
+	if pk.dev == nil {
+		return nil, errors.New("b200: Replicate needs a resident key (Setup, or one Prove / BatchProve first)")
+	}
+	if len(devices) == 0 {
+		return nil, errors.New("b200: Replicate needs at least one device")
+	}
+	devs := make([]C.int, len(devices))
+	for i, d := range devices {
+		devs[i] = C.int(d)
+	}
+	rk := &ReplicatedKey{}
+	if err := call(func() C.int { return C.b200g16_group_init(&devs[0], C.int(len(devs)), &rk.grp) }); err != nil {
+		return nil, err
+	}
+	if err := call(func() C.int { return C.b200g16_group_pk_replicate(rk.grp, pk.dev, &rk.dev) }); err != nil {
+		rk.Free()
+		return nil, err
+	}
+	return rk, nil
+}
+
+// BatchProveSolved proves k solved witnesses of one circuit over the group, rs[j], ss[j] the blinding scalars of
+// proof j: one b200g16_group_prove_batch call, the proofs split into contiguous ranges over the devices.  Proof j
+// equals BatchProve's proof for the same solution and r, s.  A circuit's commitments and proofs of knowledge are the
+// caller's, as in ProveSolved.
+func (rk *ReplicatedKey) BatchProveSolved(solutions []*cs.R1CSSolution, rs, ss []fr.Element) ([]*groth16_bn254.Proof, error) {
+	k := len(solutions)
+	if len(rs) != k || len(ss) != k {
+		return nil, errors.New("b200: BatchProveSolved needs one r and one s per solution")
+	}
+	if k == 0 {
+		return nil, nil
+	}
+	nWires, nCons := len(solutions[0].W), len(solutions[0].A)
+	wires := make([]fr.Element, 0, k*nWires)
+	A := make([]fr.Element, 0, k*nCons)
+	B := make([]fr.Element, 0, k*nCons)
+	Cv := make([]fr.Element, 0, k*nCons)
+	for _, sol := range solutions {
+		if len(sol.W) != nWires || len(sol.A) != nCons || len(sol.B) != nCons || len(sol.C) != nCons {
+			return nil, errors.New("b200: BatchProveSolved needs solutions of one circuit")
+		}
+		wires = append(wires, sol.W...)
+		A = append(A, sol.A...)
+		B = append(B, sol.B...)
+		Cv = append(Cv, sol.C...)
+	}
+	out := make([]C.b200g16_proof, k)
+	err := call(func() C.int {
+		return C.b200g16_group_prove_batch(rk.grp, rk.dev, C.size_t(k), u64(unsafe.Pointer(&wires[0])), C.size_t(nWires),
+			u64(unsafe.Pointer(&A[0])), u64(unsafe.Pointer(&B[0])), u64(unsafe.Pointer(&Cv[0])), C.size_t(nCons),
+			u64(unsafe.Pointer(&rs[0])), u64(unsafe.Pointer(&ss[0])), &out[0])
+	})
+	if err != nil {
+		return nil, err
+	}
+	proofs := make([]*groth16_bn254.Proof, k)
+	for j := range proofs {
+		proofs[j] = &groth16_bn254.Proof{}
+		proofs[j].Ar = *(*curve.G1Affine)(unsafe.Pointer(&out[j].ar))
+		proofs[j].Bs = *(*curve.G2Affine)(unsafe.Pointer(&out[j].bs))
+		proofs[j].Krs = *(*curve.G1Affine)(unsafe.Pointer(&out[j].krs))
+	}
+	return proofs, nil
+}
+
+// Free releases the copies and the group (never the source key).
+func (rk *ReplicatedKey) Free() {
+	if rk.dev != nil {
+		C.b200g16_group_pk_free(rk.dev)
+		rk.dev = nil
+	}
+	if rk.grp != nil {
+		C.b200g16_group_destroy(rk.grp)
+		rk.grp = nil
 	}
 }
